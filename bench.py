@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm's CPU port (oracle/) on host cores
   python bench.py --config psgcfs|rrtstar ...              # the other BASELINE.json configurations (parity cases with a number)
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's results as DIR/<name>.npy (float64)
 
 --config cfs (default, the headline; BASELINE.json configs[2]).  One "step" = one pass of the hot path over one batch:
 CFS_FANUC.optimizer run to the reference's stop rule for every problem of a 4096-problem synthetic batch.
@@ -62,7 +63,13 @@ def parse_args():
     ap.add_argument("--grad", default="numjac", choices=["numjac", "derivest"])
     ap.add_argument("--contexts", type=int, default=0, help="library contexts (streams + buffer sets) the steps rotate over (cfs and psgcfs 24, rrtstar 8)")
     ap.add_argument("--cpu-reps", type=int, default=3, help="CPU baseline: passes of the oracle over the same batch")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the timed path computed in its last step as "
+                    "DIR/<name>.npy (float64, at most 64 MB in all), to compare two builds on the same seeded inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     a.batch = a.batch or {"cfs": 4096, "psgcfs": 2048, "rrtstar": 1024}[a.config]
     a.horizon = a.horizon or {"cfs": 50, "psgcfs": 30, "rrtstar": 40}[a.config]
     a.contexts = a.contexts or {"cfs": 24, "psgcfs": 24, "rrtstar": 8}[a.config]
@@ -124,6 +131,28 @@ class ClockSampler:
                 pass
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm), "window": window}
+
+
+DUMP_BYTES = 64 * 10 ** 6 - 4096  # 64 MB in all, less room for the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy in float64 (exact for the int32 iteration counts and status words).
+    Above DUMP_BYTES in all, the same fixed seeded sample of rows is kept of every array whose first dimension is the batch
+    (the largest one), and the sampled row indices go to rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    rows = max(a.shape[0] for a in arrays.values())
+    per_row = sum(a.nbytes for a in arrays.values() if a.shape[0] == rows) / rows
+    rest = sum(a.nbytes for a in arrays.values() if a.shape[0] != rows)
+    if rest + per_row * rows > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(rows, int((DUMP_BYTES - rest) // (per_row + 8)), replace=False))
+        arrays = {k: a[keep] if a.shape[0] == rows else a for k, a in arrays.items()}
+        arrays["rows"] = keep.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    print("bench.py: %d arrays (%.1f MB) written to %s" % (len(arrays), sum(a.nbytes for a in arrays.values()) / 1e6, path),
+          file=sys.stderr, flush=True)
 
 
 def bind_to_gpu_numa(index):
@@ -298,6 +327,7 @@ def make_env(args):
     e.main_stream = torch.cuda.Stream(device=e.dev)
     e.flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=e.dev)  # 256 MB > 126 MB L2
     e.launches = 0
+    e.outputs = None  # --dump-outputs: host copies of the last timed step's results (rank 0)
     return e
 
 
@@ -439,6 +469,8 @@ def bench_solver(args, e):
     ms_dev = run_steps(e, ctxs, streams, args.steps, lambda c: issue(c, False), False,
                        after=None if os.environ.get("BENCH_NO_GATHER") else final_gather)
     barrier(e)
+    if args.dump_outputs and e.rank == 0:  # what cfs_solve_batch_device returned for the last timed step's batch
+        e.outputs = {k: v.cpu().numpy() for k, v in d_out[(args.steps - 1) % NC].items()}
     rank_ms = [ms_dev]
     if e.world > 1:  # every rank's own device time (diagnostic: the value uses the max)
         t_all = torch.zeros(e.world, dtype=torch.float64, device=e.dev)
@@ -476,8 +508,7 @@ def bench_solver(args, e):
     NP = min(NC, 8)
     run_steps(e, ctxs[:NP], streams[:NP], NP, issue_pageable, True)
     barrier(e)
-    steps_p = min(args.steps, 24)
-    ms_page = run_steps(e, ctxs[:NP], streams[:NP], steps_p, issue_pageable, True)
+    ms_page = run_steps(e, ctxs[:NP], streams[:NP], args.steps, issue_pageable, True)
     barrier(e)
     (ms_page,) = max_over_ranks(e, [ms_page])
 
@@ -575,8 +606,8 @@ def bench_solver(args, e):
                        "api": "cfs_solve_batch_async + cfs_wait (host pointers, pinned): every array of the class contract in "
                               "(x0, ff, caug, x_) and out (u, x_, cost_all, e_u_all, iters, status), H2D + solve + D2H of every "
                               "step inside the timed events, %d contexts in rotation" % NC},
-        "e2e_pageable": {"value": e.world * B * steps_p / (ms_page * 1e-3), "unit": unit, "steps": steps_p,
-                         "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "ms_per_step": ms_page / steps_p,
+        "e2e_pageable": {"value": e.world * B * args.steps / (ms_page * 1e-3), "unit": unit, "steps": args.steps,
+                         "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "ms_per_step": ms_page / args.steps,
                          "api": "the same entry with pageable (numpy / mxGetPr-like) caller buffers: the library stages them "
                                 "through its own pinned buffers (one memcpy each way), %d contexts in rotation" % NP},
         "gpu_launches": int(launches_timed),
@@ -754,6 +785,11 @@ def bench_rrtstar(args, e):
     e.launches = 0
     ms_dev = run_steps(e, ctxs, streams, args.steps, lambda c: issue(c, False), False)
     barrier(e)
+    if args.dump_outputs and e.rank == 0:  # the last timed step: per-seed routes and CFS results, and the best-of
+        b = buf[(args.steps - 1) % NC]
+        i = b["ints"]
+        e.outputs = {k: v.cpu().numpy() for k, v in dict(best=b["best"], routes=b["routes"], route_len=i[0], tree_nodes=i[1], fail=i[2],
+                                                         u=b["u"], x=b["x"], cost=b["c"], eu=b["eu"], iters=b["it"], status=b["st"]).items()}
     e.flush.zero_()
     barrier(e)
     ms_e2e = run_steps(e, ctxs, streams, args.steps, lambda c: issue(c, True), False)
@@ -838,6 +874,11 @@ def main():
         bench_rrtstar(args, e)
     else:
         bench_solver(args, e)
+    if e.outputs is not None:
+        o = e.outputs
+        for k in ("cost", "eu"):  # NaN after each problem's last iteration (include/cfs_b200.h): written as 0, iters.npy has the length
+            o[k] = np.where(np.arange(o[k].shape[1]) < o["iters"][:, None], o[k], 0.0)
+        dump_outputs(args.dump_outputs, o)
     if e.world > 1:
         e.dist.destroy_process_group()
 

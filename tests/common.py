@@ -13,6 +13,30 @@ def golden(name):
     return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name))
 
 
+FROZEN_KEYS = ("QQ", "ff", "caug", "alpha")
+
+
+def assert_rounding_close(got, ref, what):
+    """got equals ref up to the rounding of a matrix product: |got - ref| <= 1e-13 max|ref|"""
+    got, ref = np.asarray(got, dtype=np.float64), np.asarray(ref, dtype=np.float64)
+    assert got.shape == ref.shape and np.abs(got - ref).max() <= 1e-13 * np.abs(ref).max(), what
+
+
+def frozen_inputs(name, s):
+    """sys_info `s` of the golden configuration `name` with QQ, ff, caug and alpha as they were when its goldens were computed
+    (tests/golden/solver_inputs.npz, written by tests/golden/make_solver_inputs.py).  The config builders compute these with
+    BLAS / LAPACK products and SIMD sums whose last bits change with the CPU, the BLAS kernel and its thread count, and some
+    golden problems amplify that above the golden tolerances.  The freshly built values must agree with the frozen ones to
+    rounding; the solve then starts from the exact numbers the goldens came from."""
+    g = golden("solver_inputs.npz")
+    out = dict(s)
+    for k in FROZEN_KEYS:
+        ref = g["%s.%s" % (name, k)]
+        assert_rounding_close(s.get(k, 0.0), ref, (name, k))
+        out[k] = ref if ref.ndim else float(ref)
+    return out
+
+
 def main_fanuc_config():
     """main_FANUC.m:13-60,106-127 : M200i, H=30, one capsule obstacle."""
     robot = M.robotproperty2("M200i")

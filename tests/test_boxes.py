@@ -2,7 +2,6 @@
 dist_arm_surface.m:44).  CPU: known answers of the oracle's segment-to-box distance (degenerate, inside, edge-parallel, corner
 cases), an independent brute-force cross-check, the STL -> box tool on a synthetic mesh, and the frozen golden built from the
 reference's map/assembly line_Assem1.STL.  GPU (-m gpu): K1 / K1d / K6 / the fused solver against the oracle on those boxes."""
-import os
 import struct
 
 import numpy as np
@@ -95,13 +94,10 @@ def test_box_golden_matches_the_oracle(oracle):
             d, lid = oracle.dist_arm(r, g["theta"][i], o7)[:2]
             assert d == g["dist"][i, j] and lid == g["linkid"][i, j]
     robot = M.robotproperty2("M16iB")
-    s = M.make_sys_info(robot, 5, 30, g["solve1.theta0"], g["solve1.thetag"])
+    s = common.frozen_inputs("box_solve1", M.make_sys_info(robot, 5, 30, g["solve1.theta0"], g["solve1.thetag"]))
     P = common.oracle_problem(oracle, "M16iB", obs, s)
     res = P.solve_batch(s["xR"][:, 0][None], s["ff"][None], np.array([s["caug"]]), s["x_"][None])
     assert int(res["iters"][0]) == int(g["solve1.iters"]) and np.array_equal(res["x"][0], g["solve1.x"])
-    if os.path.exists(tests_stl := "/root/reference/map/assembly line_Assem1.STL"):   # build container only
-        fresh = stl_boxes.boxes_from_stl(tests_stl, max_boxes=512, near=[3.25, 8.5, 0.8], radius=1.6, max_keep=12, max_size=1.2)
-        assert np.array_equal(np.stack([o["l"] for o in fresh], axis=2), g["box_l"])
 
 
 @pytest.mark.gpu

@@ -146,22 +146,24 @@ def test_main_fanuc_oracle_golden(oracle):
 # ---- golden fixtures (tests/golden/, frozen by tests/golden/make_golden.py) ------------------------------------------
 def _golden_cases(O):
     """name -> (ROBOT, obs, sys_info, solver, grad, noise): the reference's shipped configurations rebuilt from the
-    committed input fixtures (no /root/reference at test time)."""
+    committed input fixtures, with the solver inputs the goldens were computed from (common.frozen_inputs)."""
     inp = common.golden("inputs.npz")
     cases = {}
     ROBOT, robot, obs, s = common.main_fanuc_config()
+    s = common.frozen_inputs("main_fanuc", s)
     cases["main_fanuc_cfs"] = (ROBOT, obs, s, 0, 0, None)
     noise = np.random.default_rng(123).normal(0.0, 0.1, size=(1, s["MAX_O_ITER"], s["H"] * 5))
     cases["main_fanuc_psgcfs"] = (ROBOT, obs, s, 1, 0, noise)
     ROBOT, robot, obs, s = common.main_2l_config()
-    cases["main_2l_cfs"] = (ROBOT, obs, s, 0, 0, None)
+    cases["main_2l_cfs"] = (ROBOT, obs, common.frozen_inputs("main_2l", s), 0, 0, None)
     ROBOT, robot, obs, s = common.main_cfs_m16ib_config(inp["xuori"])
+    s = common.frozen_inputs("m16ib_script", s)
     cases["m16ib_script_derivest"] = (ROBOT, obs, s, 0, 1, None)
     obs2 = [dict(obs[0], l=np.array(common.OBS_M16_SCRIPT_ALT))]
     cases["m16ib_script_alt_derivest"] = (ROBOT, obs2, s, 0, 1, None)
     cases["m16ib_script_alt_numjac"] = (ROBOT, obs2, s, 0, 0, None)
     ROBOT, robot, obs, s = common.rrtstar_route_config(inp["route_wp"])
-    cases["rrtstar_cfs"] = (ROBOT, obs, s, 0, 0, None)
+    cases["rrtstar_cfs"] = (ROBOT, obs, common.frozen_inputs("rrtstar", s), 0, 0, None)
     return cases
 
 

@@ -32,21 +32,29 @@ def _problem(fx):
 
 def test_fixtures_match_the_configurations_and_round_trip(tmp_path, oracle):
     """the fixtures make_reference_golden.m reads hold exactly the golden configurations; solving FROM a fixture reproduces the
-    frozen oracle golden of the same case (so MATLAB and the oracle are fed identical numbers)."""
+    frozen oracle golden of the same case (so MATLAB and the oracle are fed identical numbers).  The arrays the config builders
+    compute with BLAS / LAPACK (QQ, ff, caug, Aaug, Baug, alpha) match the committed fixture to rounding (common.frozen_inputs),
+    every other array exactly."""
     g = common.golden("cases.npz")
     for name, arrays in export_fixtures.cases().items():
         p = tmp_path / (name + ".bin")
         fixture_io.write_fixture(str(p), arrays)
         fx = fixture_io.read_fixture(str(p))
-        ROBOT, obs, s, solver, noise = _problem(fx)
+        assert set(fx) == set(arrays) and all(np.array_equal(fx[k], np.asarray(arrays[k], dtype=np.float64)) for k in fx), name
+        committed = os.path.join(HERE, "golden", "fixtures", name + ".bin")
+        assert os.path.exists(committed), "run python tests/golden/export_fixtures.py"
+        cf = fixture_io.read_fixture(committed)
+        assert set(cf) == set(fx), name
+        for k in fx:
+            if k in ("QQ", "ff", "caug", "Aaug", "Baug", "alpha"):
+                common.assert_rounding_close(fx[k], cf[k], (name, k))
+            else:
+                assert np.array_equal(cf[k], fx[k]), (name, k)
+        ROBOT, obs, s, solver, noise = _problem(cf)
         P = common.oracle_problem(oracle, ROBOT, obs, s, solver=solver)
         r = P.solve_batch(s["xR"][:, 0][None], s["ff"][None], np.array([s["caug"]]), s["x_"][None], noise=noise)
         assert int(r["iters"][0]) == int(g[name + ".iters"]) and int(r["status"][0]) == int(g[name + ".status"])
         assert np.array_equal(r["x"][0], g[name + ".x"]), name
-        committed = os.path.join(HERE, "golden", "fixtures", name + ".bin")
-        assert os.path.exists(committed), "run python tests/golden/export_fixtures.py"
-        cf = fixture_io.read_fixture(committed)
-        assert set(cf) == set(fx) and all(np.array_equal(cf[k], fx[k]) for k in fx), name
 
 
 def _compare(name, ref, out):
