@@ -201,6 +201,41 @@ int cfs_get_con(cfs_ctx *ctx, int grad_mode, int margin_is_D, const double *x0, 
 /* RRT_FANUC.feasible (Lib/RRT_FANUC.m:146-181) for N candidate nodes: feasible[i]=1 iff every link distance to every
  * obstacle is >= obs.D; dmin = min distance over links and obstacles. */
 int cfs_nodes_feasible(cfs_ctx *ctx, int N, const double *theta /*nj x N*/, unsigned char *feasible, double *dmin);
+/* ---- continuous collision checks (extension: the reference checks RRT nodes only, RRT_FANUC.m:129,146-181) ------------
+ * Clearance of a configuration: c(theta) = min over links l and obstacles j of (d_lj(theta) - m_j), d_lj the link-axis distance
+ * of cfs_nodes_feasible / cfs_dist_grad (capsules and boxes, "axes touch" rule included), m_j = obs{j}.D if margin_is_D != 0,
+ * else obs{j}.epsilon.  At one configuration the hit test gives exactly the verdict of cfs_nodes_feasible.
+ * Paths: an edge is theta(s) = theta_a + s (theta_b - theta_a), s in [0, 1] (RRT edges, route polylines); segment k of a
+ * trajectory is the double integrator between its waypoints, theta(tau) = theta_k + omega_k tau + (tau^2 / 2) u_k, tau in
+ * [0, dt], from state x_k (x0 for k = 0) with control u_k -- exact for CFS trajectories (A = [I dt I; 0 I], B = [dt^2/2 I; dt I]).
+ * Motion bound: cfs_set_robot computes per joint R_j >= ||dp/dtheta_j|| for every link-axis endpoint p of the links l >= j at
+ * every theta (triangle inequality over the DH / robot.T translations and the capsule endpoints), so that
+ * |c(theta1) - c(theta2)| <= sum_j R_j TV_j (TV_j: total variation of joint j between them).
+ * Algorithm (conservative advancement, tolerance eta > 0), sequential per item:
+ *   vmax = sum_j R_j |theta_b,j - theta_a,j| (edge), sum_j R_j max(|omega_j|, |omega_j + u_j dt|) (segment);
+ *   s = 0; loop: evaluate c(s); c < -eta/2 -> HIT at s; s at the end (or vmax == 0) -> CLEAR;
+ *   else s += (c + eta) / vmax, clamped to the end.  More than max_evals evaluations needed -> UNDECIDED.
+ * Guarantees: a CLEAR item has c >= -eta along its whole path; a HIT item has a witness with c < -eta/2 and c >= -eta before it.
+ * So an item whose true minimum is >= -eta/2 is CLEAR, one below -eta is HIT; the eta/2 threshold keeps waypoints that the
+ * linearised CFS constraint leaves ~1e-9 below the margin from counting as hits.  CFS_E_ARG unless eta > 0 and
+ * min_j m_j - eta >= 1e-4 (the touch rule then never fires inside the certified band) and max_evals >= 1.  No robot or
+ * obstacles yet: CFS_E_STATE.  N = 0 / B = 0: no-op.  Results are deterministic (no order-dependent reduction). */
+enum { CFS_CHECK_CLEAR = 0, CFS_CHECK_HIT = 1, CFS_CHECK_UNDECIDED = 2 };
+/* per edge: verdict, s_hit (-1 if none), cmin = smallest c evaluated, evals (may be NULL) */
+int cfs_check_edges(cfs_ctx *ctx, int N, const double *theta_a /*nj x N*/, const double *theta_b /*nj x N*/, double eta,
+                    int margin_is_D, int max_evals, int *verdict, double *s_hit, double *cmin, int *evals);
+/* per trajectory (x must be the roll-out of u, as every solve entry returns it): verdict = HIT if any segment hits, else
+ * UNDECIDED if any segment is, else CLEAR; t_hit = earliest hit time in [0, H dt] (k dt + tau, -1 if none); cmin = min over
+ * segments; evals = sum over segments (may be NULL) */
+int cfs_check_trajectories(cfs_ctx *ctx, int B, int H, const double *x0 /*2nj x B*/, const double *x /*2njH x B*/,
+                           const double *u /*njH x B*/, double eta, int margin_is_D, int max_evals, int *verdict,
+                           double *t_hit, double *cmin, int *evals);
+/* the same with every pointer a DEVICE pointer; asynchronous on the context stream unless sync != 0 */
+int cfs_check_edges_device(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta, int margin_is_D,
+                           int max_evals, int *verdict, double *s_hit, double *cmin, int *evals, int sync);
+int cfs_check_trajectories_device(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u, double eta,
+                                  int margin_is_D, int max_evals, int *verdict, double *t_hit, double *cmin, int *evals,
+                                  int sync);
 /* RRT_FANUC.getRandNode nearest scan + steer (Lib/RRT_FANUC.m:116-129) for S samples against one tree:
  * parent[s] = argmin_i ||(nodes(:,i)-sample(:,s)).*ratial|| (first minimum, 0-based), newnode = parent + (sample-parent)*step/||parent-sample||. */
 int cfs_nearest_steer(cfs_ctx *ctx, int n_nodes, const double *nodes /*nj x n_nodes*/, int S, const double *samples /*nj x S*/,

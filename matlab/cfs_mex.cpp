@@ -22,6 +22,13 @@
 //     cubicpolytraj resampling to sys_info.H + 1 points, cost set-up from its blocks (Q 2nj x 2nj, Rblk nj x nj, R*r_scale),
 //     CFS_FANUC.optimizer.  sys_info.{H, njoint, robot, lim, MAX_input, epsilon_O, MAX_O_ITER}.
 //
+//   [verdict, s_hit, cmin, evals] = cfs_mex('check', ROBOT, obs, sys_info, 'edges', A, B [, eta, margin_is_D])
+//   [verdict, t_hit, cmin, evals] = cfs_mex('check', ROBOT, obs, sys_info, 'trajectory', x0, x_, u [, eta, margin_is_D])
+//     continuous collision checks (extension; include/cfs_b200.h cfs_check_edges / cfs_check_trajectories): the edges
+//     A(:,i) -> B(:,i) (njoint x N), or the solved trajectories x0 (nstate x B), x_ (nstate*H x B), u (njoint*H x B) between
+//     their waypoints.  sys_info.robot and sys_info.njoint (or, for the RRT stage's sys_info, nstate).  eta = 1e-3 and
+//     margin_is_D = 1 (obs{j}.D; 0: obs{j}.epsilon) by default.  verdict: 0 clear, 1 hit, 2 undecided (1 x N int32).
+//
 //   cfs_mex('device', id)   bind this MATLAB process to GPU `id` (call before anything else; parfor workers:
 //                           cfs_mex('device', mod(labindex - 1, gpuDeviceCount)), see matlab/s_Parallel_rrt.m).
 //                           Default: environment variable CFS_DEVICE, else 0.
@@ -349,8 +356,49 @@ static void cmd_routes(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[
   if (nlhs > 5) plhs[5] = st;
 }
 
+// ---- 'check' ------------------------------------------------------------------------------------------------------------------
+static void cmd_check(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
+  if (nrhs < 6)
+    mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex('check', ROBOT, obs, sys_info, 'edges', A, B [, eta, margin_is_D]) or "
+                                 "cfs_mex('check', ROBOT, obs, sys_info, 'trajectory', x0, x_, u [, eta, margin_is_D])");
+  const std::string robot_name = str(prhs[0]), what = str(prhs[3]);
+  const mxArray *obs = prhs[1], *si = prhs[2];
+  if (what != "edges" && what != "trajectory") mexErrMsgIdAndTxt("cfs:arg", "check '%s' (edges | trajectory)", what.c_str());
+  const bool edges = what == "edges";
+  if (!edges && nrhs < 7) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex('check', ROBOT, obs, sys_info, 'trajectory', x0, x_, u [, eta, margin_is_D])");
+  const mxArray *njf = field(si, "njoint", false);
+  const int nj = (int)scalar(njf ? njf : field(si, "nstate"), "sys_info.njoint");
+  const int nopt = edges ? 6 : 7;
+  const double eta = nrhs > nopt ? scalar(prhs[nopt], "eta") : 1e-3;
+  const int margin_is_D = nrhs > nopt + 1 ? (scalar(prhs[nopt + 1], "margin_is_D") != 0.0) : 1;
+  ensure_ctx();
+  bind_robot(robot_name, field(si, "robot"), nj);
+  bind_obstacles(obs);
+  const size_t N = mxGetN(prhs[4]);
+  std::vector<int> verdict(N), evals(N);
+  mxArray *where = mxCreateDoubleMatrix(1, N, mxREAL), *cmin = mxCreateDoubleMatrix(1, N, mxREAL);
+  if (edges) {
+    const double *A = dbl(prhs[4], (size_t)nj * N, "A (njoint x N)"), *B = dbl(prhs[5], (size_t)nj * N, "B (njoint x N)");
+    check(cfs_check_edges(g_ctx, (int)N, A, B, eta, margin_is_D, 4096, verdict.data(), mxGetPr(where), mxGetPr(cmin), evals.data()),
+          "cfs_check_edges");
+  } else {
+    const double *x0 = dbl(prhs[4], (size_t)2 * nj * N, "x0 (nstate x B)");
+    const double *u = dbl(prhs[6], 0, "u (njoint*H x B)");
+    const size_t nu = mxGetNumberOfElements(prhs[6]);
+    if (N == 0 || nu % ((size_t)nj * N) != 0) mexErrMsgIdAndTxt("cfs:arg", "u has %d elements: not njoint*H x B with B = %d", (int)nu, (int)N);
+    const int H = (int)(nu / ((size_t)nj * N));
+    const double *x = dbl(prhs[5], (size_t)2 * nj * H * N, "x_ (nstate*H x B)");
+    check(cfs_check_trajectories(g_ctx, (int)N, H, x0, x, u, eta, margin_is_D, 4096, verdict.data(), mxGetPr(where), mxGetPr(cmin),
+                                 evals.data()), "cfs_check_trajectories");
+  }
+  out_int(plhs[0], verdict);
+  if (nlhs > 1) plhs[1] = where;
+  if (nlhs > 2) plhs[2] = cmin;
+  if (nlhs > 3) out_int(plhs[3], evals);
+}
+
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
-  if (nrhs < 1) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex(command, ...); commands: solve, rrt, routes, device");
+  if (nrhs < 1) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex(command, ...); commands: solve, rrt, routes, check, device");
   const std::string cmd = str(prhs[0]);
   if (cmd == "device") {
     if (nrhs < 2) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex('device', id)");
@@ -362,6 +410,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
   if (cmd == "solve") return cmd_solve(nlhs, plhs, nrhs - 1, prhs + 1);
   if (cmd == "rrt") return cmd_rrt(nlhs, plhs, nrhs - 1, prhs + 1);
   if (cmd == "routes") return cmd_routes(nlhs, plhs, nrhs - 1, prhs + 1);
+  if (cmd == "check") return cmd_check(nlhs, plhs, nrhs - 1, prhs + 1);
   if (cmd == "CFS" || cmd == "PSGCFS" || cmd == "CHOMP") return cmd_solve(nlhs, plhs, nrhs, prhs);  // short calling form
-  mexErrMsgIdAndTxt("cfs:arg", "unknown command '%s' (solve | rrt | routes | device)", cmd.c_str());
+  mexErrMsgIdAndTxt("cfs:arg", "unknown command '%s' (solve | rrt | routes | check | device)", cmd.c_str());
 }

@@ -16,11 +16,13 @@ SOLVER_CFS, SOLVER_PSGCFS = 0, 1
 GRAD_NUMJAC, GRAD_DERIVEST = 0, 1
 STATUS_CONVERGED, STATUS_MAX_ITER, STATUS_INFEASIBLE, STATUS_NUMERICAL, STATUS_NO_ROUTE = 0, 1, 2, 3, 5
 FLAG_TOUCH = 0x100
+CHECK_CLEAR, CHECK_HIT, CHECK_UNDECIDED = 0, 1, 2
 
 # every symbol include/cfs_b200.h declares (tests check that the library exports all of them)
 SYMBOLS = ["cfs_create", "cfs_destroy", "cfs_last_error", "cfs_version", "cfs_set_stream", "cfs_set_option", "cfs_set_robot", "cfs_set_obstacles", "cfs_set_obstacles_ex",
            "cfs_set_cost", "cfs_set_cost_blocks", "cfs_solve_start_goal", "cfs_solve_start_goal_async", "cfs_solve_routes", "cfs_solve_routes_async", "cfs_solve_routes_var", "cfs_solve_routes_var_async", "cfs_solve_routes_device", "cfs_resample_routes", "cfs_solve_batch", "cfs_solve_batch_async", "cfs_chomp_batch", "cfs_wait", "cfs_solve_batch_device", "cfs_dist_grad", "cfs_time_dist_grad", "cfs_get_con",
-           "cfs_nodes_feasible", "cfs_nearest_steer", "cfs_rrt_find_routes", "cfs_rrt_find_routes_device", "cfs_get_stats", "cfs_set_timing", "cfs_get_iter_times", "cfs_get_problem_steps", "cfs_get_qp_profile", "cfs_get_warp_profile", "cfs_measure_fp64_peak"]
+           "cfs_nodes_feasible", "cfs_nearest_steer", "cfs_rrt_find_routes", "cfs_rrt_find_routes_device", "cfs_get_stats", "cfs_set_timing", "cfs_get_iter_times", "cfs_get_problem_steps", "cfs_get_qp_profile", "cfs_get_warp_profile", "cfs_measure_fp64_peak",
+           "cfs_check_edges", "cfs_check_trajectories", "cfs_check_edges_device", "cfs_check_trajectories_device"]
 
 
 class CfsError(RuntimeError):
@@ -340,6 +342,51 @@ class Context:
         rc = self._lib.cfs_nodes_feasible(self._h, C.c_int(N), _dp(theta), _dp(feas), _dp(dmin))
         self._check(rc, "cfs_nodes_feasible")
         return feas.astype(bool), dmin
+
+    def check_edges(self, theta_a, theta_b, eta=1e-3, margin_is_D=True, max_evals=4096):
+        """Continuous collision check of the joint-space edges theta_a[i] -> theta_b[i] ((N, nj) each; include/cfs_b200.h).
+        Returns dict(verdict (CHECK_CLEAR / CHECK_HIT / CHECK_UNDECIDED), s_hit (-1 if none), cmin, evals), each (N,)."""
+        ta, tb = _f64(theta_a), _f64(theta_b)
+        N = ta.shape[0]
+        assert ta.shape == (N, self.nj) and tb.shape == ta.shape
+        out = dict(verdict=np.zeros(N, dtype=np.int32), s_hit=np.zeros(N), cmin=np.zeros(N), evals=np.zeros(N, dtype=np.int32))
+        rc = self._lib.cfs_check_edges(self._h, C.c_int(N), _dp(ta), _dp(tb), C.c_double(eta), C.c_int(1 if margin_is_D else 0),
+                                       C.c_int(max_evals), _dp(out["verdict"]), _dp(out["s_hit"]), _dp(out["cmin"]),
+                                       _dp(out["evals"]))
+        self._check(rc, "cfs_check_edges")
+        return out
+
+    def check_trajectories(self, x0, x, u, eta=1e-3, margin_is_D=True, max_evals=4096):
+        """Continuous collision check of B solved trajectories: x0 (B, 2nj), x (B, 2njH) the roll-out of u (B, njH), as every
+        solve returns them.  Returns dict(verdict, t_hit (-1 if none), cmin, evals), each (B,)."""
+        x0, x, u = _f64(x0), _f64(x), _f64(u)
+        B = x0.shape[0]
+        H = u.shape[1] // self.nj
+        assert x0.shape == (B, 2 * self.nj) and u.shape == (B, H * self.nj) and x.shape == (B, 2 * H * self.nj)
+        out = dict(verdict=np.zeros(B, dtype=np.int32), t_hit=np.zeros(B), cmin=np.zeros(B), evals=np.zeros(B, dtype=np.int32))
+        rc = self._lib.cfs_check_trajectories(self._h, C.c_int(B), C.c_int(max(H, 1)), _dp(x0), _dp(x), _dp(u), C.c_double(eta),
+                                              C.c_int(1 if margin_is_D else 0), C.c_int(max_evals), _dp(out["verdict"]),
+                                              _dp(out["t_hit"]), _dp(out["cmin"]), _dp(out["evals"]))
+        self._check(rc, "cfs_check_trajectories")
+        return out
+
+    def check_edges_ptr(self, N, theta_a, theta_b, verdict, s_hit, cmin, evals, eta=1e-3, margin_is_D=True, max_evals=4096,
+                        sync=True):
+        """cfs_check_edges_device: every array argument a device pointer (int; evals may be 0)."""
+        vp = lambda p: C.c_void_p(p) if p else None
+        rc = self._lib.cfs_check_edges_device(self._h, C.c_int(N), vp(theta_a), vp(theta_b), C.c_double(eta),
+                                              C.c_int(1 if margin_is_D else 0), C.c_int(max_evals), vp(verdict), vp(s_hit),
+                                              vp(cmin), vp(evals), C.c_int(1 if sync else 0))
+        self._check(rc, "cfs_check_edges_device")
+
+    def check_trajectories_ptr(self, B, H, x0, x, u, verdict, t_hit, cmin, evals, eta=1e-3, margin_is_D=True, max_evals=4096,
+                               sync=True):
+        """cfs_check_trajectories_device: every array argument a device pointer (int; evals may be 0)."""
+        vp = lambda p: C.c_void_p(p) if p else None
+        rc = self._lib.cfs_check_trajectories_device(self._h, C.c_int(B), C.c_int(H), vp(x0), vp(x), vp(u), C.c_double(eta),
+                                                     C.c_int(1 if margin_is_D else 0), C.c_int(max_evals), vp(verdict),
+                                                     vp(t_hit), vp(cmin), vp(evals), C.c_int(1 if sync else 0))
+        self._check(rc, "cfs_check_trajectories_device")
 
     def nearest_steer(self, nodes, samples, ratial, step=0.1):
         nodes, samples = _f64(nodes), _f64(samples)

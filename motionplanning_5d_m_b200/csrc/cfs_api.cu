@@ -52,6 +52,7 @@ struct cfs_ctx {
   DerivestTab *ddv = nullptr;
   bool have_robot = false, have_obs = false, have_cost = false;
   int nj = 0, nobs = 0;
+  double motion_R[CFS_MAXL] = {0};  // per-joint motion bound of the continuous checks (cfs_set_robot); kernel argument, not in DevTables
   // cost
   int H = 0, n = 0;
   bool has_lim = false, has_bounds = false;
@@ -68,7 +69,8 @@ struct cfs_ctx {
   DevBuf th0, thg;
   // batch buffers
   DevBuf x0, ff, caug, xref, noise, u, x, cost, eu, u0, v0, cost0, dist, grad, lid, iters, status, flags, listA, listB,
-      counters, slab, scratch_theta, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen, rrt_in;
+      counters, slab, scratch_theta, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen, rrt_in,
+      chk_in, chk_out, chk_seg, chk_ctr;
   int slab_grid = 0, slab_ld = 0;
   // pinned staging of the host-pointer entries: pageable caller buffers (MATLAB's mxGetPr memory, numpy arrays) are copied
   // through these so that cudaMemcpyAsync stays asynchronous; pinned / registered caller buffers are used in place
@@ -271,7 +273,8 @@ extern "C" void cfs_destroy(cfs_ctx *ctx) {
                     &ctx->u0, &ctx->v0, &ctx->cost0, &ctx->dist, &ctx->grad, &ctx->lid, &ctx->iters, &ctx->status,
                     &ctx->flags, &ctx->listA, &ctx->listB, &ctx->counters, &ctx->slab, &ctx->scratch_theta,
                     &ctx->scratch_out, &ctx->qpsteps, &ctx->fupper, &ctx->probsteps, &ctx->routes, &ctx->psg_w, &ctx->psg_cost,
-                    &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen, &ctx->rrt_in};
+                    &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen, &ctx->rrt_in,
+                    &ctx->chk_in, &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr};
   for (DevBuf *b : bufs) free_buf(*b);
   if (ctx->dQblk) cudaFree(ctx->dQblk);
   double *ds[] = {ctx->dQQraw, ctx->dQQ, ctx->dG, ctx->dgn, ctx->dGI, ctx->dgnI, ctx->dlim, ctx->dumax, ctx->dworkL, ctx->dworkY};
@@ -303,6 +306,26 @@ static int upload_tables(cfs_ctx *ctx) {
   CU(cudaMemcpyAsync(ctx->dtab, &ctx->htab, sizeof(DevTables), cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return 0;
+}
+
+// Motion bound of the continuous checks: R[j] >= ||dp/dtheta_j|| for every link-axis endpoint p of the links l >= j, at every
+// theta.  Joint j turns everything downstream of it about an axis through its frame origin: the own translation contributes its
+// rotating part a_j (the constant part -- d_j along the axis, or robot.T on the 2L arm -- does not move), every later link at most
+// |a_i| + |(tx_i, ty_i, dz_i)|, the endpoint itself |cap|.  Triangle inequality; the same sums in the same order as
+// orc_motion_bound (tests/check_oracle.c).
+static void motion_bound(const DevTables &t, int nj, double R[CFS_MAXL]) {
+  for (int j = 0; j < CFS_MAXL; ++j) R[j] = 0.0;
+  for (int j = 0; j < nj; ++j) {
+    double reach = fabs(t.link[j].a);
+    for (int l = j; l < nj; ++l) {
+      const LinkTab &L = t.link[l];
+      if (l > j) reach = reach + (fabs(L.a) + sqrt((L.tx * L.tx + L.ty * L.ty) + L.dz * L.dz));
+      for (int k = 0; k < 2; ++k) {
+        const double c = sqrt((L.cap[k][0] * L.cap[k][0] + L.cap[k][1] * L.cap[k][1]) + L.cap[k][2] * L.cap[k][2]);
+        if (reach + c > R[j]) R[j] = reach + c;
+      }
+    }
+  }
 }
 
 extern "C" int cfs_set_robot(cfs_ctx *ctx, int robot_kind, const double *DH, int dh_rows, const double *base,
@@ -342,6 +365,7 @@ extern "C" int cfs_set_robot(cfs_ctx *ctx, int robot_kind, const double *DH, int
   t.dt = dt;
   t.kind = robot_kind;
   t.nj = n_joints;
+  motion_bound(t, n_joints, ctx->motion_R);
   ctx->nj = n_joints;
   ctx->have_robot = true;
   ctx->have_cost = false;  // n depends on nj
@@ -1489,6 +1513,146 @@ extern "C" int cfs_nodes_feasible(cfs_ctx *ctx, int N, const double *theta, unsi
   CU(launch_nodes_feasible(ctx->dtab, nj, ctx->nobs, N, ptr<double>(ctx->scratch_theta), d_feas, d_dmin, st));
   CU(cudaMemcpyAsync(feasible, d_feas, (size_t)N, cudaMemcpyDeviceToHost, st));
   if (dmin) CU(cudaMemcpyAsync(dmin, d_dmin, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  return 0;
+}
+
+// ---- continuous collision checks (k_check.cu) ------------------------------------------------------------------------
+static_assert(CHK_CLEAR == CFS_CHECK_CLEAR && CHK_HIT == CFS_CHECK_HIT && CHK_UNDECIDED == CFS_CHECK_UNDECIDED, "verdict codes");
+
+static int check_check_args(cfs_ctx *ctx, const char *who, int N, double eta, int margin_is_D, int max_evals) {
+  if (!ctx) return CFS_E_ARG;
+  int rc = check_ready(ctx, false);
+  if (rc) return rc;
+  if (N < 0) return fail(ctx, CFS_E_ARG, "%s: negative count %d", who, N);
+  if (!(eta > 0.0) || !std::isfinite(eta)) return fail(ctx, CFS_E_ARG, "%s: eta must be positive and finite (%g)", who, eta);
+  if (max_evals < 1) return fail(ctx, CFS_E_ARG, "%s: max_evals=%d", who, max_evals);
+  for (int j = 0; j < ctx->nobs; ++j) {
+    const double m = margin_is_D ? ctx->htab.obs[j].D : ctx->htab.obs[j].eps;
+    if (!(m - eta >= 1e-4))  // below it the touch rule (|d| < 1e-4) could fire inside the certified band
+      return fail(ctx, CFS_E_ARG, "%s: margin %g of obstacle %d minus eta %g is below 1e-4", who, m, j, eta);
+  }
+  return 0;
+}
+
+static CheckArgs check_base(cfs_ctx *ctx, int mode, int N, double eta, int margin_is_D, int max_evals) {
+  CheckArgs a;
+  memset(&a, 0, sizeof(a));
+  a.tab = ctx->dtab; a.mode = mode; a.N = N; a.nj = ctx->nj; a.nobs = ctx->nobs;
+  a.margin_is_D = margin_is_D ? 1 : 0; a.max_evals = max_evals; a.eta = eta;
+  for (int k = 0; k < CFS_MAXL; ++k) a.R[k] = ctx->motion_R[k];
+  a.counter = ptr<int>(ctx->chk_ctr);
+  return a;
+}
+
+static int check_edges_dev(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta, int margin_is_D,
+                           int max_evals, int *verdict, double *s_hit, double *cmin, int *evals) {
+  int rc;
+  if ((rc = ensure(ctx, ctx->chk_ctr, 64))) return rc;
+  CheckArgs a = check_base(ctx, 0, N, eta, margin_is_D, max_evals);
+  a.theta_a = theta_a; a.theta_b = theta_b;
+  a.verdict = verdict; a.s_hit = s_hit; a.cmin = cmin; a.evals = evals;
+  CU(launch_check(a, ctx->device, ctx->stream));
+  return 0;
+}
+
+static int check_traj_dev(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u, double eta,
+                          int margin_is_D, int max_evals, int *verdict, double *t_hit, double *cmin, int *evals) {
+  int rc;
+  const size_t S = (size_t)B * H;
+  if ((rc = ensure(ctx, ctx->chk_ctr, 64))) return rc;
+  if ((rc = ensure(ctx, ctx->chk_seg, (2 * sizeof(double) + 2 * sizeof(int)) * S + 64))) return rc;
+  double *ss = ptr<double>(ctx->chk_seg), *sc = ss + S;
+  int *sv = reinterpret_cast<int *>(sc + S), *se = sv + S;
+  CheckArgs a = check_base(ctx, 1, (int)S, eta, margin_is_D, max_evals);
+  a.H = H; a.x0 = x0; a.x = x; a.u = u;
+  a.verdict = sv; a.s_hit = ss; a.cmin = sc; a.evals = se;
+  CU(launch_check(a, ctx->device, ctx->stream));
+  CU(launch_check_reduce(B, H, ctx->htab.dt, sv, ss, sc, se, verdict, t_hit, cmin, evals, ctx->stream));
+  return 0;
+}
+
+extern "C" int cfs_check_edges_device(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta,
+                                      int margin_is_D, int max_evals, int *verdict, double *s_hit, double *cmin, int *evals,
+                                      int sync) {
+  int rc = check_check_args(ctx, "cfs_check_edges", N, eta, margin_is_D, max_evals);
+  if (rc) return rc;
+  if (N == 0) return 0;
+  if (!theta_a || !theta_b || !verdict || !s_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_edges_device: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  if ((rc = check_edges_dev(ctx, N, theta_a, theta_b, eta, margin_is_D, max_evals, verdict, s_hit, cmin, evals))) return rc;
+  if (sync) CU(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int cfs_check_edges(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta, int margin_is_D,
+                               int max_evals, int *verdict, double *s_hit, double *cmin, int *evals) {
+  int rc = check_check_args(ctx, "cfs_check_edges", N, eta, margin_is_D, max_evals);
+  if (rc) return rc;
+  if (N == 0) return 0;
+  if (!theta_a || !theta_b || !verdict || !s_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_edges: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  const int nj = ctx->nj;
+  cudaStream_t st = ctx->stream;
+  if ((rc = ensure(ctx, ctx->chk_in, sizeof(double) * 2 * (size_t)nj * N))) return rc;
+  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)N + 64))) return rc;
+  double *d_a = ptr<double>(ctx->chk_in), *d_b = d_a + (size_t)nj * N;
+  double *d_s = ptr<double>(ctx->chk_out), *d_c = d_s + N;
+  int *d_v = reinterpret_cast<int *>(d_c + N), *d_e = d_v + N;
+  CU(cudaMemcpyAsync(d_a, theta_a, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d_b, theta_b, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
+  if ((rc = check_edges_dev(ctx, N, d_a, d_b, eta, margin_is_D, max_evals, d_v, d_s, d_c, d_e))) return rc;
+  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(s_hit, d_s, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  if (evals) CU(cudaMemcpyAsync(evals, d_e, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  return 0;
+}
+
+static int check_traj_args(cfs_ctx *ctx, const char *who, int B, int H, double eta, int margin_is_D, int max_evals) {
+  int rc = check_check_args(ctx, who, B, eta, margin_is_D, max_evals);
+  if (rc) return rc;
+  if (H < 1) return fail(ctx, CFS_E_ARG, "%s: H=%d", who, H);
+  if ((long long)B * H > 0x7fffffffLL) return fail(ctx, CFS_E_ARG, "%s: B*H=%lld segments", who, (long long)B * H);
+  return 0;
+}
+
+extern "C" int cfs_check_trajectories_device(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u,
+                                             double eta, int margin_is_D, int max_evals, int *verdict, double *t_hit,
+                                             double *cmin, int *evals, int sync) {
+  int rc = check_traj_args(ctx, "cfs_check_trajectories", B, H, eta, margin_is_D, max_evals);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  if (!x0 || !x || !u || !verdict || !t_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_trajectories_device: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  if ((rc = check_traj_dev(ctx, B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin, evals))) return rc;
+  if (sync) CU(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int cfs_check_trajectories(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u, double eta,
+                                      int margin_is_D, int max_evals, int *verdict, double *t_hit, double *cmin, int *evals) {
+  int rc = check_traj_args(ctx, "cfs_check_trajectories", B, H, eta, margin_is_D, max_evals);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  if (!x0 || !x || !u || !verdict || !t_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_trajectories: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  const size_t nj = ctx->nj, nx0 = 2 * nj * B, nx = 2 * nj * H * B, nu = nj * H * B;
+  cudaStream_t st = ctx->stream;
+  if ((rc = ensure(ctx, ctx->chk_in, sizeof(double) * (nx0 + nx + nu)))) return rc;
+  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)B + 64))) return rc;
+  double *d_x0 = ptr<double>(ctx->chk_in), *d_x = d_x0 + nx0, *d_u = d_x + nx;
+  double *d_t = ptr<double>(ctx->chk_out), *d_c = d_t + B;
+  int *d_v = reinterpret_cast<int *>(d_c + B), *d_e = d_v + B;
+  CU(cudaMemcpyAsync(d_x0, x0, sizeof(double) * nx0, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d_x, x, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d_u, u, sizeof(double) * nu, cudaMemcpyHostToDevice, st));
+  if ((rc = check_traj_dev(ctx, B, H, d_x0, d_x, d_u, eta, margin_is_D, max_evals, d_v, d_t, d_c, d_e))) return rc;
+  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(t_hit, d_t, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
+  if (evals) CU(cudaMemcpyAsync(evals, d_e, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return 0;
 }

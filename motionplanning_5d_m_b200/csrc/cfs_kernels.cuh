@@ -39,6 +39,26 @@ cudaError_t launch_nodes_feasible(const DevTables *tab, int nj, int nobs, int N,
 cudaError_t launch_nearest_steer(int nj, int n_nodes, const double *nodes, int S, const double *samples,
                                  const double *ratial, double step, int *parent, double *newnode, cudaStream_t s);
 
+// ---- continuous collision checks of edges / trajectory segments (k_check.cu) ------------------------------------------------
+enum { CHK_CLEAR = 0, CHK_HIT = 1, CHK_UNDECIDED = 2 };  // = CFS_CHECK_* of include/cfs_b200.h
+struct CheckArgs {
+  const DevTables *tab;
+  int mode;                        // 0: edges, 1: trajectory segments (item = b*H + k)
+  int N, H, nj, nobs, margin_is_D, max_evals;
+  double eta;
+  double R[CFS_MAXL];              // motion bound per joint (cfs_set_robot); a kernel argument, not part of DevTables
+  const double *theta_a, *theta_b; // mode 0: nj x N
+  const double *x0, *x, *u;        // mode 1: 2nj x B, 2njH x B, njH x B
+  int *verdict;                    // per item
+  double *s_hit, *cmin;
+  int *evals;                      // per item, may be nullptr
+  int *counter;                    // work queue head (zeroed by launch_check)
+};
+cudaError_t launch_check(const CheckArgs &a, int device, cudaStream_t s);
+// per-segment results (B*H each) -> per-trajectory verdict, t_hit, cmin, evals (evals may be nullptr)
+cudaError_t launch_check_reduce(int B, int H, double dt, const int *sv, const double *ss, const double *sc, const int *se,
+                                int *verdict, double *t_hit, double *cmin, int *evals, cudaStream_t s);
+
 // work order of the fused solver (longest expected problems first): order[] = problems by descending number of reference
 // waypoints inside an obstacle margin; count[] is scratch (B ints each)
 cudaError_t launch_work_order(const DevTables *tab, int nj, int nobs, int B, int H, const double *xref, int margin_is_D,

@@ -107,11 +107,35 @@ def rrtstar_sys_info(robot, x0, goal_th, ratial, nstate=5):
                 ratial=np.asarray(ratial, dtype=np.float64), goal_th=np.asarray(goal_th, dtype=np.float64))
 
 
-def rrtstar_cfs(ctx, robot, scene=None, ROBOT="M200i", num_seed=6, horizon=40, rng=None, smooth_all=False, nrnd=NRND_DEFAULT):
+def route_edges(routes, route_len):
+    """Routes (S, W, nj), the first route_len[s] waypoints of route s valid, -> the edges of their polylines:
+    theta_a, theta_b (E, nj) and the route each edge belongs to (E,), ready for Context.check_edges."""
+    routes = np.asarray(routes, dtype=np.float64)
+    rl = np.minimum(np.maximum(np.asarray(route_len).reshape(-1), 0), routes.shape[1])
+    owner = np.repeat(np.arange(routes.shape[0]), np.maximum(rl - 1, 0))
+    k = np.concatenate([np.arange(max(n - 1, 0)) for n in rl]).astype(np.int64) if rl.size else np.zeros(0, dtype=np.int64)
+    return (np.ascontiguousarray(routes[owner, k]), np.ascontiguousarray(routes[owner, k + 1]), owner)
+
+
+def combine_verdicts(verdict, owner, n):
+    """Per-group verdict of item verdicts: HIT if any item hits, else UNDECIDED if any is, else CLEAR; -1 for a group without
+    items (a seed without a route)."""
+    out = np.full(n, -1, dtype=np.int32)
+    for code in (_lib.CHECK_CLEAR, _lib.CHECK_UNDECIDED, _lib.CHECK_HIT):
+        out[np.unique(owner[verdict == code])] = code
+    return out
+
+
+def rrtstar_cfs(ctx, robot, scene=None, ROBOT="M200i", num_seed=6, horizon=40, rng=None, smooth_all=False, nrnd=NRND_DEFAULT,
+                check=False):
     """RRTstar_CFS.m end to end on the device: s_Parallel_rrt (:76) -> cubicpolytraj resampling to horizon+1 points (:96-100)
     -> CFS stage set-up (:106-187: R*10, Q_v = [100 20 1 1 1]) -> CFS_FANUC.optimizer (:194-195).
     smooth_all=False: the reference's flow (the shortest route is smoothed).  smooth_all=True: every seed's route is smoothed in
-    one batch and the cheapest trajectory wins (the multi-GPU best-of, multi_gpu.best_of, continues this over ranks)."""
+    one batch and the cheapest trajectory wins (the multi-GPU best-of, multi_gpu.best_of, continues this over ranks).
+    check=True (extension, include/cfs_b200.h cfs_check_*): continuous collision checks with the default tolerance against
+    obs{j}.D -- route_check = per-seed verdict of the route polyline (-1: no route), traj_check = the check of every smoothed
+    trajectory; with smooth_all the winner is the cheapest CLEAR trajectory, or the cheapest one if none is CLEAR, and clear says
+    which."""
     sc = scene or SCENE_RRTSTAR
     s = rrtstar_sys_info(robot, sc["x0"], sc["goal"], sc["ratial"])
     par = s_Parallel_rrt(sc["obs"], s, sc["goal"], sc["region_g"], sc["region_s"], sc["sample_off"], ROBOT, "RRT", num_seed, ctx=ctx,
@@ -131,8 +155,38 @@ def rrtstar_cfs(ctx, robot, scene=None, ROBOT="M200i", num_seed=6, horizon=40, r
         ok = (sol["status"] & 0xFF) < 2
         fin = np.where(ok & (sol["iters"] > 0), sol["cost_hist"][np.arange(num_seed), np.maximum(sol["iters"], 1) - 1], np.inf)
         win = int(np.argmin(fin))
-        return dict(rrt=par, sol=sol, winner=win, cost=float(fin[win]), x=sol["x"][win], u=sol["u"][win])
+        if not check:
+            return dict(rrt=par, sol=sol, winner=win, cost=float(fin[win]), x=sol["x"][win], u=sol["u"][win])
+        route_check = _check_routes(ctx, routes, rl)
+        traj = _check_smoothed(ctx, routes[:, 0], sol)
+        clear = (traj["verdict"] == _lib.CHECK_CLEAR) & np.isfinite(fin)
+        if clear.any():
+            win = int(np.argmin(np.where(clear, fin, np.inf)))
+        return dict(rrt=par, sol=sol, winner=win, cost=float(fin[win]), x=sol["x"][win], u=sol["u"][win], route_check=route_check,
+                    traj_check=traj, clear=bool(clear[win]))
     sol = ctx.solve_routes(par["route"].T[None], 0.1, 20)
     it = int(sol["iters"][0])
-    return dict(rrt=par, sol=sol, winner=par["id"], cost=float(sol["cost_hist"][0, it - 1]) if it else np.inf, x=sol["x"][0],
-                u=sol["u"][0])
+    out = dict(rrt=par, sol=sol, winner=par["id"], cost=float(sol["cost_hist"][0, it - 1]) if it else np.inf, x=sol["x"][0],
+               u=sol["u"][0])
+    if check:
+        rl = np.array([len(r) for r in par["routes"]], dtype=np.int32)
+        rl[par["fail"]] = 0
+        routes = np.zeros((num_seed, max(int(rl.max()), 2), 5))
+        for k, r in enumerate(par["routes"]):
+            routes[k, :rl[k]] = r[:rl[k]]
+        traj = _check_smoothed(ctx, par["route"].T[:1], sol)
+        out.update(route_check=_check_routes(ctx, routes, rl), traj_check=traj,
+                   clear=bool(traj["verdict"][0] == _lib.CHECK_CLEAR))
+    return out
+
+
+def _check_routes(ctx, routes, route_len):
+    ta, tb, owner = route_edges(routes, route_len)
+    ev = ctx.check_edges(ta, tb) if owner.size else dict(verdict=np.zeros(0, dtype=np.int32))
+    return combine_verdicts(ev["verdict"], owner, routes.shape[0])
+
+
+def _check_smoothed(ctx, first, sol):
+    """first (B, nj): the first waypoint of every route, which is the first resampled point and so x0 = [first; 0]"""
+    x0 = np.concatenate([first, np.zeros_like(first)], axis=1)
+    return ctx.check_trajectories(x0, sol["x"], sol["u"])
