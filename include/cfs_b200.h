@@ -236,6 +236,50 @@ int cfs_check_edges_device(cfs_ctx *ctx, int N, const double *theta_a, const dou
 int cfs_check_trajectories_device(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u, double eta,
                                   int margin_is_D, int max_evals, int *verdict, double *t_hit, double *cmin, int *evals,
                                   int sync);
+
+/* ---- per-waypoint margin offsets and the checked solve ----
+ * cfs_solve_batch_margins: cfs_solve_batch plus margin_off (nobs x H per problem: element (b nobs + j) H + (i - 1) for
+ * waypoint i = 1..H, the [prob][obs][i] order; NULL = no offsets).  The obstacle row of (obstacle j, waypoint i) becomes
+ * dist - (m_j + margin_off) instead of dist - m_j (m_j = epsilon for CFS, D for PSGCFS); nothing else changes, and all-zero
+ * offsets give bit for bit the result of cfs_solve_batch.  Entries must be finite and >= 0 (CFS_E_ARG).  The _device form checks
+ * them on the device and synchronises once for that.  Uses: time-varying clearance, and the repair of cfs_solve_checked.
+ *
+ * cfs_solve_checked: a solve whose trajectories come back with a continuous collision check, after repairing the ones that
+ * cut an obstacle margin between waypoints (CFS constrains the waypoints only).  The check margin is the solver's (epsilon for
+ * CFS, D for PSGCFS); eta, max_evals as in cfs_check_trajectories (same argument rules); rounds >= 0; gain > 0 and finite.
+ *   Round 0 is exactly cfs_solve_batch_device followed by cfs_check_trajectories_device.
+ *   After each check, every problem whose current verdict is HIT and whose status low byte is < 2 gets, for each HIT segment k
+ *   with witness theta* (the point where the check found c < -eta/2) and each obstacle j with clearance c_j(theta*) < -eta/2,
+ *   inc = gain (eta - c_j) at waypoints k and k+1 (those in 1..H; waypoint 0 is x0); a waypoint between two HIT segments gets
+ *   the larger increment, not the sum.  The increments add to its offsets (starting at 0).
+ *   Round r = 1..rounds re-solves those problems from the caller's original xref with their accumulated offsets.  A candidate
+ *   whose status low byte is < 2 replaces the problem's solution and is checked again; a failed one (INFEASIBLE / NUMERICAL)
+ *   leaves the previous solution, and the problem stops repairing.  Problems with status >= 2 after round 0 are returned as
+ *   round 0 left them.  The loop ends after `rounds` rounds or when no problem is left to repair.
+ * Outputs: u, x, cost_hist, e_u_hist (may be NULL), iters, status of the returned solution; verdict, t_hit, cmin of its check;
+ * rounds_used = the round that produced it (0 = the first solve); margin_off (may be NULL): the offsets that returned solution
+ * was solved with (0 where rounds_used is 0), so cfs_solve_batch_margins with them reproduces it.  A CLEAR verdict carries the
+ * guarantee of cfs_check_trajectories.
+ * Each round reads one count back from the device, and the statistics of round 0 are collected, so the _device form
+ * synchronises after round 0 and once per round.  cfs_get_stats describes round 0's solve.  The host form is synchronous. */
+int cfs_solve_batch_margins(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
+                            const double *xref, const double *noise, const double *margin_off /*nobs H x B or NULL*/,
+                            double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                            double *e_u_hist, int *iters, int *status);
+int cfs_solve_batch_margins_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                   const double *caug, const double *xref, const double *noise, const double *margin_off,
+                                   double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                                   double *e_u_hist, int *iters, int *status, int sync);
+int cfs_solve_checked(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
+                      const double *xref, const double *noise, double eps_outer, int max_outer, double alpha, double eta,
+                      int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
+                      int *iters, int *status, int *verdict /*B*/, double *t_hit /*B*/, double *cmin /*B*/,
+                      int *rounds_used /*B*/, double *margin_off /*nobs H x B or NULL*/);
+int cfs_solve_checked_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
+                             const double *xref, const double *noise, double eps_outer, int max_outer, double alpha, double eta,
+                             int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
+                             int *iters, int *status, int *verdict, double *t_hit, double *cmin, int *rounds_used,
+                             double *margin_off, int sync);
 /* RRT_FANUC.getRandNode nearest scan + steer (Lib/RRT_FANUC.m:116-129) for S samples against one tree:
  * parent[s] = argmin_i ||(nodes(:,i)-sample(:,s)).*ratial|| (first minimum, 0-based), newnode = parent + (sample-parent)*step/||parent-sample||. */
 int cfs_nearest_steer(cfs_ctx *ctx, int n_nodes, const double *nodes /*nj x n_nodes*/, int S, const double *samples /*nj x S*/,

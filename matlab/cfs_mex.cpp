@@ -22,6 +22,14 @@
 //     cubicpolytraj resampling to sys_info.H + 1 points, cost set-up from its blocks (Q 2nj x 2nj, Rblk nj x nj, R*r_scale),
 //     CFS_FANUC.optimizer.  sys_info.{H, njoint, robot, lim, MAX_input, epsilon_O, MAX_O_ITER}.
 //
+//   [u, x_, cost_all, e_u_all, iters, status, verdict, t_hit, cmin, rounds_used, margin_off] =
+//       cfs_mex('solve_checked', solver, grad, ROBOT, obs, sys_info [, noise [, eta, rounds, gain]])
+//     'solve' followed by a continuous collision check of every trajectory and up to `rounds` re-solves of the HIT ones with
+//     raised per-waypoint margins (extension; include/cfs_b200.h cfs_solve_checked).  solver 'CFS' | 'PSGCFS'; noise may be [];
+//     eta = 1e-3, rounds = 4, gain = 2 by default.  verdict (1 x B int32: 0 clear, 1 hit, 2 undecided), t_hit, cmin (1 x B),
+//     rounds_used (1 x B int32, 0 = the first solve), margin_off (H*nobs x B: reshape(margin_off(:, b), H, nobs) are the
+//     offsets the returned solution of problem b was solved with).
+//
 //   [verdict, s_hit, cmin, evals] = cfs_mex('check', ROBOT, obs, sys_info, 'edges', A, B [, eta, margin_is_D])
 //   [verdict, t_hit, cmin, evals] = cfs_mex('check', ROBOT, obs, sys_info, 'trajectory', x0, x_, u [, eta, margin_is_D])
 //     continuous collision checks (extension; include/cfs_b200.h cfs_check_edges / cfs_check_trajectories): the edges
@@ -175,9 +183,13 @@ static void out_int(mxArray *&dst, const std::vector<int> &v) {
 }
 
 // ---- 'solve' ------------------------------------------------------------------------------------------------------------------
-static void cmd_solve(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
-  if (nrhs < 5) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex('solve', solver, grad, ROBOT, obs, sys_info [, noise | uu])");
+// checked: the 'solve_checked' command (cfs_solve_checked), prhs[6..8] = eta, rounds, gain (optional)
+static void cmd_solve(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[], bool checked = false) {
+  if (nrhs < 5)
+    mexErrMsgIdAndTxt("cfs:arg", checked ? "usage: cfs_mex('solve_checked', solver, grad, ROBOT, obs, sys_info [, noise [, eta, rounds, gain]])"
+                                         : "usage: cfs_mex('solve', solver, grad, ROBOT, obs, sys_info [, noise | uu])");
   const std::string solver = str(prhs[0]), grad = str(prhs[1]), robot_name = str(prhs[2]);
+  if (checked && solver == "CHOMP") mexErrMsgIdAndTxt("cfs:arg", "solve_checked: solver '%s' (CFS | PSGCFS)", solver.c_str());
   if (solver != "CFS" && solver != "PSGCFS" && solver != "CHOMP")
     mexErrMsgIdAndTxt("cfs:arg", "solver '%s' (CFS | PSGCFS | CHOMP)", solver.c_str());
   const bool chomp = solver == "CHOMP";
@@ -234,6 +246,26 @@ static void cmd_solve(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]
   mxArray *x = mxCreateDoubleMatrix(2 * n, B, mxREAL), *cost = mxCreateDoubleMatrix(K > 0 ? K : 1, B, mxREAL),
           *eu = mxCreateDoubleMatrix(K > 0 ? K : 1, B, mxREAL);
   mxArray *it = mxCreateNumericMatrix(1, B, mxINT32_CLASS, mxREAL), *st = mxCreateNumericMatrix(1, B, mxINT32_CLASS, mxREAL);
+  if (checked) {
+    auto opt = [&](int i, double def, const char *what) {
+      return (nrhs > i && prhs[i] && !mxIsEmpty(prhs[i])) ? scalar(prhs[i], what) : def;
+    };
+    const double eta = opt(6, 1e-3, "eta"), gain = opt(8, 2.0, "gain");
+    const int rounds = (int)opt(7, 4.0, "rounds");
+    const size_t OH = mxGetNumberOfElements(obs) * (size_t)H;
+    mxArray *vd = mxCreateNumericMatrix(1, B, mxINT32_CLASS, mxREAL), *th = mxCreateDoubleMatrix(1, B, mxREAL),
+            *cm = mxCreateDoubleMatrix(1, B, mxREAL), *ru = mxCreateNumericMatrix(1, B, mxINT32_CLASS, mxREAL),
+            *mo = mxCreateDoubleMatrix(OH, B, mxREAL);
+    check(cfs_solve_checked(g_ctx, (int)B, psg ? CFS_SOLVER_PSGCFS : CFS_SOLVER_CFS, grad == "derivest" ? CFS_GRAD_DERIVEST : CFS_GRAD_NUMJAC,
+                            x0.data(), mxGetPr(ff), mxGetPr(caug), mxGetPr(xref), noise, scalar(field(si, "epsilon_O"), "sys_info.epsilon_O"),
+                            K, alpha ? scalar(alpha, "sys_info.alpha") : 0.0, eta, 4096, rounds, gain, mxGetPr(plhs[0]), mxGetPr(x),
+                            mxGetPr(cost), mxGetPr(eu), (int *)mxGetData(it), (int *)mxGetData(st), (int *)mxGetData(vd), mxGetPr(th),
+                            mxGetPr(cm), (int *)mxGetData(ru), OH ? mxGetPr(mo) : nullptr),
+          "cfs_solve_checked");
+    mxArray *outs[11] = {plhs[0], x, cost, eu, it, st, vd, th, cm, ru, mo};
+    for (int k = 1; k < 11 && k < nlhs; ++k) plhs[k] = outs[k];
+    return;
+  }
   if (chomp) {
     if (!alpha) mexErrMsgIdAndTxt("cfs:arg", "CHOMP needs sys_info.alpha");
     check(cfs_chomp_batch(g_ctx, (int)B, x0.data(), mxGetPr(ff), mxGetPr(caug), mxGetPr(xref), noise, scalar(alpha, "sys_info.alpha"), K,
@@ -398,7 +430,7 @@ static void cmd_check(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]
 }
 
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
-  if (nrhs < 1) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex(command, ...); commands: solve, rrt, routes, check, device");
+  if (nrhs < 1) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex(command, ...); commands: solve, solve_checked, rrt, routes, check, device");
   const std::string cmd = str(prhs[0]);
   if (cmd == "device") {
     if (nrhs < 2) mexErrMsgIdAndTxt("cfs:arg", "usage: cfs_mex('device', id)");
@@ -411,6 +443,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
   if (cmd == "rrt") return cmd_rrt(nlhs, plhs, nrhs - 1, prhs + 1);
   if (cmd == "routes") return cmd_routes(nlhs, plhs, nrhs - 1, prhs + 1);
   if (cmd == "check") return cmd_check(nlhs, plhs, nrhs - 1, prhs + 1);
+  if (cmd == "solve_checked") return cmd_solve(nlhs, plhs, nrhs - 1, prhs + 1, true);
   if (cmd == "CFS" || cmd == "PSGCFS" || cmd == "CHOMP") return cmd_solve(nlhs, plhs, nrhs, prhs);  // short calling form
-  mexErrMsgIdAndTxt("cfs:arg", "unknown command '%s' (solve | rrt | routes | check | device)", cmd.c_str());
+  mexErrMsgIdAndTxt("cfs:arg", "unknown command '%s' (solve | solve_checked | rrt | routes | check | device)", cmd.c_str());
 }

@@ -22,7 +22,8 @@ CHECK_CLEAR, CHECK_HIT, CHECK_UNDECIDED = 0, 1, 2
 SYMBOLS = ["cfs_create", "cfs_destroy", "cfs_last_error", "cfs_version", "cfs_set_stream", "cfs_set_option", "cfs_set_robot", "cfs_set_obstacles", "cfs_set_obstacles_ex",
            "cfs_set_cost", "cfs_set_cost_blocks", "cfs_solve_start_goal", "cfs_solve_start_goal_async", "cfs_solve_routes", "cfs_solve_routes_async", "cfs_solve_routes_var", "cfs_solve_routes_var_async", "cfs_solve_routes_device", "cfs_resample_routes", "cfs_solve_batch", "cfs_solve_batch_async", "cfs_chomp_batch", "cfs_wait", "cfs_solve_batch_device", "cfs_dist_grad", "cfs_time_dist_grad", "cfs_get_con",
            "cfs_nodes_feasible", "cfs_nearest_steer", "cfs_rrt_find_routes", "cfs_rrt_find_routes_device", "cfs_get_stats", "cfs_set_timing", "cfs_get_iter_times", "cfs_get_problem_steps", "cfs_get_qp_profile", "cfs_get_warp_profile", "cfs_measure_fp64_peak",
-           "cfs_check_edges", "cfs_check_trajectories", "cfs_check_edges_device", "cfs_check_trajectories_device"]
+           "cfs_check_edges", "cfs_check_trajectories", "cfs_check_edges_device", "cfs_check_trajectories_device",
+           "cfs_solve_batch_margins", "cfs_solve_batch_margins_device", "cfs_solve_checked", "cfs_solve_checked_device"]
 
 
 class CfsError(RuntimeError):
@@ -262,6 +263,74 @@ class Context:
                                        _dp(out["iters"]), _dp(out["status"]))
         self._check(rc, "cfs_solve_batch")
         return out
+
+    def solve_batch_margins(self, x0, ff, caug, xref, margin_off, eps_outer, max_outer, solver=SOLVER_CFS, grad=GRAD_NUMJAC,
+                            noise=None, alpha=0.0):
+        """solve_batch with per-waypoint margin offsets margin_off (B, nobs, H) or None (cfs_solve_batch_margins): the obstacle
+        row of (j, i) uses dist - (margin_j + margin_off[b, j, i - 1])."""
+        x0, ff, caug, xref = _f64(x0), _f64(ff), _f64(caug), _f64(xref)
+        B = x0.shape[0]
+        if not getattr(self, "n", 0):
+            raise CfsError("cost not set (cfs_set_cost)")
+        n, N = self.n, 2 * self.n
+        assert x0.shape == (B, 2 * self.nj) and ff.shape == (B, n) and xref.shape == (B, N) and caug.shape == (B,)
+        off = None if margin_off is None else _f64(margin_off).reshape(B, self.nobs * self.H)
+        nz = None if noise is None else _f64(noise)
+        out = dict(u=np.empty((B, n)), x=np.empty((B, N)), cost_hist=np.empty((B, max_outer)), e_u_hist=np.empty((B, max_outer)),
+                   iters=np.empty(B, dtype=np.int32), status=np.empty(B, dtype=np.int32))
+        rc = self._lib.cfs_solve_batch_margins(self._h, C.c_int(B), C.c_int(solver), C.c_int(grad), _dp(x0), _dp(ff), _dp(caug),
+                                               _dp(xref), _dp(nz), _dp(off), C.c_double(eps_outer), C.c_int(max_outer),
+                                               C.c_double(alpha), _dp(out["u"]), _dp(out["x"]), _dp(out["cost_hist"]),
+                                               _dp(out["e_u_hist"]), _dp(out["iters"]), _dp(out["status"]))
+        self._check(rc, "cfs_solve_batch_margins")
+        return out
+
+    def solve_checked(self, x0, ff, caug, xref, eps_outer, max_outer, eta=1e-3, rounds=4, gain=2.0, max_evals=4096,
+                      solver=SOLVER_CFS, grad=GRAD_NUMJAC, noise=None, alpha=0.0):
+        """Checked solve (cfs_solve_checked): the solve, a continuous check of every trajectory, and up to `rounds` re-solves of
+        the HIT ones with raised per-waypoint margins.  Returns the solve's dict plus verdict, t_hit, cmin, rounds_used (B,) and
+        margin_off (B, nobs, H)."""
+        x0, ff, caug, xref = _f64(x0), _f64(ff), _f64(caug), _f64(xref)
+        B = x0.shape[0]
+        if not getattr(self, "n", 0):
+            raise CfsError("cost not set (cfs_set_cost)")
+        n, N = self.n, 2 * self.n
+        assert x0.shape == (B, 2 * self.nj) and ff.shape == (B, n) and xref.shape == (B, N) and caug.shape == (B,)
+        nz = None if noise is None else _f64(noise)
+        out = dict(u=np.empty((B, n)), x=np.empty((B, N)), cost_hist=np.empty((B, max_outer)), e_u_hist=np.empty((B, max_outer)),
+                   iters=np.empty(B, dtype=np.int32), status=np.empty(B, dtype=np.int32), verdict=np.empty(B, dtype=np.int32),
+                   t_hit=np.empty(B), cmin=np.empty(B), rounds_used=np.empty(B, dtype=np.int32),
+                   margin_off=np.zeros((B, self.nobs, self.H)))
+        rc = self._lib.cfs_solve_checked(self._h, C.c_int(B), C.c_int(solver), C.c_int(grad), _dp(x0), _dp(ff), _dp(caug), _dp(xref),
+                                         _dp(nz), C.c_double(eps_outer), C.c_int(max_outer), C.c_double(alpha), C.c_double(eta),
+                                         C.c_int(max_evals), C.c_int(rounds), C.c_double(gain), _dp(out["u"]), _dp(out["x"]),
+                                         _dp(out["cost_hist"]), _dp(out["e_u_hist"]), _dp(out["iters"]), _dp(out["status"]),
+                                         _dp(out["verdict"]), _dp(out["t_hit"]), _dp(out["cmin"]), _dp(out["rounds_used"]),
+                                         _dp(out["margin_off"]))
+        self._check(rc, "cfs_solve_checked")
+        return out
+
+    def solve_batch_margins_ptr(self, B, x0, ff, caug, xref, margin_off, eps_outer, max_outer, u, x, cost_hist, e_u_hist, iters,
+                                status, solver=SOLVER_CFS, grad=GRAD_NUMJAC, noise=0, alpha=0.0, sync=True):
+        """cfs_solve_batch_margins_device: every array argument a device pointer (int; margin_off, noise, e_u_hist may be 0)."""
+        vp = lambda p: C.c_void_p(p) if p else None
+        rc = self._lib.cfs_solve_batch_margins_device(self._h, C.c_int(B), C.c_int(solver), C.c_int(grad), vp(x0), vp(ff), vp(caug),
+                                                      vp(xref), vp(noise), vp(margin_off), C.c_double(eps_outer), C.c_int(max_outer),
+                                                      C.c_double(alpha), vp(u), vp(x), vp(cost_hist), vp(e_u_hist), vp(iters),
+                                                      vp(status), C.c_int(1 if sync else 0))
+        self._check(rc, "cfs_solve_batch_margins_device")
+
+    def solve_checked_ptr(self, B, x0, ff, caug, xref, eps_outer, max_outer, u, x, cost_hist, e_u_hist, iters, status, verdict, t_hit,
+                          cmin, rounds_used, margin_off=0, eta=1e-3, rounds=4, gain=2.0, max_evals=4096, solver=SOLVER_CFS,
+                          grad=GRAD_NUMJAC, noise=0, alpha=0.0, sync=True):
+        """cfs_solve_checked_device: every array argument a device pointer (int; margin_off, noise, e_u_hist may be 0)."""
+        vp = lambda p: C.c_void_p(p) if p else None
+        rc = self._lib.cfs_solve_checked_device(self._h, C.c_int(B), C.c_int(solver), C.c_int(grad), vp(x0), vp(ff), vp(caug),
+                                                vp(xref), vp(noise), C.c_double(eps_outer), C.c_int(max_outer), C.c_double(alpha),
+                                                C.c_double(eta), C.c_int(max_evals), C.c_int(rounds), C.c_double(gain), vp(u), vp(x),
+                                                vp(cost_hist), vp(e_u_hist), vp(iters), vp(status), vp(verdict), vp(t_hit), vp(cmin),
+                                                vp(rounds_used), vp(margin_off), C.c_int(1 if sync else 0))
+        self._check(rc, "cfs_solve_checked_device")
 
     def chomp_batch(self, x0, ff, caug, xref, u_init, alpha, max_outer):
         """CHOMP_FANUC.optimizer (Lib/CHOMP_FANUC.m:54-165) for B problems: x0 (B,2nj), ff (B,n), caug (B,), xref (B,2njH),

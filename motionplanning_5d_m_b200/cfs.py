@@ -57,7 +57,10 @@ class _SolverBase:
         ctx.set_cost(s["H"], s["QQ"], s.get("lim"), s.get("MAX_input") if self.SOLVER == _lib.SOLVER_CFS else None)
         return ctx
 
-    def optimizer(self, noise=None, rng=None):
+    def optimizer(self, noise=None, rng=None, check=None):
+        """check=None: the reference's optimizer.  check=dict(eta=1e-3, rounds=4, gain=2.0, max_evals=4096) (any subset): the
+        checked solve (Context.solve_checked); the result then also carries verdict, t_hit, cmin, rounds_used and margin_off
+        (nobs x H) of the returned trajectory."""
         s = self.sys_info
         ctx = self._context()
         K = int(s["MAX_O_ITER"])
@@ -66,11 +69,15 @@ class _SolverBase:
             # deterministic method.  Drawn here with the reference's distribution, one row per outer iteration (all
             # MAX_O_ITER rows up front: the reference only draws when a step is taken, INTEGRATION.md).
             noise = (rng or np.random.default_rng()).normal(0.0, 0.1, size=(K, self.nn))
-        out = ctx.solve_batch(np.asarray(s["xR"], dtype=np.float64)[:, 0][None], np.asarray(s["ff"])[None],
-                              np.array([s["caug"]], dtype=np.float64), self.x_[None], float(s["epsilon_O"]), K,
-                              solver=self.SOLVER, grad=self.GRAD,
-                              noise=None if noise is None else np.asarray(noise, dtype=np.float64)[None],
-                              alpha=float(s.get("alpha", 0.0)))
+        solve = ctx.solve_batch if check is None else lambda *a, **kw: ctx.solve_checked(*a, **kw, **dict(check))
+        out = solve(np.asarray(s["xR"], dtype=np.float64)[:, 0][None], np.asarray(s["ff"])[None],
+                    np.array([s["caug"]], dtype=np.float64), self.x_[None], float(s["epsilon_O"]), K,
+                    solver=self.SOLVER, grad=self.GRAD,
+                    noise=None if noise is None else np.asarray(noise, dtype=np.float64)[None],
+                    alpha=float(s.get("alpha", 0.0)))
+        if check is not None:
+            self.verdict, self.t_hit, self.cmin = int(out["verdict"][0]), float(out["t_hit"][0]), float(out["cmin"][0])
+            self.rounds_used, self.margin_off = int(out["rounds_used"][0]), out["margin_off"][0].copy()
         it = int(out["iters"][0])
         self.u = out["u"][0].copy()
         self.x_ = out["x"][0].copy()
@@ -140,7 +147,12 @@ class BatchCFS:
         self.ctx.set_cost(sys_info["H"], sys_info["QQ"], sys_info.get("lim"),
                           sys_info.get("MAX_input") if solver == _lib.SOLVER_CFS else None)
 
-    def optimizer(self, x0, ff, caug, xref, noise=None):
+    def optimizer(self, x0, ff, caug, xref, noise=None, check=None):
+        """check=None: the plain batched solve.  check=dict(eta=1e-3, rounds=4, gain=2.0, max_evals=4096) (any subset): the
+        checked solve (Context.solve_checked), whose result adds verdict, t_hit, cmin, rounds_used and margin_off."""
         s = self.sys_info
+        if check is not None:
+            return self.ctx.solve_checked(x0, ff, caug, xref, float(s["epsilon_O"]), int(s["MAX_O_ITER"]), solver=self.solver,
+                                          grad=self.grad, noise=noise, alpha=float(s.get("alpha", 0.0)), **dict(check))
         return self.ctx.solve_batch(x0, ff, caug, xref, float(s["epsilon_O"]), int(s["MAX_O_ITER"]), solver=self.solver,
                                     grad=self.grad, noise=noise, alpha=float(s.get("alpha", 0.0)))

@@ -70,7 +70,7 @@ struct cfs_ctx {
   // batch buffers
   DevBuf x0, ff, caug, xref, noise, u, x, cost, eu, u0, v0, cost0, dist, grad, lid, iters, status, flags, listA, listB,
       counters, slab, scratch_theta, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen, rrt_in,
-      chk_in, chk_out, chk_seg, chk_ctr;
+      chk_in, chk_out, chk_seg, chk_ctr, rep_off, rep_offo, rep_in, rep_out, rep_list;
   int slab_grid = 0, slab_ld = 0;
   // pinned staging of the host-pointer entries: pageable caller buffers (MATLAB's mxGetPr memory, numpy arrays) are copied
   // through these so that cudaMemcpyAsync stays asynchronous; pinned / registered caller buffers are used in place
@@ -274,7 +274,8 @@ extern "C" void cfs_destroy(cfs_ctx *ctx) {
                     &ctx->flags, &ctx->listA, &ctx->listB, &ctx->counters, &ctx->slab, &ctx->scratch_theta,
                     &ctx->scratch_out, &ctx->qpsteps, &ctx->fupper, &ctx->probsteps, &ctx->routes, &ctx->psg_w, &ctx->psg_cost,
                     &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen, &ctx->rrt_in,
-                    &ctx->chk_in, &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr};
+                    &ctx->chk_in, &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr, &ctx->rep_off, &ctx->rep_offo, &ctx->rep_in,
+                    &ctx->rep_out, &ctx->rep_list};
   for (DevBuf *b : bufs) free_buf(*b);
   if (ctx->dQblk) cudaFree(ctx->dQblk);
   double *ds[] = {ctx->dQQraw, ctx->dQQ, ctx->dG, ctx->dgn, ctx->dGI, ctx->dgnI, ctx->dlim, ctx->dumax, ctx->dworkL, ctx->dworkY};
@@ -516,7 +517,8 @@ static int check_ready(cfs_ctx *ctx, bool need_cost) {
 // ---- the solve, device pointers --------------------------------------------------------------------------------------
 static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
                         const double *caug, const double *xref, const double *noise, double eps_outer, int max_outer,
-                        double alpha, double *u, double *x, double *cost_hist, double *e_u_hist, int *iters, int *status) {
+                        double alpha, double *u, double *x, double *cost_hist, double *e_u_hist, int *iters, int *status,
+                        const double *margin_off = nullptr) {
   const int nj = ctx->nj, H = ctx->H, n = ctx->n, np = 3 * n, O = ctx->nobs, OH = O * H;
   cudaStream_t st = ctx->stream;
   const bool psg = solver == CFS_SOLVER_PSGCFS;
@@ -578,6 +580,7 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
   a.prob_steps = ptr<int>(ctx->probsteps);
   a.prof = ctx->timing_level >= 3 ? ptr<long long>(ctx->qpsteps) + 8 : nullptr;
   a.slab_ld = n;
+  a.margin_off = O > 0 ? margin_off : nullptr;  // non-null selects the offset instantiations of every solver kernel
 
   const bool fused = ctx->use_fused && !psg && grad == CFS_GRAD_NUMJAC && fused_supported(a);
   // bulk tier of the fused solver: one warp per problem (k_warp.cu) when its shared-memory regions fit
@@ -587,7 +590,8 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
   if (fused && ctx->use_warp) {
     // direction slots in shared memory: the count that keeps the most problems resident per SM (ties: more slots); cached per
     // (n, obstacles, CTA shape)
-    const long long key = ((long long)n << 24) ^ ((long long)O << 16) ^ ((long long)ctx->warp_cfg << 8) ^ ctx->warp_zs;
+    const long long key = ((long long)n << 24) ^ ((long long)O << 16) ^ ((long long)ctx->warp_cfg << 8) ^ ctx->warp_zs ^
+                          (a.margin_off ? 1LL << 48 : 0);  // the offset instantiations have kernel attributes of their own
     if (key != ctx->warp_key) {
       ctx->warp_key = key;
       ctx->warp_zs_pick = 0;
@@ -675,6 +679,7 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
     a.esc_count = cnt + 5;
     a.work_counter2 = cnt + 4;
     a.esc_steps = ctx->esc_steps;
+    // work order: a scheduling heuristic from the reference line only; it ignores margin_off (the offsets change no result)
     if (ctx->lpt && O > 0 && B > 1) {  // listB / flags are free in the fused path: work order + its scratch
       CU(launch_work_order(ctx->dtab, nj, O, B, H, xref, a.margin_is_D, ptr<int>(ctx->flags), ptr<int>(ctx->listB), st));
       launches += 2;
@@ -1655,6 +1660,275 @@ extern "C" int cfs_check_trajectories(cfs_ctx *ctx, int B, int H, const double *
   if (evals) CU(cudaMemcpyAsync(evals, d_e, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return 0;
+}
+
+// ---- per-waypoint margin offsets and the checked solve (include/cfs_b200.h) ----------------------------------------------------
+static int check_offsets_device(cfs_ctx *ctx, const char *who, int B, const double *margin_off) {
+  const long long N = (long long)ctx->nobs * ctx->H * B;
+  int rc;
+  if (!margin_off) return 0;
+  if ((rc = ensure(ctx, ctx->chk_ctr, 64))) return rc;
+  int *bad = ptr<int>(ctx->chk_ctr) + 8, hbad = 0;
+  CU(launch_offsets_bad(N, margin_off, bad, ctx->stream));
+  CU(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (hbad) return fail(ctx, CFS_E_ARG, "%s: margin_off has a negative or non-finite entry", who);
+  return 0;
+}
+
+extern "C" int cfs_solve_batch_margins_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                              const double *caug, const double *xref, const double *noise, const double *margin_off,
+                                              double eps_outer, int max_outer, double alpha, double *u, double *x,
+                                              double *cost_hist, double *e_u_hist, int *iters, int *status, int sync) {
+  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  if (!x) return fail(ctx, CFS_E_ARG, "cfs_solve_batch_margins_device: NULL x");
+  CU(cudaSetDevice(ctx->device));
+  if ((rc = check_offsets_device(ctx, "cfs_solve_batch_margins_device", B, margin_off))) return rc;
+  ctx->pending.active = false;
+  rc = solve_device(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist, iters,
+                    status, margin_off);
+  if (rc) return rc;
+  ctx->pending.active = true;
+  ctx->pending.host = false;
+  ctx->pending.B = B;
+  ctx->pending.max_outer = max_outer;
+  ctx->pending.d_iters = iters;
+  ctx->pending.d_status = status;
+  if (sync) return finish_pending(ctx);
+  return 0;
+}
+
+// host form of the margin / checked solves: inputs to the context's batch buffers, the device form, results back (synchronous)
+struct HostBatch {
+  double *x0, *ff, *caug, *xref, *noise, *off, *u, *x, *ch, *eu;
+  int *iters, *status;
+};
+static int host_batch_in(cfs_ctx *ctx, int B, int max_outer, const double *x0, const double *ff, const double *caug,
+                         const double *xref, const double *noise, const double *off, HostBatch &d) {
+  const int nj = ctx->nj, n = ctx->n, K = max_outer > 0 ? max_outer : 1;
+  const size_t OH = (size_t)ctx->nobs * ctx->H;
+  cudaStream_t st = ctx->stream;
+  int rc;
+  if (ctx->pending.active && (rc = finish_pending(ctx))) return rc;
+  if ((rc = ensure(ctx, ctx->x0, sizeof(double) * 2 * nj * B))) return rc;
+  if ((rc = ensure(ctx, ctx->ff, sizeof(double) * (size_t)n * B))) return rc;
+  if ((rc = ensure(ctx, ctx->caug, sizeof(double) * B))) return rc;
+  if ((rc = ensure(ctx, ctx->xref, sizeof(double) * (size_t)2 * n * B))) return rc;
+  if ((rc = ensure(ctx, ctx->u, sizeof(double) * (size_t)n * B))) return rc;
+  if ((rc = ensure(ctx, ctx->x, sizeof(double) * (size_t)2 * n * B))) return rc;
+  if ((rc = ensure(ctx, ctx->cost, sizeof(double) * (size_t)K * B))) return rc;
+  if ((rc = ensure(ctx, ctx->eu, sizeof(double) * (size_t)K * B))) return rc;
+  if ((rc = ensure(ctx, ctx->iters, sizeof(int) * B))) return rc;
+  if ((rc = ensure(ctx, ctx->status, sizeof(int) * B))) return rc;
+  if (noise && (rc = ensure(ctx, ctx->noise, sizeof(double) * (size_t)n * K * B))) return rc;
+  if ((rc = ensure(ctx, ctx->rep_off, sizeof(double) * (OH ? OH : 1) * B))) return rc;
+  d.x0 = ptr<double>(ctx->x0); d.ff = ptr<double>(ctx->ff); d.caug = ptr<double>(ctx->caug); d.xref = ptr<double>(ctx->xref);
+  d.noise = noise ? ptr<double>(ctx->noise) : nullptr;
+  d.off = off ? ptr<double>(ctx->rep_off) : nullptr;
+  d.u = ptr<double>(ctx->u); d.x = ptr<double>(ctx->x); d.ch = ptr<double>(ctx->cost); d.eu = ptr<double>(ctx->eu);
+  d.iters = ptr<int>(ctx->iters); d.status = ptr<int>(ctx->status);
+  CU(cudaMemcpyAsync(d.x0, x0, sizeof(double) * 2 * nj * B, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d.ff, ff, sizeof(double) * (size_t)n * B, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d.caug, caug, sizeof(double) * B, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d.xref, xref, sizeof(double) * (size_t)2 * n * B, cudaMemcpyHostToDevice, st));
+  if (noise) CU(cudaMemcpyAsync(d.noise, noise, sizeof(double) * (size_t)n * K * B, cudaMemcpyHostToDevice, st));
+  if (off && OH) CU(cudaMemcpyAsync(d.off, off, sizeof(double) * OH * B, cudaMemcpyHostToDevice, st));
+  return 0;
+}
+static int host_batch_out(cfs_ctx *ctx, int B, int max_outer, const HostBatch &d, double *u, double *x, double *cost_hist,
+                          double *e_u_hist, int *iters, int *status) {
+  const int n = ctx->n;
+  cudaStream_t st = ctx->stream;
+  CU(cudaMemcpyAsync(u, d.u, sizeof(double) * (size_t)n * B, cudaMemcpyDeviceToHost, st));
+  if (x) CU(cudaMemcpyAsync(x, d.x, sizeof(double) * (size_t)2 * n * B, cudaMemcpyDeviceToHost, st));
+  if (max_outer > 0) {
+    CU(cudaMemcpyAsync(cost_hist, d.ch, sizeof(double) * (size_t)max_outer * B, cudaMemcpyDeviceToHost, st));
+    if (e_u_hist) CU(cudaMemcpyAsync(e_u_hist, d.eu, sizeof(double) * (size_t)max_outer * B, cudaMemcpyDeviceToHost, st));
+  }
+  CU(cudaMemcpyAsync(iters, d.iters, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(status, d.status, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  return 0;
+}
+
+extern "C" int cfs_solve_batch_margins(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                       const double *caug, const double *xref, const double *noise, const double *margin_off,
+                                       double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                                       double *e_u_hist, int *iters, int *status) {
+  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  if (margin_off)
+    for (size_t e = 0, N = (size_t)ctx->nobs * ctx->H * B; e < N; ++e)
+      if (!(margin_off[e] >= 0.0 && margin_off[e] < INFINITY))
+        return fail(ctx, CFS_E_ARG, "cfs_solve_batch_margins: margin_off[%zu] = %g is negative or not finite", e, margin_off[e]);
+  CU(cudaSetDevice(ctx->device));
+  HostBatch d;
+  if ((rc = host_batch_in(ctx, B, max_outer, x0, ff, caug, xref, noise, margin_off, d))) return rc;
+  ctx->pending.active = false;
+  rc = solve_device(ctx, B, solver, grad, d.x0, d.ff, d.caug, d.xref, d.noise, eps_outer, max_outer, alpha, d.u, d.x, d.ch,
+                    e_u_hist ? d.eu : nullptr, d.iters, d.status, d.off);
+  if (rc) return rc;
+  if ((rc = collect_stats(ctx, B, max_outer, d.iters, d.status))) return rc;
+  return host_batch_out(ctx, B, max_outer, d, u, x, cost_hist, e_u_hist, iters, status);
+}
+
+static int check_checked_args(cfs_ctx *ctx, const char *who, int B, int solver, double eta, int max_evals, int rounds, double gain) {
+  int rc = check_traj_args(ctx, who, B, ctx->H > 0 ? ctx->H : 1, eta, solver == CFS_SOLVER_PSGCFS, max_evals);
+  if (rc) return rc;
+  if (rounds < 0) return fail(ctx, CFS_E_ARG, "%s: rounds=%d", who, rounds);
+  if (!(gain > 0.0) || !std::isfinite(gain)) return fail(ctx, CFS_E_ARG, "%s: gain must be positive and finite (%g)", who, gain);
+  return 0;
+}
+
+// The round loop.  Problem-indexed state lives in the caller's (device) buffers; the sub-batch of a round (at most B problems) in
+// context buffers: rep_in = x0 | ff | caug | xref | noise | offsets, rep_out = u | x | cost | e_u | verdict | t_hit | cmin (doubles)
+// then iters | status | verdict (ints), rep_list = sel | list A | list B | count.  rep_off holds the accumulated offsets of every
+// problem; margin_off_out (NULL: not returned) receives the offsets of the round each returned solution comes from.
+static int solve_checked_dev(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
+                             const double *xref, const double *noise, double eps_outer, int max_outer, double alpha, double eta,
+                             int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
+                             int *iters, int *status, int *verdict, double *t_hit, double *cmin, int *rounds_used,
+                             double *margin_off_out) {
+  const int nj = ctx->nj, n = ctx->n, H = ctx->H, O = ctx->nobs, K = max_outer;
+  const size_t OH = (size_t)O * H, nx0 = 2 * nj, N = 2 * (size_t)n, nnz = noise ? (size_t)n * K : 0;
+  const int margin_is_D = solver == CFS_SOLVER_PSGCFS;
+  cudaStream_t st = ctx->stream;
+  int rc;
+  ctx->pending.active = false;
+  // round 0: the plain solve and its check
+  if ((rc = solve_device(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist,
+                         iters, status)))
+    return rc;
+  if ((rc = collect_stats(ctx, B, max_outer, iters, status))) return rc;  // cfs_get_stats: round 0's solve
+  if ((rc = check_traj_dev(ctx, B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin, nullptr))) return rc;
+  CU(cudaMemsetAsync(rounds_used, 0, sizeof(int) * B, st));
+  if ((rc = ensure(ctx, ctx->rep_off, sizeof(double) * (OH ? OH : 1) * B))) return rc;
+  double *off = ptr<double>(ctx->rep_off);
+  if (OH) CU(cudaMemsetAsync(off, 0, sizeof(double) * OH * B, st));
+  if (OH && margin_off_out) CU(cudaMemsetAsync(margin_off_out, 0, sizeof(double) * OH * B, st));
+  if (rounds == 0 || O == 0) return 0;
+
+  const size_t in_row = nx0 + n + 1 + N + nnz + OH, out_row = n + N + 2 * (size_t)(K > 0 ? K : 1) + 2;
+  if ((rc = ensure(ctx, ctx->rep_in, sizeof(double) * in_row * B))) return rc;
+  if ((rc = ensure(ctx, ctx->rep_out, sizeof(double) * out_row * B + sizeof(int) * 3 * (size_t)B))) return rc;
+  if ((rc = ensure(ctx, ctx->rep_list, sizeof(int) * (3 * (size_t)B + 2)))) return rc;
+  double *sx0 = ptr<double>(ctx->rep_in), *sff = sx0 + nx0 * B, *scaug = sff + (size_t)n * B, *sxref = scaug + B,
+         *snoise = sxref + N * B, *soff = snoise + nnz * B;
+  const int Kc = K > 0 ? K : 1;
+  double *su = ptr<double>(ctx->rep_out), *sx = su + (size_t)n * B, *sch = sx + N * B, *seu = sch + (size_t)Kc * B,
+         *sth = seu + (size_t)Kc * B, *scm = sth + B;
+  int *sit = reinterpret_cast<int *>(scm + B), *sst = sit + B, *sv = sst + B;
+  int *sel = ptr<int>(ctx->rep_list), *lst[2] = {sel + B, sel + 2 * (size_t)B}, *d_count = sel + 3 * (size_t)B;
+  CheckArgs ca = check_base(ctx, 1, B * H, eta, margin_is_D, max_evals);
+  ca.H = H;
+  // per-segment results of the last check of nb trajectories, as check_traj_dev lays them out in chk_seg
+  auto seg_results = [&](int nb) {
+    const size_t S = (size_t)nb * H;
+    ca.s_hit = ptr<double>(ctx->chk_seg);
+    ca.verdict = reinterpret_cast<int *>(ca.s_hit + 2 * S);
+  };
+
+  // after round 0: HIT and status < 2 -> list; increments from the round-0 check
+  CU(launch_repair_select(B, verdict, status, nullptr, sel, lst[0], d_count, st));
+  ca.x0 = x0; ca.x = x; ca.u = u;
+  seg_results(B);
+  CU(launch_repair_margins(ca, B, d_count, sel, nullptr, gain, off, st));
+  int cur = 0;
+  for (int r = 1; r <= rounds; ++r) {
+    int c = 0;  // one count readback per round
+    CU(cudaMemcpyAsync(&c, d_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (c == 0) break;
+    const int *L = lst[cur];
+    // gather the sub-batch from the caller's original inputs (re-solved from xref, not warm-started) and the offsets
+    CU(launch_rows_copy(c, L, x0, sx0, nx0, 0, nullptr, st));
+    CU(launch_rows_copy(c, L, ff, sff, n, 0, nullptr, st));
+    CU(launch_rows_copy(c, L, caug, scaug, 1, 0, nullptr, st));
+    CU(launch_rows_copy(c, L, xref, sxref, N, 0, nullptr, st));
+    if (noise) CU(launch_rows_copy(c, L, noise, snoise, nnz, 0, nullptr, st));
+    CU(launch_rows_copy(c, L, off, soff, OH, 0, nullptr, st));
+    if ((rc = solve_device(ctx, c, solver, grad, sx0, sff, scaug, sxref, noise ? snoise : nullptr, eps_outer, max_outer, alpha, su,
+                           sx, sch, e_u_hist ? seu : nullptr, sit, sst, soff)))
+      return rc;
+    if ((rc = check_traj_dev(ctx, c, H, sx0, sx, su, eta, margin_is_D, max_evals, sv, sth, scm, nullptr))) return rc;
+    // accepted candidates (status < 2) replace the solution; failed ones leave it and stop repairing
+    CU(launch_rows_copy(c, L, su, u, n, 1, sst, st));
+    CU(launch_rows_copy(c, L, sx, x, N, 1, sst, st));
+    if (K > 0) {
+      CU(launch_rows_copy(c, L, sch, cost_hist, K, 1, sst, st));
+      if (e_u_hist) CU(launch_rows_copy(c, L, seu, e_u_hist, K, 1, sst, st));
+    }
+    CU(launch_ints_copy(c, L, sit, iters, 1, sst, -1, st));
+    CU(launch_ints_copy(c, L, sst, status, 1, sst, -1, st));
+    CU(launch_ints_copy(c, L, sv, verdict, 1, sst, -1, st));
+    CU(launch_rows_copy(c, L, sth, t_hit, 1, 1, sst, st));
+    CU(launch_rows_copy(c, L, scm, cmin, 1, 1, sst, st));
+    CU(launch_ints_copy(c, L, nullptr, rounds_used, 1, sst, r, st));
+    if (margin_off_out) CU(launch_rows_copy(c, L, soff, margin_off_out, OH, 1, sst, st));
+    if (r == rounds) break;
+    CU(launch_repair_select(c, sv, sst, L, sel, lst[cur ^ 1], d_count, st));
+    ca.x0 = sx0; ca.x = sx; ca.u = su;
+    seg_results(c);
+    CU(launch_repair_margins(ca, c, d_count, sel, L, gain, off, st));
+    cur ^= 1;
+  }
+  return 0;
+}
+
+extern "C" int cfs_solve_checked_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                        const double *caug, const double *xref, const double *noise, double eps_outer,
+                                        int max_outer, double alpha, double eta, int max_evals, int rounds, double gain, double *u,
+                                        double *x, double *cost_hist, double *e_u_hist, int *iters, int *status, int *verdict,
+                                        double *t_hit, double *cmin, int *rounds_used, double *margin_off, int sync) {
+  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
+  if (rc) return rc;
+  if ((rc = check_checked_args(ctx, "cfs_solve_checked_device", B, solver, eta, max_evals, rounds, gain))) return rc;
+  if (B == 0) return 0;
+  if (!x || !verdict || !t_hit || !cmin || !rounds_used) return fail(ctx, CFS_E_ARG, "cfs_solve_checked_device: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  if ((rc = solve_checked_dev(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, eta, max_evals, rounds,
+                              gain, u, x, cost_hist, e_u_hist, iters, status, verdict, t_hit, cmin, rounds_used, margin_off)))
+    return rc;
+  if (sync) CU(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int cfs_solve_checked(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
+                                 const double *xref, const double *noise, double eps_outer, int max_outer, double alpha, double eta,
+                                 int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
+                                 int *iters, int *status, int *verdict, double *t_hit, double *cmin, int *rounds_used,
+                                 double *margin_off) {
+  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
+  if (rc) return rc;
+  if ((rc = check_checked_args(ctx, "cfs_solve_checked", B, solver, eta, max_evals, rounds, gain))) return rc;
+  if (B == 0) return 0;
+  if (!x || !verdict || !t_hit || !cmin || !rounds_used) return fail(ctx, CFS_E_ARG, "cfs_solve_checked: NULL buffer");
+  CU(cudaSetDevice(ctx->device));
+  HostBatch d;
+  if ((rc = host_batch_in(ctx, B, max_outer, x0, ff, caug, xref, noise, nullptr, d))) return rc;
+  const size_t OH = (size_t)ctx->nobs * ctx->H;
+  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)B + 64))) return rc;
+  double *d_t = ptr<double>(ctx->chk_out), *d_c = d_t + B;
+  int *d_v = reinterpret_cast<int *>(d_c + B), *d_r = d_v + B;
+  double *d_off = nullptr;
+  if (margin_off && OH) {
+    if ((rc = ensure(ctx, ctx->rep_offo, sizeof(double) * OH * B))) return rc;
+    d_off = ptr<double>(ctx->rep_offo);
+  }
+  if ((rc = solve_checked_dev(ctx, B, solver, grad, d.x0, d.ff, d.caug, d.xref, d.noise, eps_outer, max_outer, alpha, eta, max_evals,
+                              rounds, gain, d.u, d.x, d.ch, e_u_hist ? d.eu : nullptr, d.iters, d.status, d_v, d_t, d_c, d_r,
+                              d_off)))
+    return rc;
+  cudaStream_t st = ctx->stream;
+  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(t_hit, d_t, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(rounds_used, d_r, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
+  if (d_off) CU(cudaMemcpyAsync(margin_off, d_off, sizeof(double) * OH * B, cudaMemcpyDeviceToHost, st));
+  return host_batch_out(ctx, B, max_outer, d, u, x, cost_hist, e_u_hist, iters, status);
 }
 
 extern "C" int cfs_nearest_steer(cfs_ctx *ctx, int n_nodes, const double *nodes, int S, const double *samples,

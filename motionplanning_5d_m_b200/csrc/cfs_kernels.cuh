@@ -58,6 +58,23 @@ cudaError_t launch_check(const CheckArgs &a, int device, cudaStream_t s);
 // per-segment results (B*H each) -> per-trajectory verdict, t_hit, cmin, evals (evals may be nullptr)
 cudaError_t launch_check_reduce(int B, int H, double dt, const int *sv, const double *ss, const double *sc, const int *se,
                                 int *verdict, double *t_hit, double *cmin, int *evals, cudaStream_t s);
+// repair increments of the checked solve: per trajectory b, segments in order; for every HIT segment k the witness theta* of
+// s_hit[k] and its clearance per obstacle c_j; obstacles with c_j < -eta/2 get inc = gain (eta - c_j) at waypoints k and k+1
+// (1..H only), the maximum over the adjacent HIT segments, added to margin_off[(b nobs + j) H + i - 1].  a.verdict / a.s_hit
+// are the per-segment results of launch_check (mode 1); x0 / x / u the checked trajectories.
+// sel[t] (t < *count, at most nmax) are positions in the checked set, map[pos] (nullptr: identity) the problem of margin_off
+cudaError_t launch_repair_margins(const CheckArgs &a, int nmax, const int *count, const int *sel, const int *map, double gain,
+                                  double *margin_off, cudaStream_t s);
+// the round loop of the checked solve: stable selection of the positions p < N with verdict[p] == HIT and status low byte < 2
+// (sel = positions, next = map[p] or p, *count); row gather (dst[t] = src[list[t]]) / scatter (dst[list[t]] = src[t], skipped
+// where st[t] low byte >= 2); fill >= 0 writes that value instead of src
+cudaError_t launch_repair_select(int N, const int *verdict, const int *status, const int *map, int *sel, int *next, int *count,
+                                 cudaStream_t s);
+cudaError_t launch_rows_copy(int n_rows, const int *list, const double *src, double *dst, long long len, int scatter, const int *st,
+                             cudaStream_t s);
+cudaError_t launch_ints_copy(int n_rows, const int *list, const int *src, int *dst, int scatter, const int *st, int fill,
+                             cudaStream_t s);
+cudaError_t launch_offsets_bad(long long N, const double *off, int *bad, cudaStream_t s);
 
 // work order of the fused solver (longest expected problems first): order[] = problems by descending number of reference
 // waypoints inside an obstacle margin; count[] is scratch (B ints each)
@@ -171,6 +188,11 @@ struct SolveArgs {
   // still ahead); it_stop = 0: run to the stop rule
   int it_stop;
   int *cont_out, *cont_out_count;
+  // per-waypoint margin offsets [prob][obs][i] (same layout as dist), finite and >= 0, or nullptr: the obstacle row of (j, i)
+  // uses dist - (margin_j + off) instead of dist - margin_j.  Read only by the instantiations compiled with the offset flag (the
+  // launch wrappers pick them when margin_off != nullptr), so the kernels launched without offsets are unchanged.  Last member:
+  // the parameter offsets of every other field stay where they were.
+  const double *margin_off;
 };
 cudaError_t launch_solve_init(const SolveArgs &a, cudaStream_t s);
 cudaError_t launch_v0(const SolveArgs &a, cudaStream_t s);

@@ -58,7 +58,9 @@ __host__ __device__ inline FusedLayout fused_layout(int n, int nj, int OH, int m
   return L;
 }
 
-template <int NJ, int NT, int QS, int MINB, int QZ, int MAXREG = (MINB == 1 ? 255 : 168)>
+// OFF: the obstacle rows read a.margin_off (per-waypoint margin offsets of the checked solve); a separate instantiation, the one
+// without it is unchanged
+template <int NJ, int NT, int QS, int MINB, int QZ, int MAXREG = (MINB == 1 ? 255 : 168), bool OFF = false>
 __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = a.n, nj = NJ, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + 4 * n, N = 2 * n;
@@ -184,7 +186,8 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs 
 #pragma unroll 1
       for (int cid = tid; cid < OH; cid += NT) {  // I = distance - margin (CFS_FANUC.m:117)
         const int j = cid / H;
-        s.orhs[cid] -= a.margin_is_D ? tab.obs[j].D : tab.obs[j].eps;
+        const double margin = a.margin_is_D ? tab.obs[j].D : tab.obs[j].eps;
+        s.orhs[cid] -= OFF ? margin + a.margin_off[(size_t)b * OH + cid] : margin;
       }
       __syncthreads();
 #pragma unroll 1
@@ -338,38 +341,33 @@ static int grid_of(K kernel, int nt, size_t smem, int device) {
   return sms * per;
 }
 
+typedef void (*FusedKernel)(SolveArgs);
+template <int NJ, bool OFF>
+static FusedKernel fused_kernel_nj(int tier) {
+  if (tier == 0) return k_cfs_fused<NJ, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ, 168, OFF>;
+  if (tier == 1) return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0, 255, OFF>;
+  return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168, OFF>;
+}
+// tier 0 bulk, 1 heavy, 2 slim heavy; the margin-offset instantiations when a.margin_off is set
+static FusedKernel fused_kernel(const SolveArgs &a, int tier) {
+  const bool off = a.margin_off != nullptr;
+  if (a.nj == 2) return off ? fused_kernel_nj<2, true>(tier) : fused_kernel_nj<2, false>(tier);
+  if (a.nj == 5) return off ? fused_kernel_nj<5, true>(tier) : fused_kernel_nj<5, false>(tier);
+  return nullptr;
+}
+
 int fused_max_grid(const SolveArgs &a, int device, int tier) {
-  const size_t smem = fused_smem_bytes(a, tier);
-  if (tier == 0) {
-    if (a.nj == 2) return grid_of(k_cfs_fused<2, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ>, FUSED_BULK_NT, smem, device);
-    if (a.nj == 5) return grid_of(k_cfs_fused<5, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ>, FUSED_BULK_NT, smem, device);
-  } else if (tier == 1) {
-    if (a.nj == 2) return grid_of(k_cfs_fused<2, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0>, FUSED_HEAVY_NT, smem, device);
-    if (a.nj == 5) return grid_of(k_cfs_fused<5, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0>, FUSED_HEAVY_NT, smem, device);
-  } else {
-    if (a.nj == 2) return grid_of(k_cfs_fused<2, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168>, FUSED_HEAVY_NT, smem, device);
-    if (a.nj == 5) return grid_of(k_cfs_fused<5, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168>, FUSED_HEAVY_NT, smem, device);
-  }
-  return 0;
+  FusedKernel k = fused_kernel(a, tier);
+  if (!k) return 0;
+  return grid_of(k, tier == 0 ? FUSED_BULK_NT : FUSED_HEAVY_NT, fused_smem_bytes(a, tier), device);
 }
 
 cudaError_t launch_fused(const SolveArgs &a_in, int grid, int tier, cudaStream_t st) {
   SolveArgs a = a_in;
   a.tier = tier ? 1 : 0;
-  const size_t smem = fused_smem_bytes(a, tier);
-  if (tier == 0) {
-    if (a.nj == 2) k_cfs_fused<2, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ><<<grid, FUSED_BULK_NT, smem, st>>>(a);
-    else if (a.nj == 5) k_cfs_fused<5, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ><<<grid, FUSED_BULK_NT, smem, st>>>(a);
-    else return cudaErrorInvalidValue;
-  } else if (tier == 1) {
-    if (a.nj == 2) k_cfs_fused<2, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0><<<grid, FUSED_HEAVY_NT, smem, st>>>(a);
-    else if (a.nj == 5) k_cfs_fused<5, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0><<<grid, FUSED_HEAVY_NT, smem, st>>>(a);
-    else return cudaErrorInvalidValue;
-  } else {
-    if (a.nj == 2) k_cfs_fused<2, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168><<<grid, FUSED_HEAVY_NT, smem, st>>>(a);
-    else if (a.nj == 5) k_cfs_fused<5, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168><<<grid, FUSED_HEAVY_NT, smem, st>>>(a);
-    else return cudaErrorInvalidValue;
-  }
+  FusedKernel k = fused_kernel(a, tier);
+  if (!k) return cudaErrorInvalidValue;
+  k<<<grid, tier == 0 ? FUSED_BULK_NT : FUSED_HEAVY_NT, fused_smem_bytes(a, tier), st>>>(a);
   return cudaGetLastError();
 }
 

@@ -35,6 +35,9 @@ size_t qp_smem_bytes(const SolveArgs &a) {
 // ============================================================================================================
 // The kernel
 // ============================================================================================================
+// OFF: the obstacle rows read a.margin_off (per-waypoint margin offsets of the checked solve); a separate instantiation, the one
+// without it is unchanged
+template <bool OFF>
 __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int n = a.n, nj = a.nj, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + 4 * n;
@@ -95,7 +98,8 @@ __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
       const int j = cid / H, i = cid % H;
       const double *gr = a.grad + ((size_t)b * OH + cid) * nj;
       const double dist = a.dist[(size_t)b * OH + cid];
-      const double margin = a.margin_is_D ? a.tab->obs[j].D : a.tab->obs[j].eps;
+      double margin = a.margin_is_D ? a.tab->obs[j].D : a.tab->obs[j].eps;
+      if (OFF) margin = margin + a.margin_off[(size_t)b * OH + cid];
       double gu = 0.0;
       for (int k = 0; k < nj; ++k) {
         s.ocoef[cid * nj + k] = -gr[k];                 // l = -Diff'*Bj(1:njoint,:)   (CFS_FANUC.m:121)
@@ -218,15 +222,16 @@ int qp_max_grid(const SolveArgs &a, int device) {
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   const size_t smem = qp_smem_bytes(a);
-  cudaFuncSetAttribute(k_qp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, k_qp, QP_THREADS, smem);
+  void (*k)(SolveArgs) = a.margin_off ? k_qp<true> : k_qp<false>;
+  cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, k, QP_THREADS, smem);
   if (per < 1) per = 1;
   return sms * per;
 }
 
 cudaError_t launch_qp(const SolveArgs &a, int grid, cudaStream_t st) {
   const size_t smem = qp_smem_bytes(a);
-  k_qp<<<grid, QP_THREADS, smem, st>>>(a);
+  (a.margin_off ? k_qp<true> : k_qp<false>)<<<grid, QP_THREADS, smem, st>>>(a);
   return cudaGetLastError();
 }
 

@@ -137,8 +137,9 @@ __host__ __device__ inline WarpSmem warp_smem(int n, int nj, int OH, int zs, int
 }
 
 // PROF: clock64 split of every problem into gradient phase / QP / everything (timing level 3: cfs_get_warp_profile); a separate
-// instantiation so that the production kernel keeps its register budget
-template <int NJ, int NT, int MAXREG, int OC, bool PROF = false>
+// instantiation so that the production kernel keeps its register budget.  OFF: the obstacle rows read a.margin_off (the
+// checked solve's per-waypoint margin offsets); also a separate instantiation, the one without it is unchanged.
+template <int NJ, int NT, int MAXREG, int OC, bool PROF = false, bool OFF = false>
 __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int WPC = NT / 32;
@@ -240,7 +241,8 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
           for (int jj = 0; jj < OC; ++jj) {
             if (j0 + jj >= O) continue;
             const int cid = (j0 + jj) * H + i;
-            const double margin = a.margin_is_D ? tab.obs[j0 + jj].D : tab.obs[j0 + jj].eps;
+            double margin = a.margin_is_D ? tab.obs[j0 + jj].D : tab.obs[j0 + jj].eps;
+            if (OFF) margin = margin + a.margin_off[(size_t)b * OH + cid];
             double gu = 0.0, sg = 0.0;
 #pragma unroll 1
             for (int k = 0; k < NJ; ++k) {
@@ -384,7 +386,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
 // DERIVEST gradients come from their own kernel) keeps its structure -- gradient kernel | QP kernel per outer iteration -- but
 // the QP kernel (k_qp.cu: one CTA per problem) is replaced by this one: same prologue / epilogue, wqp_solve in the middle.
 // Problems whose working set outgrows the warp tier are appended to esc_list and taken by k_qp in the same iteration.
-template <int NJ, int NT>
+template <int NJ, int NT, bool OFF = false>
 __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int WPC = NT / 32;
@@ -423,7 +425,8 @@ __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
     for (int cid = lane; cid < OH; cid += 32) {
       const int j = cid / H, i = cid - j * H;
       const double *gr = a.grad + ((size_t)b * OH + cid) * NJ;
-      const double margin = a.margin_is_D ? a.tab->obs[j].D : a.tab->obs[j].eps;
+      double margin = a.margin_is_D ? a.tab->obs[j].D : a.tab->obs[j].eps;
+      if (OFF) margin = margin + a.margin_off[(size_t)b * OH + cid];
       double gu = 0.0, sg = 0.0;
 #pragma unroll
       for (int k = 0; k < NJ; ++k) {
@@ -545,27 +548,29 @@ int warp_warps_per_cta(int cfg) { return kWarpNT[cfg] / 32; }
 size_t warp_slab_bytes_per_warp(const SolveArgs &a) { return sizeof(double) * warp_slab_doubles(a.n, a.warp_zs); }
 
 typedef void (*WarpKernel)(SolveArgs);
-template <int NJ>
+template <int NJ, bool OFF>
 static WarpKernel warp_kernel_nj(int cfg, bool two) {
   switch (cfg) {
-    case 0: return two ? k_cfs_warp<NJ, 384, 168, 2> : k_cfs_warp<NJ, 384, 168, 1>;
-    case 1: return two ? k_cfs_warp<NJ, 96, 224, 2> : k_cfs_warp<NJ, 96, 224, 1>;
-    case 2: return two ? k_cfs_warp<NJ, 128, 168, 2> : k_cfs_warp<NJ, 128, 168, 1>;
-    case 3: return two ? k_cfs_warp<NJ, 32, 168, 2> : k_cfs_warp<NJ, 32, 168, 1>;
-    case 4: return two ? k_cfs_warp<NJ, 64, 168, 2> : k_cfs_warp<NJ, 64, 168, 1>;
+    case 0: return two ? k_cfs_warp<NJ, 384, 168, 2, false, OFF> : k_cfs_warp<NJ, 384, 168, 1, false, OFF>;
+    case 1: return two ? k_cfs_warp<NJ, 96, 224, 2, false, OFF> : k_cfs_warp<NJ, 96, 224, 1, false, OFF>;
+    case 2: return two ? k_cfs_warp<NJ, 128, 168, 2, false, OFF> : k_cfs_warp<NJ, 128, 168, 1, false, OFF>;
+    case 3: return two ? k_cfs_warp<NJ, 32, 168, 2, false, OFF> : k_cfs_warp<NJ, 32, 168, 1, false, OFF>;
+    case 4: return two ? k_cfs_warp<NJ, 64, 168, 2, false, OFF> : k_cfs_warp<NJ, 64, 168, 1, false, OFF>;
   }
   return nullptr;
 }
-static WarpKernel warp_kernel(int nj, int cfg, int nobs, bool prof = false) {
-  if (prof && nj == 5 && cfg == 3 && nobs <= 1) return k_cfs_warp<5, 32, 168, 1, true>;
-  if (nj == 2) return warp_kernel_nj<2>(cfg, nobs > 1);
-  if (nj == 5) return warp_kernel_nj<5>(cfg, nobs > 1);
+// off: the margin-offset instantiations (a.margin_off != nullptr); the phase profile has none (timing level 3 measures the
+// unchecked solve)
+static WarpKernel warp_kernel(int nj, int cfg, int nobs, bool prof = false, bool off = false) {
+  if (prof && !off && nj == 5 && cfg == 3 && nobs <= 1) return k_cfs_warp<5, 32, 168, 1, true>;
+  if (nj == 2) return off ? warp_kernel_nj<2, true>(cfg, nobs > 1) : warp_kernel_nj<2, false>(cfg, nobs > 1);
+  if (nj == 5) return off ? warp_kernel_nj<5, true>(cfg, nobs > 1) : warp_kernel_nj<5, false>(cfg, nobs > 1);
   return nullptr;
 }
 
 int warp_max_grid(const SolveArgs &a, int device, int cfg) {
   const size_t smem = warp_smem_bytes(a, cfg);
-  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs);
+  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, false, a.margin_off != nullptr);
   if (!k) return 0;
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -578,9 +583,10 @@ int warp_max_grid(const SolveArgs &a, int device, int cfg) {
 }
 
 cudaError_t launch_warp(const SolveArgs &a, int grid, int cfg, cudaStream_t st) {
-  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, a.prof != nullptr);
+  const bool off = a.margin_off != nullptr;
+  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, a.prof != nullptr, off);
   if (!k) return cudaErrorInvalidValue;
-  if (a.prof) {  // the profiled instantiation is a function of its own: same opt-in limits as warp_max_grid sets
+  if (a.prof && !off) {  // the profiled instantiation is a function of its own: same opt-in limits as warp_max_grid sets
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   }
@@ -597,7 +603,8 @@ bool qp_warp_supported(const SolveArgs &a) {
 
 int qp_warp_max_grid(const SolveArgs &a, int device) {
   const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0).total;
-  WarpKernel k = a.nj == 2 ? k_qp_warp<2, 128> : k_qp_warp<5, 128>;
+  const bool off = a.margin_off != nullptr;
+  WarpKernel k = a.nj == 2 ? (off ? k_qp_warp<2, 128, true> : k_qp_warp<2, 128>) : (off ? k_qp_warp<5, 128, true> : k_qp_warp<5, 128>);
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return 0;
@@ -608,8 +615,9 @@ int qp_warp_max_grid(const SolveArgs &a, int device) {
 
 cudaError_t launch_qp_warp(const SolveArgs &a, int grid, cudaStream_t st) {
   const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0).total;
-  if (a.nj == 2) k_qp_warp<2, 128><<<grid, 128, smem, st>>>(a);
-  else if (a.nj == 5) k_qp_warp<5, 128><<<grid, 128, smem, st>>>(a);
+  const bool off = a.margin_off != nullptr;
+  if (a.nj == 2) (off ? k_qp_warp<2, 128, true> : k_qp_warp<2, 128>)<<<grid, 128, smem, st>>>(a);
+  else if (a.nj == 5) (off ? k_qp_warp<5, 128, true> : k_qp_warp<5, 128>)<<<grid, 128, smem, st>>>(a);
   else return cudaErrorInvalidValue;
   return cudaGetLastError();
 }

@@ -1,0 +1,54 @@
+// checked_harness.cpp -- the stub harness (harness.cpp: mex.h stand-in, argument builders, the existing mexh_* entries) plus an
+// entry point for the gateway's 'solve_checked' command.  Test infrastructure only; tests/test_mex_solve_checked.py compiles it
+// together with matlab/cfs_mex.cpp into a library of its own.
+#include "harness.cpp"
+
+// [u, x_, cost_all, e_u_all, iters, status, verdict, t_hit, cmin, rounds_used, margin_off] =
+//     cfs_mex('solve_checked', solver, grad, ROBOT, obs, sys_info, [], eta, rounds, gain)
+// All matrices column-major as MATLAB stores them; lim / max_input may be NULL.
+extern "C" int mexh_solve_checked(const char *solver, const char *grad, const char *robot_name, int nj, int H, int B, int dh_rows,
+                                  const double *DH, const double *base, const double *cap_p, const double *T, double dt, int nobs,
+                                  const double *obs_l, const double *obs_D, const double *obs_eps, const double *QQ,
+                                  const double *lim, const double *max_input, const double *xR, const double *ff,
+                                  const double *caug, const double *xref, double eps_outer, int max_outer, double eta, int rounds,
+                                  double gain, double *u, double *x, double *cost, double *eu, int *iters, int *status,
+                                  int *verdict, double *t_hit, double *cmin, int *rounds_used, double *margin_off) {
+  const size_t n = (size_t)H * nj;
+  g_err[0] = 0;
+  mxArray *si = strct();
+  const double Hd = H, njd = nj, Kd = max_outer, rd = rounds;
+  si->fields["H"] = dbl(1, 1, &Hd);
+  si->fields["njoint"] = dbl(1, 1, &njd);
+  si->fields["robot"] = robot_struct(nj, dh_rows, DH, base, cap_p, T, dt);
+  si->fields["QQ"] = dbl(n, n, QQ);
+  if (lim) si->fields["lim"] = dbl(nj, 1, lim);
+  if (max_input) si->fields["MAX_input"] = dbl(n, 1, max_input);
+  si->fields["xR"] = dbl(2 * nj, B, xR);
+  si->fields["ff"] = dbl(n, B, ff);
+  si->fields["caug"] = dbl(1, B, caug);
+  si->fields["x_"] = dbl(2 * n, B, xref);
+  si->fields["epsilon_O"] = dbl(1, 1, &eps_outer);
+  si->fields["MAX_O_ITER"] = dbl(1, 1, &Kd);
+  const mxArray *prhs[10] = {chr("solve_checked"), chr(solver), chr(grad), chr(robot_name), obs_cell(nobs, obs_l, obs_D, obs_eps), si,
+                             dbl(0, 0, nullptr), dbl(1, 1, &eta), dbl(1, 1, &rd), dbl(1, 1, &gain)};
+  mxArray *plhs[11] = {nullptr};
+  int rc = 0;
+  try {
+    mexFunction(11, plhs, 10, prhs);
+    std::memcpy(u, plhs[0]->d.data(), sizeof(double) * n * B);
+    std::memcpy(x, plhs[1]->d.data(), sizeof(double) * 2 * n * B);
+    std::memcpy(cost, plhs[2]->d.data(), sizeof(double) * max_outer * B);
+    std::memcpy(eu, plhs[3]->d.data(), sizeof(double) * max_outer * B);
+    std::memcpy(iters, plhs[4]->i32.data(), sizeof(int) * B);
+    std::memcpy(status, plhs[5]->i32.data(), sizeof(int) * B);
+    std::memcpy(verdict, plhs[6]->i32.data(), sizeof(int) * B);
+    std::memcpy(t_hit, plhs[7]->d.data(), sizeof(double) * B);
+    std::memcpy(cmin, plhs[8]->d.data(), sizeof(double) * B);
+    std::memcpy(rounds_used, plhs[9]->i32.data(), sizeof(int) * B);
+    std::memcpy(margin_off, plhs[10]->d.data(), sizeof(double) * (size_t)nobs * H * B);
+  } catch (const mex_error &e) {
+    snprintf(g_err, sizeof(g_err), "%s: %s", e.id.c_str(), e.msg.c_str());
+    rc = 1;
+  }
+  return finish(rc);
+}
