@@ -229,7 +229,9 @@ __device__ __forceinline__ int w_scan(const WView &s, const WDims &P, int &maske
     double accA0 = 0.0, accA1 = 0.0, accB0 = 0.0, accB1 = 0.0;
     const bool hasA = j0 < O, hasB = j0 + 1 < O;
     const double *cA = s.ocoef + ((size_t)j0 * H + i0) * NJ, *cB = cA + (size_t)H * NJ;
-#pragma unroll
+    // one joint's scans per trip: the unrolled form (the NJ independent scans interleaved) is ~1 000 instructions more
+    // of the QP's hot loop and measured slower (DESIGN.md section 4b)
+#pragma unroll 1
     for (int k = 0; k < NJ; ++k) {
       const double a0 = v0 ? s.uq[i0 * NJ + k] : 0.0, a1 = v1 ? s.uq[i1 * NJ + k] : 0.0;
       double s0, s1, t0, t1;
