@@ -100,6 +100,20 @@ int cfs_set_obstacles_ex(cfs_ctx *ctx, const double *seg /*3x2xn_obs*/, const in
 int cfs_set_cost(cfs_ctx *ctx, int H, const double *QQ /*n x n, n=H*n_joints*/, const double *lim /*n_joints*/,
                  const double *max_input /*n*/);
 
+/* Joint position limits (extension: the reference has none, robotproperty2.m).  qmin / qmax: n_joints entries each, or both
+ * NULL to clear the limits.  qmin_k may be -INFINITY and qmax_k +INFINITY for a joint without that side.  CFS_E_ARG if only
+ * one pointer is NULL, an entry is NaN, qmin_k > qmax_k, qmin_k = +INFINITY or qmax_k = -INFINITY (a limit no position meets);
+ * CFS_E_STATE without a robot.  cfs_set_robot clears the limits.
+ * With limits set, the QP of every CFS and PSGCFS solve (cfs_solve_batch*, cfs_solve_start_goal*, cfs_solve_routes*,
+ * cfs_solve_batch_margins*, every round of cfs_solve_checked*; both gradient modes) also has, for every waypoint i = 1..H and
+ * joint k, the rows theta_i,k <= qmax_k and -theta_i,k <= -qmin_k, theta_i the roll-out of u from x0 (waypoint 0 is x0 and is
+ * not constrained); an infinite bound gives a row that can never be violated.  Nothing else changes: stop rule, cost, status
+ * codes, the reference's rows.  The limits hold at the waypoints only: theta is quadratic on a segment and may overshoot a
+ * limit both of its ends satisfy.  A start outside the limits gives what the QP gives, normally CFS_STATUS_INFEASIBLE.
+ * cfs_get_con appends the 2n rows (upper rows, then lower rows, [waypoint][joint] order).  cfs_chomp_batch, the unconstrained
+ * baseline, does not read the limits. */
+int cfs_set_joint_limits(cfs_ctx *ctx, const double *qmin /*n_joints or NULL*/, const double *qmax /*n_joints or NULL*/);
+
 /* Same as cfs_set_cost with QQ built ON THE DEVICE from the blocks the mains assemble it from (main_FANUC.m:64-97,
  * RRTstar_CFS.m:124-160, main_2L.m:69-92): QQ = Baug'*Qaug*Baug + r_scale*(R+R'), Qaug = blkdiag(stage_w*Q ... term_w*Q),
  * R = blkdiag(Rblk).  Enables cfs_solve_start_goal.  (SURVEY.md section 8f, N2.) */
@@ -160,7 +174,8 @@ int cfs_solve_routes_device(cfs_ctx *ctx, int B, int W, const int *route_len, in
 /* The resampling step alone: sampled (nj x (H+1) x B) = cubicpolytraj(route, (0:W-1)*dt, linspace(0,(W-1)*dt,H+1)). */
 int cfs_resample_routes(cfs_ctx *ctx, int B, int W, int H, const double *routes /*nj x W x B*/, double *sampled);
 /* CHOMP_FANUC(obs, sys_info, uu, ROBOT).optimizer()  (Lib/CHOMP_FANUC.m:54-165), the gradient-descent baseline planner of the
- * reference (SURVEY.md section 8f, N4), for B problems that share robot, obstacles and cost:
+ * reference (SURVEY.md section 8f, N4), for B problems that share robot, obstacles and cost.  Unconstrained: it does not
+ * read the joint limits of cfs_set_joint_limits.
  *   u_init = uu (n x B), xref = sys_info.x_, alpha = sys_info.alpha; obs{j}.D / obs{j}.epsilon from cfs_set_obstacles.
  *   Every outer iteration: dm_f per link (:115-134), derivest gradient of dist_link_*(linkid) (:151,:156), the update
  *   u <- u - alpha*3*(QQ*u + ff + 2000*dcostObs) (:75), roll-out, cost_all(k) = get_cost(u) + fobs_m() (:63).
@@ -194,7 +209,8 @@ int cfs_time_dist_grad(cfs_ctx *ctx, int N, int grad_mode, const double *theta /
 
 /* CFS_FANUC.get_con (Lib/CFS_FANUC.m:101-135) for ONE problem, dense and in the reference's row order
  * (per obstacle j, step i: 1 obstacle row, nj rows +Baug_w, nj rows -Baug_w).  Ainq is m x n column-major,
- * m = n_obs*H*(1+2nj) (or n_obs*H when no lim was set).  margin_is_D: 0 -> obs.epsilon (CFS), 1 -> obs.D (PSGCFS). */
+ * m = n_obs*H*(1+2nj) (or n_obs*H when no lim was set), plus 2n joint position rows after them when joint limits are set
+ * (cfs_set_joint_limits).  margin_is_D: 0 -> obs.epsilon (CFS), 1 -> obs.D (PSGCFS). */
 int cfs_get_con(cfs_ctx *ctx, int grad_mode, int margin_is_D, const double *x0, const double *xcur /*2njH*/,
                 const double *u /*n*/, double *Ainq, double *binq);
 

@@ -41,6 +41,9 @@
 //                           cfs_mex('device', mod(labindex - 1, gpuDeviceCount)), see matlab/s_Parallel_rrt.m).
 //                           Default: environment variable CFS_DEVICE, else 0.
 //
+// 'solve', 'solve_checked' and 'routes' read the optional sys_info.qlim (njoint x 2 = [min max] per joint): joint position limits of the
+// CFS / PSGCFS solve (extension, include/cfs_b200.h cfs_set_joint_limits); a call without it solves without limits.
+//
 // Robot, obstacles and cost are cached by content hash: the Cholesky factor + Gram operator of cfs_set_cost (3.9 ms at
 // n = 250) are rebuilt only when QQ / lim / MAX_input / H / robot really change between calls.
 // Build (on a machine with MATLAB; this container has no mex.h, so the file is shipped as source and compiled against
@@ -183,6 +186,16 @@ static void out_int(mxArray *&dst, const std::vector<int> &v) {
 }
 
 // ---- 'solve' ------------------------------------------------------------------------------------------------------------------
+// joint position limits (extension, cfs_set_joint_limits) from the optional sys_info.qlim = [min max] per joint (njoint x 2),
+// set or cleared by every command that solves (si == nullptr: cleared): the cached context never keeps the limits of an
+// earlier call
+static void bind_qlim(const mxArray *si, int nj) {
+  const mxArray *ql = si ? field(si, "qlim", false) : nullptr;
+  if (ql && (mxGetM(ql) != (size_t)nj || mxGetN(ql) != 2)) mexErrMsgIdAndTxt("cfs:arg", "sys_info.qlim must be njoint x 2 ([min max])");
+  const double *qlp = ql ? dbl(ql, 2 * (size_t)nj, "sys_info.qlim (njoint x 2)") : nullptr;
+  check(cfs_set_joint_limits(g_ctx, qlp, qlp ? qlp + nj : nullptr), "cfs_set_joint_limits");
+}
+
 // checked: the 'solve_checked' command (cfs_solve_checked), prhs[6..8] = eta, rounds, gain (optional)
 static void cmd_solve(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[], bool checked = false) {
   if (nrhs < 5)
@@ -216,6 +229,7 @@ static void cmd_solve(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]
     check(cfs_set_cost(g_ctx, H, QQ, limp, mip), "cfs_set_cost");
     g_hash_cost = h;
   }
+  bind_qlim(chomp ? nullptr : si, nj);  // CHOMP does not read the limits
   // ---- the batch ----------------------------------------------------------------------------------------------------
   const mxArray *xR = field(si, "xR"), *ff = field(si, "ff"), *caug = field(si, "caug"), *xref = field(si, "x_");
   const size_t B = mxGetNumberOfElements(caug);
@@ -373,6 +387,7 @@ static void cmd_routes(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[
     check(cfs_set_cost_blocks(g_ctx, H, Q, Rb, r_scale, 0.1, 10000.0, limp, mip), "cfs_set_cost_blocks");  // RRTstar_CFS.m:139-150
     g_hash_cost = h;
   }
+  bind_qlim(si, nj);
   const int K = (int)scalar(field(si, "MAX_O_ITER"), "sys_info.MAX_O_ITER");
   plhs[0] = mxCreateDoubleMatrix(n, B, mxREAL);
   mxArray *x = mxCreateDoubleMatrix(2 * n, B, mxREAL), *cost = mxCreateDoubleMatrix(K > 0 ? K : 1, B, mxREAL),

@@ -23,7 +23,8 @@ SYMBOLS = ["cfs_create", "cfs_destroy", "cfs_last_error", "cfs_version", "cfs_se
            "cfs_set_cost", "cfs_set_cost_blocks", "cfs_solve_start_goal", "cfs_solve_start_goal_async", "cfs_solve_routes", "cfs_solve_routes_async", "cfs_solve_routes_var", "cfs_solve_routes_var_async", "cfs_solve_routes_device", "cfs_resample_routes", "cfs_solve_batch", "cfs_solve_batch_async", "cfs_chomp_batch", "cfs_wait", "cfs_solve_batch_device", "cfs_dist_grad", "cfs_time_dist_grad", "cfs_get_con",
            "cfs_nodes_feasible", "cfs_nearest_steer", "cfs_rrt_find_routes", "cfs_rrt_find_routes_device", "cfs_get_stats", "cfs_set_timing", "cfs_get_iter_times", "cfs_get_problem_steps", "cfs_get_qp_profile", "cfs_get_warp_profile", "cfs_measure_fp64_peak",
            "cfs_check_edges", "cfs_check_trajectories", "cfs_check_edges_device", "cfs_check_trajectories_device",
-           "cfs_solve_batch_margins", "cfs_solve_batch_margins_device", "cfs_solve_checked", "cfs_solve_checked_device"]
+           "cfs_solve_batch_margins", "cfs_solve_batch_margins_device", "cfs_solve_checked", "cfs_solve_checked_device",
+           "cfs_set_joint_limits"]
 
 
 class CfsError(RuntimeError):
@@ -79,6 +80,7 @@ class Context:
         self.device = device
         self.nj = self.H = self.n = self.nobs = 0
         self.has_lim = False
+        self.has_qlim = False
 
     def close(self):
         if getattr(self, "_h", None):
@@ -109,6 +111,19 @@ class Context:
                                      _dp(cap), C.c_int(njoint), _dp(T), C.c_double(robot["delta_t"]))
         self._check(rc, "cfs_set_robot")
         self.nj = njoint
+        self.has_qlim = False  # cfs_set_robot clears the joint limits
+
+    def set_joint_limits(self, qmin, qmax):
+        """Joint position limits of every following CFS / PSGCFS solve (cfs_set_joint_limits): qmin, qmax (nj,), +-inf for a side
+        without a limit; set_joint_limits(None, None) clears them."""
+        lo = None if qmin is None else _f64(np.asarray(qmin, dtype=np.float64).reshape(-1))
+        hi = None if qmax is None else _f64(np.asarray(qmax, dtype=np.float64).reshape(-1))
+        for v in (lo, hi):
+            if v is not None and v.shape[0] != self.nj:
+                raise CfsError("set_joint_limits: expected %d entries, got %d" % (self.nj, v.shape[0]))
+        rc = self._lib.cfs_set_joint_limits(self._h, _dp(lo), _dp(hi))
+        self._check(rc, "cfs_set_joint_limits")
+        self.has_qlim = lo is not None
 
     def set_obstacles(self, obs):
         """obs: list of dicts with l (3x2), D, epsilon (main_FANUC.m:56-60).  shape == 'box' (extension): l = [min corner, max
@@ -395,7 +410,7 @@ class Context:
         return ms.value
 
     def get_con(self, x0, xcur, u, grad=GRAD_NUMJAC, margin_is_D=False):
-        m = self.nobs * self.H * ((1 + 2 * self.nj) if self.has_lim else 1)
+        m = self.nobs * self.H * ((1 + 2 * self.nj) if self.has_lim else 1) + (2 * self.n if self.has_qlim else 0)
         A = np.zeros((m, self.n), order="F")
         b = np.zeros(m)
         rc = self._lib.cfs_get_con(self._h, C.c_int(grad), C.c_int(1 if margin_is_D else 0), _dp(_f64(x0)),

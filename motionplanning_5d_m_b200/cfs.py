@@ -27,6 +27,17 @@ class EVAL:
         return 0.5 * u @ s["Qaug"] @ u + s["paug"] @ u + s["caug"]
 
 
+def _apply_qlim(ctx, sys_info):
+    """Joint position limits from the optional sys_info["qlim"] (nj x 2, [min max] per joint; +-inf for a side without a
+    limit), or none: a context shared between calls never keeps the limits of an earlier one."""
+    q = sys_info.get("qlim")
+    if q is None:
+        ctx.set_joint_limits(None, None)
+    else:
+        q = np.asarray(q, dtype=np.float64).reshape(-1, 2)
+        ctx.set_joint_limits(q[:, 0], q[:, 1])
+
+
 class _SolverBase:
     SOLVER = _lib.SOLVER_CFS
     GRAD = _lib.GRAD_NUMJAC
@@ -55,6 +66,7 @@ class _SolverBase:
         ctx.set_robot(robot, s["njoint"])
         ctx.set_obstacles(self.obs)
         ctx.set_cost(s["H"], s["QQ"], s.get("lim"), s.get("MAX_input") if self.SOLVER == _lib.SOLVER_CFS else None)
+        _apply_qlim(ctx, s)
         return ctx
 
     def optimizer(self, noise=None, rng=None, check=None):
@@ -149,8 +161,10 @@ class BatchCFS:
 
     def optimizer(self, x0, ff, caug, xref, noise=None, check=None):
         """check=None: the plain batched solve.  check=dict(eta=1e-3, rounds=4, gain=2.0, max_evals=4096) (any subset): the
-        checked solve (Context.solve_checked), whose result adds verdict, t_hit, cmin, rounds_used and margin_off."""
+        checked solve (Context.solve_checked), whose result adds verdict, t_hit, cmin, rounds_used and margin_off.  Joint
+        position limits: sys_info["qlim"] (optional), applied to the context on every call."""
         s = self.sys_info
+        _apply_qlim(self.ctx, s)
         if check is not None:
             return self.ctx.solve_checked(x0, ff, caug, xref, float(s["epsilon_O"]), int(s["MAX_O_ITER"]), solver=self.solver,
                                           grad=self.grad, noise=noise, alpha=float(s.get("alpha", 0.0)), **dict(check))

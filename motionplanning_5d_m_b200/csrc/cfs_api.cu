@@ -56,6 +56,10 @@ struct cfs_ctx {
   // cost
   int H = 0, n = 0;
   bool has_lim = false, has_bounds = false;
+  // joint position limits (cfs_set_joint_limits): [qmax | qmin] (CFS_MAXL each) on the host and the device
+  bool has_qlim = false;
+  double hqlim[2 * CFS_MAXL] = {0};
+  double *dqlim = nullptr;
   double qq_norm_inf = 0.0;
   double *dQQraw = nullptr;  // QQ exactly as given (PSGCFS gradient); dQQ holds (QQ+QQ')/2
   double *dQQ = nullptr, *dG = nullptr, *dgn = nullptr, *dGI = nullptr, *dgnI = nullptr;
@@ -70,7 +74,7 @@ struct cfs_ctx {
   // batch buffers
   DevBuf x0, ff, caug, xref, noise, u, x, cost, eu, u0, v0, cost0, dist, grad, lid, iters, status, flags, listA, listB,
       counters, slab, scratch_theta, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen, rrt_in,
-      chk_in, chk_out, chk_seg, chk_ctr, rep_off, rep_offo, rep_in, rep_out, rep_list;
+      chk_in, chk_out, chk_seg, chk_ctr, rep_off, rep_offo, rep_in, rep_out, rep_list, zero_off;
   int slab_grid = 0, slab_ld = 0;
   // pinned staging of the host-pointer entries: pageable caller buffers (MATLAB's mxGetPr memory, numpy arrays) are copied
   // through these so that cudaMemcpyAsync stays asynchronous; pinned / registered caller buffers are used in place
@@ -275,9 +279,10 @@ extern "C" void cfs_destroy(cfs_ctx *ctx) {
                     &ctx->scratch_out, &ctx->qpsteps, &ctx->fupper, &ctx->probsteps, &ctx->routes, &ctx->psg_w, &ctx->psg_cost,
                     &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen, &ctx->rrt_in,
                     &ctx->chk_in, &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr, &ctx->rep_off, &ctx->rep_offo, &ctx->rep_in,
-                    &ctx->rep_out, &ctx->rep_list};
+                    &ctx->rep_out, &ctx->rep_list, &ctx->zero_off};
   for (DevBuf *b : bufs) free_buf(*b);
   if (ctx->dQblk) cudaFree(ctx->dQblk);
+  if (ctx->dqlim) cudaFree(ctx->dqlim);
   double *ds[] = {ctx->dQQraw, ctx->dQQ, ctx->dG, ctx->dgn, ctx->dGI, ctx->dgnI, ctx->dlim, ctx->dumax, ctx->dworkL, ctx->dworkY};
   for (double *d : ds)
     if (d) cudaFree(d);
@@ -368,6 +373,8 @@ extern "C" int cfs_set_robot(cfs_ctx *ctx, int robot_kind, const double *DH, int
   t.nj = n_joints;
   motion_bound(t, n_joints, ctx->motion_R);
   ctx->nj = n_joints;
+  ctx->has_qlim = false;  // nj may change
+  for (double &v : ctx->hqlim) v = 0.0;
   ctx->have_robot = true;
   ctx->have_cost = false;  // n depends on nj
   return upload_tables(ctx);
@@ -411,6 +418,33 @@ extern "C" int cfs_set_obstacles_ex(cfs_ctx *ctx, const double *seg, const int *
 
 extern "C" int cfs_set_obstacles(cfs_ctx *ctx, const double *seg, const double *D, const double *eps, int n_obs) {
   return cfs_set_obstacles_ex(ctx, seg, nullptr, D, eps, n_obs);
+}
+
+extern "C" int cfs_set_joint_limits(cfs_ctx *ctx, const double *qmin, const double *qmax) {
+  if (!ctx) return CFS_E_ARG;
+  if (!ctx->have_robot) return fail(ctx, CFS_E_STATE, "cfs_set_joint_limits: call cfs_set_robot first");
+  if (!qmin != !qmax) return fail(ctx, CFS_E_ARG, "cfs_set_joint_limits: qmin and qmax must both be given or both be NULL");
+  const int nj = ctx->nj;
+  if (!qmin) {
+    ctx->has_qlim = false;
+    for (double &v : ctx->hqlim) v = 0.0;
+    return 0;
+  }
+  for (int k = 0; k < nj; ++k)
+    if (qmin[k] != qmin[k] || qmax[k] != qmax[k] || !(qmin[k] <= qmax[k]) || qmin[k] == INFINITY || qmax[k] == -INFINITY)
+      return fail(ctx, CFS_E_ARG, "cfs_set_joint_limits: joint %d has qmin = %g, qmax = %g", k, qmin[k], qmax[k]);
+  CU(cudaSetDevice(ctx->device));
+  if (!ctx->dqlim) CU(cudaMalloc(&ctx->dqlim, sizeof(double) * 2 * CFS_MAXL));
+  double h[2 * CFS_MAXL] = {0};
+  for (int k = 0; k < nj; ++k) {  // the kernels' layout: qmax (nj) | qmin (nj)
+    h[k] = qmax[k];
+    h[nj + k] = qmin[k];
+  }
+  CU(cudaMemcpyAsync(ctx->dqlim, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  for (int k = 0; k < 2 * CFS_MAXL; ++k) ctx->hqlim[k] = h[k];
+  ctx->has_qlim = true;
+  return 0;
 }
 
 extern "C" int cfs_set_cost(cfs_ctx *ctx, int H, const double *QQ, const double *lim, const double *max_input) {
@@ -581,6 +615,17 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
   a.prof = ctx->timing_level >= 3 ? ptr<long long>(ctx->qpsteps) + 8 : nullptr;
   a.slab_ld = n;
   a.margin_off = O > 0 ? margin_off : nullptr;  // non-null selects the offset instantiations of every solver kernel
+  if (ctx->has_qlim) {
+    // the joint-limit instantiations are offset instantiations too: without offsets they read zeros, and dist - (m + 0.0)
+    // equals dist - m bit for bit
+    a.qlim = ctx->dqlim;
+    if (!a.margin_off) {
+      const size_t ne = (size_t)(OH > 0 ? OH : 1) * B;
+      if ((rc = ensure(ctx, ctx->zero_off, sizeof(double) * ne))) return rc;
+      CU(cudaMemsetAsync(ctx->zero_off.p, 0, sizeof(double) * ne, st));
+      a.margin_off = ptr<double>(ctx->zero_off);
+    }
+  }
 
   const bool fused = ctx->use_fused && !psg && grad == CFS_GRAD_NUMJAC && fused_supported(a);
   // bulk tier of the fused solver: one warp per problem (k_warp.cu) when its shared-memory regions fit
@@ -591,7 +636,8 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
     // direction slots in shared memory: the count that keeps the most problems resident per SM (ties: more slots); cached per
     // (n, obstacles, CTA shape)
     const long long key = ((long long)n << 24) ^ ((long long)O << 16) ^ ((long long)ctx->warp_cfg << 8) ^ ctx->warp_zs ^
-                          (a.margin_off ? 1LL << 48 : 0);  // the offset instantiations have kernel attributes of their own
+                          (a.margin_off ? 1LL << 48 : 0) ^  // the offset instantiations have kernel attributes of their own
+                          (a.qlim ? 1LL << 49 : 0);         // ... and so have the joint-limit ones
     if (key != ctx->warp_key) {
       ctx->warp_key = key;
       ctx->warp_zs_pick = 0;
@@ -1472,6 +1518,35 @@ extern "C" int cfs_get_con(cfs_ctx *ctx, int grad_mode, int margin_is_D, const d
   CU(cudaSetDevice(ctx->device));
   const int nj = ctx->nj, H = ctx->H, n = ctx->n, O = ctx->nobs, OH = O * H;
   const int m = OH * (ctx->has_lim ? 1 + 2 * nj : 1);
+  if (ctx->has_qlim) {  // joint position rows after the reference's rows: theta_(i+1),k <= qmax_k, then -theta_(i+1),k <= -qmin_k
+    const int mt = m + 2 * n;
+    std::vector<double> A0((size_t)m * n), b0(m);
+    if (m > 0) {
+      ctx->has_qlim = false;
+      rc = cfs_get_con(ctx, grad_mode, margin_is_D, x0, xcur, u, A0.data(), b0.data());
+      ctx->has_qlim = true;
+      if (rc) return rc;
+    }
+    const double dt = ctx->htab.dt;
+    for (int c = 0; c < n; ++c) {
+      for (int r = 0; r < m; ++r) Ainq[r + (size_t)mt * c] = A0[r + (size_t)m * c];
+      const int jj = c / nj, kc = c - jj * nj;
+      for (int e = 0; e < n; ++e) {
+        const int i = e / nj, k = e - i * nj;
+        const double v = (k == kc && jj <= i) ? (0.5 * dt * dt + ((i - jj) * dt) * dt) : 0.0;
+        Ainq[m + e + (size_t)mt * c] = v;
+        Ainq[m + n + e + (size_t)mt * c] = -v;
+      }
+    }
+    for (int r = 0; r < m; ++r) binq[r] = b0[r];
+    for (int e = 0; e < n; ++e) {
+      const int i = e / nj, k = e - i * nj;
+      const double fm = x0[k] + ((i + 1) * dt) * x0[nj + k];
+      binq[m + e] = ctx->hqlim[k] - fm;
+      binq[m + n + e] = fm - ctx->hqlim[nj + k];
+    }
+    return 0;
+  }
   if (m == 0) return 0;
   cudaStream_t st = ctx->stream;
   const size_t in_d = (size_t)2 * nj + 2 * n + n;

@@ -193,6 +193,11 @@ struct SolveArgs {
   // launch wrappers pick them when margin_off != nullptr), so the kernels launched without offsets are unchanged.  Last member:
   // the parameter offsets of every other field stay where they were.
   const double *margin_off;
+  // joint position limits [qmax (nj) | qmin (nj)] on the device, +-inf for a side without a limit, or nullptr: every QP gets the
+  // rows theta_(i+1),k <= qmax_k and -theta_(i+1),k <= -qmin_k (ids OH + 4n + 2e + neg, e = i nj + k; DESIGN.md section 3d).
+  // Read only by the limit instantiations, which are also margin-offset instantiations: the launch wrappers require margin_off
+  // (a zero buffer when the solve has no offsets) whenever qlim is set.  Last member, like margin_off.
+  const double *qlim;
 };
 cudaError_t launch_solve_init(const SolveArgs &a, cudaStream_t s);
 cudaError_t launch_v0(const SolveArgs &a, cudaStream_t s);

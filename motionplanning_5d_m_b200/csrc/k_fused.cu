@@ -44,10 +44,10 @@ struct FusedLayout {
   size_t qp_bytes, xs, us, tab, mbar, total;
 };
 
-__host__ __device__ inline FusedLayout fused_layout(int n, int nj, int OH, int m, int qs, int nt, int qz) {
+__host__ __device__ inline FusedLayout fused_layout(int n, int nj, int OH, int m, int qs, int nt, int qz, bool lim = false) {
   FusedLayout L;
   size_t off[QP_NOFF];
-  L.qp_bytes = qp_smem_layout(n, nj, OH, m, off, qs, nt, qz);
+  L.qp_bytes = qp_smem_layout(n, nj, OH, m, off, qs, nt, qz, lim);
   size_t o = L.qp_bytes;
   L.xs = o; o += sizeof(double) * 2 * n;
   L.us = o; o += sizeof(double) * n;
@@ -59,14 +59,14 @@ __host__ __device__ inline FusedLayout fused_layout(int n, int nj, int OH, int m
 }
 
 // OFF: the obstacle rows read a.margin_off (per-waypoint margin offsets of the checked solve); a separate instantiation, the one
-// without it is unchanged
-template <int NJ, int NT, int QS, int MINB, int QZ, int MAXREG = (MINB == 1 ? 255 : 168), bool OFF = false>
+// without it is unchanged.  LIM (only with OFF): the QP also has the joint position rows of a.qlim.
+template <int NJ, int NT, int QS, int MINB, int QZ, int MAXREG = (MINB == 1 ? 255 : 168), bool OFF = false, bool LIM = false>
 __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  const int n = a.n, nj = NJ, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + 4 * n, N = 2 * n;
+  const int n = a.n, nj = NJ, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + (LIM ? 6 : 4) * n, N = 2 * n;
   const int tid = threadIdx.x;
-  const FusedLayout L = fused_layout(n, nj, OH, m, QS, NT, QZ);
-  const QpView s = qp_view(smem_raw, n, nj, OH, m, QS, NT, QZ);
+  const FusedLayout L = fused_layout(n, nj, OH, m, QS, NT, QZ, LIM);
+  const QpView s = qp_view(smem_raw, n, nj, OH, m, QS, NT, QZ, LIM);
   const bool heavy = a.tier == 1;
   double *xs = reinterpret_cast<double *>(smem_raw + L.xs);  // x_  (CFS_FANUC.m:55)
   double *us = reinterpret_cast<double *>(smem_raw + L.us);  // u   (CFS_FANUC.m:56)
@@ -134,6 +134,11 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs 
     if (tid < 8) {
       s.lim[tid] = (tid < nj && has_vel) ? a.lim[tid] : 0.0;
       s.w0[tid] = (tid < nj) ? x0[nj + tid] : 0.0;
+      if (LIM) {  // qmax | qmin | theta0 of the joint position rows
+        s.lim[8 + tid] = (tid < nj) ? a.qlim[tid] : 0.0;
+        s.lim[16 + tid] = (tid < nj) ? a.qlim[nj + tid] : 0.0;
+        s.lim[24 + tid] = (tid < nj) ? x0[tid] : 0.0;
+      }
     }
     const double nrm0 = sqrt(block_sum<NT>(part, s.red));
     const double cost0 = a.cost0[b];
@@ -224,7 +229,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs 
       // ---- Solve_QP (CFS_FANUC.m:85) ----
       int q = 0, steps = 0;
       const int masked = qp_mask_antiparallel<NT>(s, dims);
-      const int qst = qp_solve<NT, QS, (MINB == 1), NJ, QZ>(s, dims, cost0, fupper, false, q, steps, qmax_seen, pf, tck, prof,
+      const int qst = qp_solve<NT, QS, (MINB == 1), NJ, QZ, LIM>(s, dims, cost0, fupper, false, q, steps, qmax_seen, pf, tck, prof,
                                                         heavy ? 0x7fffffff : a.esc_steps, masked);
       steps_total += steps;
       steps_prob += steps;
@@ -244,7 +249,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_fused(SolveArgs 
       const double e_u = sqrt(block_sum<NT>(pe, s.red));
       double pc = 0.0;
 #pragma unroll 1
-      for (int w = tid; w < q; w += NT) pc -= s.lam[w] * slack_at<NJ>(s.act[w], dims, s, s.v0s);
+      for (int w = tid; w < q; w += NT) pc -= s.lam[w] * slack_at<NJ, LIM>(s.act[w], dims, s, s.v0s);
       const double cost = cost0 + 0.5 * block_sum<NT>(pc, s.red);
       double px = 0.0;
       if (tid < nj) {
@@ -313,7 +318,8 @@ size_t fused_smem_bytes(const SolveArgs &a, int tier) {
   int nt, qs, qz;
   tier_cfg(tier, nt, qs, qz);
   const int OH = a.nobs * a.H;
-  return fused_layout(a.n, a.nj, OH, OH + 4 * a.n, qs, nt, qz).total;
+  const bool lim = a.qlim != nullptr;
+  return fused_layout(a.n, a.nj, OH, OH + (lim ? 6 : 4) * a.n, qs, nt, qz, lim).total;
 }
 
 bool fused_supported(const SolveArgs &a) {
@@ -342,17 +348,19 @@ static int grid_of(K kernel, int nt, size_t smem, int device) {
 }
 
 typedef void (*FusedKernel)(SolveArgs);
-template <int NJ, bool OFF>
+template <int NJ, bool OFF, bool LIM = false>
 static FusedKernel fused_kernel_nj(int tier) {
-  if (tier == 0) return k_cfs_fused<NJ, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ, 168, OFF>;
-  if (tier == 1) return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0, 255, OFF>;
-  return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168, OFF>;
+  if (tier == 0) return k_cfs_fused<NJ, FUSED_BULK_NT, FUSED_BULK_QS, 3, FUSED_BULK_QZ, 168, OFF, LIM>;
+  if (tier == 1) return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_HEAVY_QS, 1, 0, 255, OFF, LIM>;
+  return k_cfs_fused<NJ, FUSED_HEAVY_NT, FUSED_SLIM_QS, 1, 0, 168, OFF, LIM>;
 }
-// tier 0 bulk, 1 heavy, 2 slim heavy; the margin-offset instantiations when a.margin_off is set
+// tier 0 bulk, 1 heavy, 2 slim heavy; the margin-offset instantiations when a.margin_off is set, the joint-limit ones (which
+// also read the offsets) when a.qlim is set
 static FusedKernel fused_kernel(const SolveArgs &a, int tier) {
-  const bool off = a.margin_off != nullptr;
-  if (a.nj == 2) return off ? fused_kernel_nj<2, true>(tier) : fused_kernel_nj<2, false>(tier);
-  if (a.nj == 5) return off ? fused_kernel_nj<5, true>(tier) : fused_kernel_nj<5, false>(tier);
+  const bool off = a.margin_off != nullptr, lim = a.qlim != nullptr;
+  if (lim && !off) return nullptr;
+  if (a.nj == 2) return lim ? fused_kernel_nj<2, true, true>(tier) : (off ? fused_kernel_nj<2, true>(tier) : fused_kernel_nj<2, false>(tier));
+  if (a.nj == 5) return lim ? fused_kernel_nj<5, true, true>(tier) : (off ? fused_kernel_nj<5, true>(tier) : fused_kernel_nj<5, false>(tier));
   return nullptr;
 }
 

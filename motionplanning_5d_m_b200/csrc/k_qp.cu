@@ -28,7 +28,8 @@ namespace cfs {
 size_t qp_smem_bytes(const SolveArgs &a) {
   size_t off[QP_NOFF];
   const int OH = a.nobs * a.H;
-  return qp_smem_layout(a.n, a.nj, OH, OH + 4 * a.n, off);
+  const bool lim = a.qlim != nullptr;
+  return qp_smem_layout(a.n, a.nj, OH, OH + (lim ? 6 : 4) * a.n, off, QP_QS, QP_THREADS, 0, lim);
 }
 
 
@@ -36,13 +37,13 @@ size_t qp_smem_bytes(const SolveArgs &a) {
 // The kernel
 // ============================================================================================================
 // OFF: the obstacle rows read a.margin_off (per-waypoint margin offsets of the checked solve); a separate instantiation, the one
-// without it is unchanged
-template <bool OFF>
+// without it is unchanged.  LIM (only with OFF): the QP also has the joint position rows of a.qlim.
+template <bool OFF, bool LIM = false>
 __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int n = a.n, nj = a.nj, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + 4 * n;
+  const int n = a.n, nj = a.nj, H = a.H, np = 3 * n, OH = a.nobs * H, m = OH + (LIM ? 6 : 4) * n;
   const int tid = threadIdx.x;
-  const QpView s = qp_view(smem_raw, n, nj, OH, m);
+  const QpView s = qp_view(smem_raw, n, nj, OH, m, QP_QS, QP_THREADS, 0, LIM);
   const double *__restrict__ G = a.G;
   const double *__restrict__ gnorm = a.gdiag;  // sqrt(diag(G))
   const int has_vel = a.has_lim, has_bnd = a.has_bounds;
@@ -86,6 +87,11 @@ __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
     if (tid < 8) {
       s.lim[tid] = (tid < nj && has_vel) ? a.lim[tid] : 0.0;
       s.w0[tid] = (tid < nj) ? x0[nj + tid] : 0.0;
+      if (LIM) {  // qmax | qmin | theta0 of the joint position rows
+        s.lim[8 + tid] = (tid < nj) ? a.qlim[tid] : 0.0;
+        s.lim[16 + tid] = (tid < nj) ? a.qlim[nj + tid] : 0.0;
+        s.lim[24 + tid] = (tid < nj) ? x0[tid] : 0.0;
+      }
     }
     // disp(i,k) = (Bj(1:njoint,:)*u)(k) of CFS_FANUC.m:120 -> s.g.  In the first outer iteration u = 0 (CFS_FANUC.m:56)
     // while x_ is the reference line; afterwards x_ is the roll-out of u, so B_theta u = theta_i - (theta_0 + i dt w_0).
@@ -141,7 +147,7 @@ __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
       }
       fup = a.cost0[b] + 0.5 * block_sum<QP_THREADS>(part, s.red) * (1.0 + 1e-9);
     }
-    const int status = qp_solve<QP_THREADS, QP_QS, true, 0>(s, dims, a.cost0[b], fup, skip_solve, q, steps,
+    const int status = qp_solve<QP_THREADS, QP_QS, true, 0, 0, LIM>(s, dims, a.cost0[b], fup, skip_solve, q, steps,
                                 qmax_seen, pf, tck, prof, 0x7fffffff, masked);
     steps_total += steps;
     if (tid == 0 && a.prob_steps) a.prob_steps[b] += steps;
@@ -161,7 +167,7 @@ __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
       // cost by duality: f(u) = f(u0) + 1/2 sum_w lam_w * (c_w u0 - rhs_w)
       double pc = 0.0;
       for (int w = tid; w < q; w += QP_THREADS) {
-        const double val0 = -slack_at<0>(s.act[w], dims, s, s.v0s);
+        const double val0 = -slack_at<0, LIM>(s.act[w], dims, s, s.v0s);
         pc += s.lam[w] * val0;
       }
       const double cost = psg ? 0.0 : a.cost0[b] + 0.5 * block_sum<QP_THREADS>(pc, s.red);  // PSGCFS: k_psg_cost
@@ -218,11 +224,18 @@ __global__ void __launch_bounds__(QP_THREADS, 3) k_qp(SolveArgs a) {
   }
 }
 
+// the margin-offset instantiation when a.margin_off is set, the joint-limit one (which also reads the offsets) when a.qlim is set
+static void (*qp_kernel(const SolveArgs &a))(SolveArgs) {
+  if (a.qlim) return a.margin_off ? k_qp<true, true> : nullptr;
+  return a.margin_off ? k_qp<true> : k_qp<false>;
+}
+
 int qp_max_grid(const SolveArgs &a, int device) {
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   const size_t smem = qp_smem_bytes(a);
-  void (*k)(SolveArgs) = a.margin_off ? k_qp<true> : k_qp<false>;
+  void (*k)(SolveArgs) = qp_kernel(a);
+  if (!k) return 0;
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, k, QP_THREADS, smem);
   if (per < 1) per = 1;
@@ -231,7 +244,9 @@ int qp_max_grid(const SolveArgs &a, int device) {
 
 cudaError_t launch_qp(const SolveArgs &a, int grid, cudaStream_t st) {
   const size_t smem = qp_smem_bytes(a);
-  (a.margin_off ? k_qp<true> : k_qp<false>)<<<grid, QP_THREADS, smem, st>>>(a);
+  void (*k)(SolveArgs) = qp_kernel(a);
+  if (!k) return cudaErrorInvalidValue;
+  k<<<grid, QP_THREADS, smem, st>>>(a);
   return cudaGetLastError();
 }
 

@@ -124,28 +124,30 @@ __device__ __forceinline__ void numjac_waypoint_lane(const DevTables &tab, const
 struct WarpSmem {
   size_t tab, mbar, regions, region_bytes, total;
 };
-__host__ __device__ inline WarpSmem warp_smem(int n, int nj, int OH, int zs, int wpc, int nobs) {
+__host__ __device__ inline WarpSmem warp_smem(int n, int nj, int OH, int zs, int wpc, int nobs, bool lim = false) {
   WarpSmem L;
   size_t o = 0;
   L.tab = o; o += CFS_TAB_HEADER_BYTES + sizeof(ObsTab) * (size_t)nobs;  // only the staged part of DevTables
   L.mbar = o; o += 16;
   o = (o + 127) / 128 * 128;
   L.regions = o;
-  L.region_bytes = (warp_region_bytes(n, nj, OH, zs) + 127) / 128 * 128;
+  L.region_bytes = (warp_region_bytes(n, nj, OH, zs, lim) + 127) / 128 * 128;
   L.total = o + L.region_bytes * wpc;
   return L;
 }
 
 // PROF: clock64 split of every problem into gradient phase / QP / everything (timing level 3: cfs_get_warp_profile); a separate
 // instantiation so that the production kernel keeps its register budget.  OFF: the obstacle rows read a.margin_off (the
-// checked solve's per-waypoint margin offsets); also a separate instantiation, the one without it is unchanged.
-template <int NJ, int NT, int MAXREG, int OC, bool PROF = false, bool OFF = false>
+// checked solve's per-waypoint margin offsets); also a separate instantiation, the one without it is unchanged.  LIM (only
+// with OFF): the QP also has the joint position rows of a.qlim.
+template <int NJ, int NT, int MAXREG, int OC, bool PROF = false, bool OFF = false, bool LIM = false>
 __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int WPC = NT / 32;
-  const int n = a.n, H = a.H, O = a.nobs, OH = O * H, m = OH + 4 * n, N = 2 * n;
+  const int n = a.n, H = a.H, O = a.nobs, OH = O * H, m = OH + (LIM ? 6 : 4) * n, N = 2 * n;
+  const int mz = LIM ? OH + 4 * n + (2 * n + 7) / 8 : m;  // bytes of the inact map (LIM: position rows as bits)
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const WarpSmem L = warp_smem(n, NJ, OH, a.warp_zs, WPC, O);
+  const WarpSmem L = warp_smem(n, NJ, OH, a.warp_zs, WPC, O, LIM);
   DevTables &tab = *reinterpret_cast<DevTables *>(smem_raw + L.tab);
   uint64_t *mbar = reinterpret_cast<uint64_t *>(smem_raw + L.mbar);
   tma_stage(&tab, a.tab, tab_bytes(a.nobs), mbar);
@@ -156,7 +158,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
   s.qcap = a.warp_qcap < WQ_QBIG - 1 ? (a.warp_qcap > 1 ? a.warp_qcap : 1) : WQ_QBIG - 1;
   double *sc = s.zc, *pm = s.zc + 2 * NJ * 32;  // gradient-phase scratch aliases the direction cache
   const double dt = tab.dt, dt2 = dt * dt;
-  const WDims P = {n, H, OH, O, m, 3 * n, a.has_lim, a.has_bounds, dt, a.G, a.gdiag, a.max_input, a.lim};
+  const WDims P = {n, H, OH, O, m, 3 * n, a.has_lim, a.has_bounds, dt, a.G, a.gdiag, a.max_input, a.lim, LIM ? a.qlim : nullptr};
   const double qnan = __longlong_as_double(0x7ff8000000000000LL);
   long long steps_total = 0;
   int qmax_seen = 0;
@@ -258,7 +260,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
         }
       }
 #pragma unroll 1
-      for (int e = lane * 4; e < m; e += 128)  // inact[] = 0, four rows per store (the region is padded to 16 B)
+      for (int e = lane * 4; e < mz; e += 128)  // inact[] = 0, four rows per store (the region is padded to 16 B)
         *reinterpret_cast<unsigned int *>(s.inact + e) = 0u;
       __syncwarp();
       if (PROF) {
@@ -271,7 +273,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
       // ---- Solve_QP (CFS_FANUC.m:85) ----
       int q = 0, steps = 0;
       const int masked = w_mask_antiparallel<NJ>(s, P);
-      const int qst = wqp_solve<NJ>(s, P, cost0, fupper, a.esc_steps, masked, q, steps, qmax_seen);
+      const int qst = wqp_solve<NJ, LIM>(s, P, cost0, fupper, a.esc_steps, masked, q, steps, qmax_seen);
       if (PROF) pf_qp += clock64() - pf_t1;
       steps_total += steps;
       steps_prob += steps;
@@ -287,7 +289,7 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
 #pragma unroll 1
         for (int w = 0; w < q; ++w) {
           const int cw = s.act[w];
-          pc += s.lam[w] * (W_ROW_DOT(cw, s.u0s) - w_row_rhs<NJ>(cw, s, P));  // lambda_w * violation at u0
+          pc += s.lam[w] * (W_ROW_DOT(cw, s.u0s) - w_row_rhs<NJ, LIM>(cw, s, P));  // lambda_w * violation at u0
         }
         cost = cost0 + 0.5 * pc;
       }
@@ -386,20 +388,21 @@ __global__ void __launch_bounds__(NT) __maxnreg__(MAXREG) k_cfs_warp(SolveArgs a
 // DERIVEST gradients come from their own kernel) keeps its structure -- gradient kernel | QP kernel per outer iteration -- but
 // the QP kernel (k_qp.cu: one CTA per problem) is replaced by this one: same prologue / epilogue, wqp_solve in the middle.
 // Problems whose working set outgrows the warp tier are appended to esc_list and taken by k_qp in the same iteration.
-template <int NJ, int NT, bool OFF = false>
+template <int NJ, int NT, bool OFF = false, bool LIM = false>
 __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int WPC = NT / 32;
-  const int n = a.n, H = a.H, O = a.nobs, OH = O * H, m = OH + 4 * n, N = 2 * n;
+  const int n = a.n, H = a.H, O = a.nobs, OH = O * H, m = OH + (LIM ? 6 : 4) * n, N = 2 * n;
+  const int mz = LIM ? OH + 4 * n + (2 * n + 7) / 8 : m;  // bytes of the inact map (LIM: position rows as bits)
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const WarpSmem L = warp_smem(n, NJ, OH, a.warp_zs, WPC, 0);
+  const WarpSmem L = warp_smem(n, NJ, OH, a.warp_zs, WPC, 0, LIM);
   WView s = warp_view(smem_raw + L.regions + L.region_bytes * wid, n, NJ, OH, a.warp_zs);
   s.zgl = a.zslab + (size_t)(blockIdx.x * WPC + wid) * warp_slab_doubles(n, a.warp_zs);
   s.Mgl = s.zgl + (size_t)(WQ_QZ - a.warp_zs) * n;
   s.qcap = a.warp_qcap < WQ_QBIG - 1 ? (a.warp_qcap > 1 ? a.warp_qcap : 1) : WQ_QBIG - 1;
   const double dt = a.tab->dt, dt2 = dt * dt;
   const bool psg = a.solver == 1;
-  const WDims P = {n, H, OH, O, m, 3 * n, a.has_lim, a.has_bounds, dt, a.G, a.gdiag, a.max_input, a.lim};
+  const WDims P = {n, H, OH, O, m, 3 * n, a.has_lim, a.has_bounds, dt, a.G, a.gdiag, a.max_input, a.lim, LIM ? a.qlim : nullptr};
   const int count = *a.count_cur;
   const int it = a.outer_iter;
   long long steps_total = 0;
@@ -419,7 +422,7 @@ __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
 #pragma unroll 2
     for (int c = lane; c < n; c += 32) s.u0s[c] = a.u0[(size_t)b * n + c];
 #pragma unroll 1
-    for (int e = lane * 4; e < m; e += 128) *reinterpret_cast<unsigned int *>(s.inact + e) = 0u;
+    for (int e = lane * 4; e < mz; e += 128) *reinterpret_cast<unsigned int *>(s.inact + e) = 0u;
     __syncwarp();
 #pragma unroll 1
     for (int cid = lane; cid < OH; cid += 32) {
@@ -450,7 +453,7 @@ __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
       __syncwarp();
     } else {
       const int masked = w_mask_antiparallel<NJ>(s, P);
-      status = wqp_solve<NJ>(s, P, a.cost0[b], (a.has_bounds && a.fupper) ? a.fupper[b] : INFINITY, 0x7fffffff, masked, q, steps,
+      status = wqp_solve<NJ, LIM>(s, P, a.cost0[b], (a.has_bounds && a.fupper) ? a.fupper[b] : INFINITY, 0x7fffffff, masked, q, steps,
                              qmax_seen);
     }
     steps_total += steps;
@@ -470,7 +473,7 @@ __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
 #pragma unroll 1
       for (int w = 0; w < q; ++w) {
         const int cw = s.act[w];
-        pc += s.lam[w] * (W_ROW_DOT(cw, s.u0s) - w_row_rhs<NJ>(cw, s, P));
+        pc += s.lam[w] * (W_ROW_DOT(cw, s.u0s) - w_row_rhs<NJ, LIM>(cw, s, P));
       }
       cost = a.cost0[b] + 0.5 * pc;
     }
@@ -533,7 +536,7 @@ __global__ void __launch_bounds__(NT, 3) k_qp_warp(SolveArgs a) {
 static const int kWarpNT[WARP_NCFG] = {384, 96, 128, 32, 64};
 
 size_t warp_smem_bytes(const SolveArgs &a, int cfg) {
-  return warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, kWarpNT[cfg] / 32, a.nobs).total;
+  return warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, kWarpNT[cfg] / 32, a.nobs, a.qlim != nullptr).total;
 }
 
 bool warp_supported(const SolveArgs &a, int cfg) {
@@ -548,29 +551,34 @@ int warp_warps_per_cta(int cfg) { return kWarpNT[cfg] / 32; }
 size_t warp_slab_bytes_per_warp(const SolveArgs &a) { return sizeof(double) * warp_slab_doubles(a.n, a.warp_zs); }
 
 typedef void (*WarpKernel)(SolveArgs);
-template <int NJ, bool OFF>
+template <int NJ, bool OFF, bool LIM = false>
 static WarpKernel warp_kernel_nj(int cfg, bool two) {
   switch (cfg) {
-    case 0: return two ? k_cfs_warp<NJ, 384, 168, 2, false, OFF> : k_cfs_warp<NJ, 384, 168, 1, false, OFF>;
-    case 1: return two ? k_cfs_warp<NJ, 96, 224, 2, false, OFF> : k_cfs_warp<NJ, 96, 224, 1, false, OFF>;
-    case 2: return two ? k_cfs_warp<NJ, 128, 168, 2, false, OFF> : k_cfs_warp<NJ, 128, 168, 1, false, OFF>;
-    case 3: return two ? k_cfs_warp<NJ, 32, 168, 2, false, OFF> : k_cfs_warp<NJ, 32, 168, 1, false, OFF>;
-    case 4: return two ? k_cfs_warp<NJ, 64, 168, 2, false, OFF> : k_cfs_warp<NJ, 64, 168, 1, false, OFF>;
+    case 0: return two ? k_cfs_warp<NJ, 384, 168, 2, false, OFF, LIM> : k_cfs_warp<NJ, 384, 168, 1, false, OFF, LIM>;
+    case 1: return two ? k_cfs_warp<NJ, 96, 224, 2, false, OFF, LIM> : k_cfs_warp<NJ, 96, 224, 1, false, OFF, LIM>;
+    case 2: return two ? k_cfs_warp<NJ, 128, 168, 2, false, OFF, LIM> : k_cfs_warp<NJ, 128, 168, 1, false, OFF, LIM>;
+    case 3: return two ? k_cfs_warp<NJ, 32, 168, 2, false, OFF, LIM> : k_cfs_warp<NJ, 32, 168, 1, false, OFF, LIM>;
+    case 4: return two ? k_cfs_warp<NJ, 64, 168, 2, false, OFF, LIM> : k_cfs_warp<NJ, 64, 168, 1, false, OFF, LIM>;
   }
   return nullptr;
 }
-// off: the margin-offset instantiations (a.margin_off != nullptr); the phase profile has none (timing level 3 measures the
-// unchecked solve)
-static WarpKernel warp_kernel(int nj, int cfg, int nobs, bool prof = false, bool off = false) {
+// off: the margin-offset instantiations (a.margin_off != nullptr); lim: the joint-limit ones (a.qlim != nullptr, always with
+// offsets).  The phase profile has neither (timing level 3 measures the unchecked solve).
+static WarpKernel warp_kernel(int nj, int cfg, int nobs, bool prof = false, bool off = false, bool lim = false) {
   if (prof && !off && nj == 5 && cfg == 3 && nobs <= 1) return k_cfs_warp<5, 32, 168, 1, true>;
-  if (nj == 2) return off ? warp_kernel_nj<2, true>(cfg, nobs > 1) : warp_kernel_nj<2, false>(cfg, nobs > 1);
-  if (nj == 5) return off ? warp_kernel_nj<5, true>(cfg, nobs > 1) : warp_kernel_nj<5, false>(cfg, nobs > 1);
+  if (lim && !off) return nullptr;
+  if (nj == 2)
+    return lim ? warp_kernel_nj<2, true, true>(cfg, nobs > 1)
+               : (off ? warp_kernel_nj<2, true>(cfg, nobs > 1) : warp_kernel_nj<2, false>(cfg, nobs > 1));
+  if (nj == 5)
+    return lim ? warp_kernel_nj<5, true, true>(cfg, nobs > 1)
+               : (off ? warp_kernel_nj<5, true>(cfg, nobs > 1) : warp_kernel_nj<5, false>(cfg, nobs > 1));
   return nullptr;
 }
 
 int warp_max_grid(const SolveArgs &a, int device, int cfg) {
   const size_t smem = warp_smem_bytes(a, cfg);
-  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, false, a.margin_off != nullptr);
+  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, false, a.margin_off != nullptr, a.qlim != nullptr);
   if (!k) return 0;
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -584,7 +592,7 @@ int warp_max_grid(const SolveArgs &a, int device, int cfg) {
 
 cudaError_t launch_warp(const SolveArgs &a, int grid, int cfg, cudaStream_t st) {
   const bool off = a.margin_off != nullptr;
-  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, a.prof != nullptr, off);
+  WarpKernel k = warp_kernel(a.nj, cfg, a.nobs, a.prof != nullptr, off, a.qlim != nullptr);
   if (!k) return cudaErrorInvalidValue;
   if (a.prof && !off) {  // the profiled instantiation is a function of its own: same opt-in limits as warp_max_grid sets
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -598,13 +606,21 @@ cudaError_t launch_warp(const SolveArgs &a, int grid, int cfg, cudaStream_t st) 
 bool qp_warp_supported(const SolveArgs &a) {
   if (a.nj != 2 && a.nj != 5) return false;
   if (a.H > 64 || a.n > 32 * W_NC || a.warp_zs < 1 || a.warp_zs > 8) return false;
-  return warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0).total <= 227 * 1024;
+  return warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0, a.qlim != nullptr).total <= 227 * 1024;
+}
+
+static WarpKernel qp_warp_kernel(const SolveArgs &a) {
+  const bool off = a.margin_off != nullptr, lim = a.qlim != nullptr;
+  if (lim && !off) return nullptr;
+  if (a.nj == 2) return lim ? k_qp_warp<2, 128, true, true> : (off ? k_qp_warp<2, 128, true> : k_qp_warp<2, 128>);
+  if (a.nj == 5) return lim ? k_qp_warp<5, 128, true, true> : (off ? k_qp_warp<5, 128, true> : k_qp_warp<5, 128>);
+  return nullptr;
 }
 
 int qp_warp_max_grid(const SolveArgs &a, int device) {
-  const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0).total;
-  const bool off = a.margin_off != nullptr;
-  WarpKernel k = a.nj == 2 ? (off ? k_qp_warp<2, 128, true> : k_qp_warp<2, 128>) : (off ? k_qp_warp<5, 128, true> : k_qp_warp<5, 128>);
+  const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0, a.qlim != nullptr).total;
+  WarpKernel k = qp_warp_kernel(a);
+  if (!k) return 0;
   int sms = 0, per = 0;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return 0;
@@ -614,11 +630,10 @@ int qp_warp_max_grid(const SolveArgs &a, int device) {
 }
 
 cudaError_t launch_qp_warp(const SolveArgs &a, int grid, cudaStream_t st) {
-  const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0).total;
-  const bool off = a.margin_off != nullptr;
-  if (a.nj == 2) (off ? k_qp_warp<2, 128, true> : k_qp_warp<2, 128>)<<<grid, 128, smem, st>>>(a);
-  else if (a.nj == 5) (off ? k_qp_warp<5, 128, true> : k_qp_warp<5, 128>)<<<grid, 128, smem, st>>>(a);
-  else return cudaErrorInvalidValue;
+  const size_t smem = warp_smem(a.n, a.nj, a.nobs * a.H, a.warp_zs, 4, 0, a.qlim != nullptr).total;
+  WarpKernel k = qp_warp_kernel(a);
+  if (!k) return cudaErrorInvalidValue;
+  k<<<grid, 128, smem, st>>>(a);
   return cudaGetLastError();
 }
 

@@ -22,7 +22,7 @@ struct QpView {  // decoded shared-memory layout
   double *tcoef;   // TMAX    coefficient of each active term
   double *twgt;    // TMAX    lambda_owner * coefficient
   double *Msm;     // QP_QS*QP_QS
-  double *lim;     // 8: velocity limits
+  double *lim;     // 8: velocity limits; lim layouts: then qmax | qmin | theta0 (8 each) of the joint position rows
   double *w0;      // 8: initial joint velocities
   int *act;        // n+2
   int *toff;       // n+3     first term of each working-set member
@@ -42,8 +42,9 @@ struct QpView {  // decoded shared-memory layout
 #define QP_NOFF 26
 // qz > 0: "cached" layout of the fused bulk tier -- the working set holds at most qz-1 rows, every member's direction
 // z_w (n doubles) stays in shared memory, and the flat term lists of the G-based refresh are not needed.
+// lim: layout of the joint-limit instantiations (m then counts the 2n position rows too)
 __host__ __device__ inline size_t qp_smem_layout(int n, int nj, int OH, int m, size_t *off /*[QP_NOFF]*/, int qs = QP_QS,
-                                                  int nt = QP_THREADS, int qz = 0) {
+                                                  int nt = QP_THREADS, int qz = 0, bool lim = false) {
   size_t o = 0;
   const int np = 3 * n;
   const int tmax = qz ? 0 : nj * OH + n + 2;
@@ -63,7 +64,7 @@ __host__ __device__ inline size_t qp_smem_layout(int n, int nj, int OH, int m, s
   off[2] = o; o += sizeof(double) * OH;
   off[3] = o; o += sizeof(double) * OH;
   off[7] = o; o += sizeof(double) * 64;
-  off[11] = o; o += sizeof(double) * 8;
+  off[11] = o; o += sizeof(double) * (lim ? 32 : 8);
   off[12] = o; o += sizeof(double) * 8;
   off[13] = o; o += sizeof(int) * nw;
   off[14] = o; o += sizeof(int) * (nw + 2);
@@ -87,10 +88,10 @@ __host__ __device__ inline size_t qp_scratch_span(int n, int nj, int OH, int qs 
 }
 
 __device__ __forceinline__ QpView qp_view(unsigned char *smem_raw, int n, int nj, int OH, int m, int qs = QP_QS,
-                                          int nt = QP_THREADS, int qz = 0) {
+                                          int nt = QP_THREADS, int qz = 0, bool lim = false) {
   QpView s;
   size_t off[QP_NOFF];
-  qp_smem_layout(n, nj, OH, m, off, qs, nt, qz);
+  qp_smem_layout(n, nj, OH, m, off, qs, nt, qz, lim);
   s.zc = reinterpret_cast<double *>(smem_raw + off[23]);
   s.zslot = reinterpret_cast<int *>(smem_raw + off[24]);
   s.yp = reinterpret_cast<double *>(smem_raw + off[25]);
@@ -124,6 +125,8 @@ __device__ __forceinline__ QpView qp_view(unsigned char *smem_raw, int n, int nj
 // cid in [0,OH): obstacle row (j,i), cid = j*H+i: nj terms on the theta primitives of waypoint i, coefficients ocoef[cid*nj+k]
 // cid >= OH: e = cid-OH, primitive pr = e>>1 in [0,2n) (omega primitives 0..n-1, controls n..2n-1), sign bit e&1
 //            (0: +row <= hi, 1: -row <= lo).  Velocity rows: CFS_FANUC.m:126-129; control rows: lb/ub of CFS_FANUC.m:85.
+//            LIM (the joint-limit instantiations): pr in [2n,3n) is the theta primitive pr-2n, the joint position rows
+//            theta <= qmax / -theta <= -qmin (DESIGN.md section 3d).
 struct Desc {
   int nterm;
   int row0;          // first primitive row; terms are consecutive rows
@@ -146,6 +149,7 @@ __device__ __forceinline__ int wp_of(int cid, int H) {  // waypoint of an obstac
   return i;
 }
 
+template <bool LIM = false>
 __device__ __forceinline__ Desc decode(int cid, const QpDims &P, const double *ocoef) {
   Desc d;
   if (cid < P.OH) {
@@ -156,7 +160,7 @@ __device__ __forceinline__ Desc decode(int cid, const QpDims &P, const double *o
   } else {
     const int e = cid - P.OH;
     d.nterm = 1;
-    d.row0 = P.n + (e >> 1);
+    d.row0 = (LIM && (e >> 1) >= 2 * P.n) ? (e >> 1) - 2 * P.n : P.n + (e >> 1);
     d.coef = (e & 1) ? -1.0 : 1.0;
     d.cv = nullptr;
   }
@@ -164,8 +168,9 @@ __device__ __forceinline__ Desc decode(int cid, const QpDims &P, const double *o
 }
 
 // c_a QQ^-1 c_b' as a bilinear form over G
+template <bool LIM = false>
 static __device__ __noinline__ double gram(int ca, int cb, const QpDims &P, const double *ocoef) {
-  const Desc a = decode(ca, P, ocoef), b = decode(cb, P, ocoef);
+  const Desc a = decode<LIM>(ca, P, ocoef), b = decode<LIM>(cb, P, ocoef);
   const double *__restrict__ G = P.G;
   if (a.nterm == 1 && b.nterm == 1) return a.coef * b.coef * G[(size_t)a.row0 * P.np + b.row0];
   double s = 0.0;
@@ -181,17 +186,22 @@ static __device__ __noinline__ double gram(int ca, int cb, const QpDims &P, cons
   return s;
 }
 
-template <int NJ>
+template <int NJ, bool LIM = false>
 __device__ __forceinline__ double prim_rhs(int pr, int neg, const QpDims &P, const QpView &s) {
   if (pr < P.n) {
     const int k = NJ ? pr % NJ : pr % P.nj;
     return neg ? s.lim[k] + s.w0[k] : s.lim[k] - s.w0[k];
   }
+  if (LIM && pr >= 2 * P.n) {  // free motion fm = theta0 + (i+1) dt omega0: qmax - fm / fm - qmin
+    const int nj = NJ ? NJ : P.nj, i = (pr - 2 * P.n) / nj, k = (pr - 2 * P.n) - i * nj;
+    const double fm = s.lim[24 + k] + ((i + 1) * P.dt) * s.w0[k];
+    return neg ? fm - s.lim[16 + k] : s.lim[8 + k] - fm;
+  }
   return P.umax[pr - P.n];
 }
 
 // slack = rhs - c u from the primitive values in `v`; with v = v0s this is minus the violation at the unconstrained minimiser
-template <int NJ>
+template <int NJ, bool LIM = false>
 static __device__ __noinline__ double slack_at(int cid, const QpDims &P, const QpView &s, const double *v) {
   if (cid < P.OH) {
     const double *c = s.ocoef + (size_t)cid * P.nj;
@@ -202,8 +212,8 @@ static __device__ __noinline__ double slack_at(int cid, const QpDims &P, const Q
     return s.orhs[cid] - val;
   }
   const int e = cid - P.OH, pr = e >> 1, neg = e & 1;
-  const double vv = v[P.n + pr];
-  return prim_rhs<NJ>(pr, neg, P, s) - (neg ? -vv : vv);
+  const double vv = (LIM && pr >= 2 * P.n) ? v[pr - 2 * P.n] : v[P.n + pr];
+  return prim_rhs<NJ, LIM>(pr, neg, P, s) - (neg ? -vv : vv);
 }
 
 // ---- block reductions (NT threads): warp shuffles, one shared-memory exchange, second stage again by shuffles -------
@@ -435,6 +445,7 @@ static __device__ __noinline__ void qp_refresh_cached(const QpView &s, const QpD
 }
 
 // e_cid' y for y = P z given as (yth | yom | z)
+template <bool LIM = false>
 static __device__ __forceinline__ double row_dot_prims(int cid, const double *yth, const double *yom, const double *z,
                                                        const QpDims &P, const double *ocoef) {
   if (cid < P.OH) {
@@ -445,16 +456,16 @@ static __device__ __forceinline__ double row_dot_prims(int cid, const double *yt
     return acc;
   }
   const int e = cid - P.OH, pr = e >> 1;
-  const double val = pr < P.n ? yom[pr] : z[pr - P.n];
+  const double val = pr < P.n ? yom[pr] : ((LIM && pr >= 2 * P.n) ? yth[pr - 2 * P.n] : z[pr - P.n]);
   return (e & 1) ? -val : val;
 }
 
 // candidate p: z_p = QQ^-1 c_p' into the candidate slot (one pass over <= nj rows of G), y_p = P z_p by prefix sums, then
 // sigma = c_p QQ^-1 c_p' = e_p'y_p and g_w = c_w QQ^-1 c_p' = e_w'y_p for every member
-template <int NT>
+template <int NT, bool LIM = false>
 static __device__ __noinline__ double qp_candidate_cached(const QpView &s, const QpDims &P, int p, int q) {
   const int tid = threadIdx.x, n = P.n;
-  const Desc dp = decode(p, P, s.ocoef);
+  const Desc dp = decode<LIM>(p, P, s.ocoef);
   double *zp = s.zc + (size_t)s.zslot[q] * n;
   const double *__restrict__ Gu = P.G + (size_t)dp.row0 * P.np + 2 * n;  // control block of the candidate's primitive rows
 #pragma unroll 1
@@ -473,7 +484,7 @@ static __device__ __noinline__ double qp_candidate_cached(const QpView &s, const
   __syncthreads();
 #pragma unroll 1
   for (int w = tid; w <= q; w += NT) {
-    const double val = row_dot_prims(w < q ? s.act[w] : p, s.yp, s.yp + n, zp, P, s.ocoef);
+    const double val = row_dot_prims<LIM>(w < q ? s.act[w] : p, s.yp, s.yp + n, zp, P, s.ocoef);
     if (w < q)
       s.g[w] = val;
     else
@@ -549,7 +560,7 @@ __device__ __forceinline__ int qp_mask_antiparallel(const QpView &s, const QpDim
 // Polish: the working-set inverse M has been rank-1 updated many times; one step of iterative refinement on
 // S_W lambda = b (S_W = C_W QQ^-1 C_W' re-read from G, b = violations at u0) removes the accumulated drift
 // (measured: 7e-10 -> 3e-13 in u).
-template <int NT, int NJ>
+template <int NT, int NJ, bool LIM = false>
 static __device__ __noinline__ void qp_polish(const QpView &s, const QpDims &P, int q, const double *M, int ldm) {
   const int tid = threadIdx.x;
   const int nch = NT / q > 0 ? NT / q : 1;  // chunks of columns per row, fixed summation order
@@ -558,7 +569,7 @@ static __device__ __noinline__ void qp_polish(const QpView &s, const QpDims &P, 
     if (ch < nch) {
       double acc = 0.0;
 #pragma unroll 1
-      for (int c = ch; c < q; c += nch) acc += gram(s.act[w], s.act[c], P, s.ocoef) * s.lam[c];
+      for (int c = ch; c < q; c += nch) acc += gram<LIM>(s.act[w], s.act[c], P, s.ocoef) * s.lam[c];
       s.pscr[ch * q + w] = acc;
     }
     __syncthreads();
@@ -566,15 +577,15 @@ static __device__ __noinline__ void qp_polish(const QpView &s, const QpDims &P, 
       double acc = 0.0;
 #pragma unroll 1
       for (int ch2 = 0; ch2 < nch; ++ch2) acc += s.pscr[ch2 * q + tid];
-      s.g[tid] = -slack_at<NJ>(s.act[tid], P, s, s.v0s) - acc;
+      s.g[tid] = -slack_at<NJ, LIM>(s.act[tid], P, s, s.v0s) - acc;
     }
   } else {
 #pragma unroll 1
     for (int w = tid; w < q; w += NT) {
       double acc = 0.0;
 #pragma unroll 1
-      for (int c = 0; c < q; ++c) acc += gram(s.act[w], s.act[c], P, s.ocoef) * s.lam[c];
-      s.g[w] = -slack_at<NJ>(s.act[w], P, s, s.v0s) - acc;
+      for (int c = 0; c < q; ++c) acc += gram<LIM>(s.act[w], s.act[c], P, s.ocoef) * s.lam[c];
+      s.g[w] = -slack_at<NJ, LIM>(s.act[w], P, s, s.v0s) - acc;
     }
   }
   __syncthreads();
@@ -598,7 +609,7 @@ static __device__ __noinline__ void qp_polish(const QpView &s, const QpDims &P, 
 // minimiser) and u(lambda) stationary on it -- a valid state of the dual method, from which qp_solve continues.  Called when
 // the working-set residual check finds the updated inverse broken (typically a nearly dependent set on an infeasible QP).
 // Returns the new size of the working set, or -1 if no consistent set was reached.
-template <int NT, int QS, int NJ>
+template <int NT, int QS, int NJ, bool LIM = false>
 static __device__ __noinline__ int qp_refactor(const QpView &s, const QpDims &P, int q0, double cost0, bool &in_smem,
                                                double *fval_new) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -613,10 +624,10 @@ static __device__ __noinline__ int qp_refactor(const QpView &s, const QpDims &P,
 #pragma unroll 1
     for (int idx = tid; idx < qc * qc; idx += NT) {  // S_W, lower triangle
       const int j = idx / qc, i = idx - j * qc;
-      if (i >= j) A[i + (size_t)ld * j] = gram(s.act[i], s.act[j], P, s.ocoef);
+      if (i >= j) A[i + (size_t)ld * j] = gram<LIM>(s.act[i], s.act[j], P, s.ocoef);
     }
 #pragma unroll 1
-    for (int i = tid; i < qc; i += NT) s.g[i] = -slack_at<NJ>(s.act[i], P, s, s.v0s);
+    for (int i = tid; i < qc; i += NT) s.g[i] = -slack_at<NJ, LIM>(s.act[i], P, s, s.v0s);
     __syncthreads();
 #pragma unroll 1
     for (int i = tid; i < qc; i += NT) {
@@ -710,7 +721,7 @@ static __device__ __noinline__ int qp_refactor(const QpView &s, const QpDims &P,
   __syncthreads();
 #pragma unroll 1
   for (int w = tid; w < qc; w += NT) {
-    const Desc d = decode(s.act[w], P, s.ocoef);
+    const Desc d = decode<LIM>(s.act[w], P, s.ocoef);
     const int t0 = s.toff[w];
     for (int k = 0; k < d.nterm; ++k) {
       s.trow[t0 + k] = d.row0 + k;
@@ -731,8 +742,9 @@ static __device__ __noinline__ int qp_refactor(const QpView &s, const QpDims &P,
 // unconstrained minimiser whose primitives are in s.v0s / s.v.  On return (status 0) s.v holds the primitives of the
 // optimum (controls in s.v[2n..3n)), s.lam / s.act / q the multipliers and the working set.
 // status: 0 optimal, 2 infeasible, 3 numerical, 4 escalate (step_cap exceeded / working set outgrew QS and !SPILL).
-// Must be called by all NT threads of the CTA.  NJ: compile-time joint count (0 = use P.nj).
-template <int NT, int QS, bool SPILL, int NJ, int QZ = 0>
+// Must be called by all NT threads of the CTA.  NJ: compile-time joint count (0 = use P.nj).  LIM: with the joint position
+// rows (never masked; s.lim holds qmax | qmin | theta0 from index 8).
+template <int NT, int QS, bool SPILL, int NJ, int QZ = 0, bool LIM = false>
 __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double cost0, double fupper, bool skip_solve,
                                         int &q_out, int &steps_out, int &qmax_seen, long long *pf, long long &tck,
                                         bool prof, int step_cap = 0x7fffffff, int masked = 0) {
@@ -815,6 +827,31 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
         }
       }
     }
+    if (LIM) {  // joint position rows: theta primitives, ids after the control rows
+#pragma unroll 1
+      for (int e = tid; e < n; e += NT) {
+        const double sg = s.gns[e];
+        if (!(sg > 0.0)) continue;
+        const double vv = s.v[e];
+        const double hi = prim_rhs<NJ, LIM>(2 * n + e, 0, P, s), lo = prim_rhs<NJ, LIM>(2 * n + e, 1, P, s);
+        const double up = hi - vv, dn = lo + vv;
+        const int cu = OH + 4 * n + 2 * e;
+        if (up < -1e-11 * (1.0 + fabs(hi)) && !s.inact[cu]) {
+          const double key = -(up * up) / sg;
+          if (key < best || bidx < 0) {
+            best = key;
+            bidx = cu;
+          }
+        }
+        if (dn < -1e-11 * (1.0 + fabs(lo)) && !s.inact[cu + 1]) {
+          const double key = -(dn * dn) / sg;
+          if (key < best || bidx < 0) {
+            best = key;
+            bidx = cu + 1;
+          }
+        }
+      }
+    }
     block_argmin<NT>(best, bidx, s.red);
     PF_ADD(QPF(2));
     if (bidx < 0 && masked) {  // this phase is feasible: unmask the next level and carry on with the same working set
@@ -840,8 +877,8 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
 #pragma unroll 1
           for (int w = tid; w < q; w += NT) {
             const int cw = s.act[w];
-            const double rhs = cw < OH ? s.orhs[cw] : prim_rhs<NJ>((cw - OH) >> 1, (cw - OH) & 1, P, s);
-            const double res = fabs(slack_at<NJ>(cw, P, s, s.v)) / (1.0 + fabs(rhs));
+            const double rhs = cw < OH ? s.orhs[cw] : prim_rhs<NJ, LIM>((cw - OH) >> 1, (cw - OH) & 1, P, s);
+            const double res = fabs(slack_at<NJ, LIM>(cw, P, s, s.v)) / (1.0 + fabs(rhs));
             worst = fmax(worst, res);
           }
           int wi = 0;
@@ -854,7 +891,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
             double fnew = fval;
             if (!CACHED && refactors < 2) {
               ++refactors;
-              q1 = qp_refactor<NT, QS, NJ>(s, P, q, cost0, in_smem, &fnew);
+              q1 = qp_refactor<NT, QS, NJ, LIM>(s, P, q, cost0, in_smem, &fnew);
               ++steps;
             }
             if (q1 < 0) {
@@ -874,7 +911,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
         status = 0;
         break;
       }
-      qp_polish<NT, NJ>(s, P, q, M, ldm);
+      qp_polish<NT, NJ, LIM>(s, P, q, M, ldm);
       polished = true;
       continue;  // re-evaluate v from the refined multipliers and scan once more
     }
@@ -887,7 +924,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
         status = 4;
         break;
       }
-      sigma = qp_candidate_cached<NT>(s, P, p, q);
+      sigma = qp_candidate_cached<NT, LIM>(s, P, p, q);
     } else if (p < OH) {
       double part = 0.0;
       if (tid < nj * nj) {
@@ -895,10 +932,13 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
         part = s.ocoef[p * nj + k] * s.ocoef[p * nj + l2] * P.G[(size_t)(r0 + k) * P.np + r0 + l2];
       }
       sigma = block_sum<NT>(part, s.red);
+    } else if (LIM) {
+      const int r0 = decode<LIM>(p, P, s.ocoef).row0;
+      sigma = P.G[(size_t)r0 * P.np + r0];
     } else {
       sigma = P.G[(size_t)(n + ((p - OH) >> 1)) * P.np + n + ((p - OH) >> 1)];
     }
-    double sp = slack_at<NJ>(p, P, s, s.v);
+    double sp = slack_at<NJ, LIM>(p, P, s, s.v);
     double lam_p = 0.0;
     // (2) bring row p into the working set
     for (;;) {
@@ -914,7 +954,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
       // independent L2 loads each) instead of one per member (up to nj x nj dependent ones), then a fixed-order sum per member.
       // twgt is free between two refreshes.
       if (!CACHED) {
-        const Desc dp = decode(p, P, s.ocoef);
+        const Desc dp = decode<LIM>(p, P, s.ocoef);
         const int T = s.toff[q];
 #pragma unroll 1
         for (int t = tid; t < T; t += NT) {
@@ -1048,7 +1088,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
           }
         }
         if (!CACHED) {
-          const Desc dp = decode(p, P, s.ocoef);
+          const Desc dp = decode<LIM>(p, P, s.ocoef);
           const int t0 = s.toff[q];
           if (tid < dp.nterm) {
             s.trow[t0 + tid] = dp.row0 + tid;
@@ -1115,7 +1155,7 @@ __device__ __forceinline__ int qp_solve(const QpView &s, const QpDims &P, double
         if (!CACHED) {
 #pragma unroll 1
           for (int w = tid; w < q; w += NT) {
-            const Desc d = decode(s.act[w], P, s.ocoef);
+            const Desc d = decode<LIM>(s.act[w], P, s.ocoef);
             const int t0 = s.toff[w];
             for (int k = 0; k < d.nterm; ++k) {
               s.trow[t0 + k] = d.row0 + k;

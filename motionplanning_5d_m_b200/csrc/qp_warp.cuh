@@ -28,6 +28,7 @@ struct WDims {
   const double *gdiag;  // sqrt(G_ii)
   const double *umax;   // MAX_input (global)
   const double *lim;    // velocity limits (global, CFS_MAXL)
+  const double *qlim;   // LIM: joint position limits [qmax (NJ) | qmin (NJ)] (global), +-inf for a side without a limit
 };
 
 struct WView {  // this warp's shared-memory region
@@ -55,9 +56,11 @@ __host__ __device__ inline size_t warp_scratch_doubles(int n, int nj, int zs) {
   return a > b ? a : b;
 }
 
-__host__ __device__ inline size_t warp_region_bytes(int n, int nj, int OH, int zs) {
+// lim: the 2n joint position rows' flags follow the inact byte map as bits (w_set_inact), so that the region grows by 2n / 8
+// bytes only and the 12-warp CTA shape keeps fitting one SM
+__host__ __device__ inline size_t warp_region_bytes(int n, int nj, int OH, int zs, bool lim = false) {
   size_t d = 3 * (size_t)n + (size_t)OH * (nj + 2) + warp_scratch_doubles(n, nj, zs) + WQ_QS * WQ_QS + 3 * (WQ_QBIG + 2) + 16;
-  size_t b = d * sizeof(double) + sizeof(int) * (2 * WQ_QZ + 8) + (size_t)(OH + 4 * n);
+  size_t b = d * sizeof(double) + sizeof(int) * (2 * WQ_QZ + 8) + (size_t)(OH + 4 * n) + (lim ? (size_t)(2 * n + 7) / 8 : 0);
   return (b + 15) / 16 * 16;
 }
 
@@ -93,6 +96,24 @@ __device__ __forceinline__ double *wz(const WView &s, int slot, int n) {
   return slot < s.zs ? s.zc + (size_t)slot * n : s.zgl + (size_t)(slot - s.zs) * n;
 }
 
+// inact flag of row cid: a byte per row, the LIM position rows (ids from OH + 4n) a bit each after the bytes.  Written by one
+// lane between two __syncwarp()s.
+template <bool LIM>
+__device__ __forceinline__ bool w_inact(const WView &s, int m0, int cid) {
+  if (LIM && cid >= m0) return (s.inact[m0 + ((cid - m0) >> 3)] >> ((cid - m0) & 7)) & 1;
+  return s.inact[cid];
+}
+template <bool LIM>
+__device__ __forceinline__ void w_set_inact(const WView &s, int m0, int cid, unsigned char v) {
+  if (LIM && cid >= m0) {
+    unsigned char *w = s.inact + m0 + ((cid - m0) >> 3);
+    const unsigned char bit = (unsigned char)(1u << ((cid - m0) & 7));
+    *w = v ? (unsigned char)(*w | bit) : (unsigned char)(*w & ~bit);
+  } else {
+    s.inact[cid] = v;
+  }
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULLMASK, v, o);
@@ -120,7 +141,16 @@ __device__ __forceinline__ int w_wp_of(int cid, int H) {
   return i;
 }
 
-template <int NJ>
+// joint position row (waypoint i + 1, joint k): +-theta <= qmax / -qmin, i.e. +-(B_theta u)(i,k) <= qmax - fm / fm - qmin with the
+// free motion fm = theta0 + (i+1) dt omega0
+__device__ __forceinline__ double w_pos_rhs(int e, int neg, int nj, const double *x0s, const double *qlim, double dt) {
+  const int i = e / nj, k = e - i * nj;
+  const double fm = x0s[k] + ((i + 1) * dt) * x0s[nj + k];
+  return neg ? fm - __ldg(qlim + nj + k) : __ldg(qlim + k) - fm;
+}
+
+// LIM: ids OH + 4n + 2e + neg are the joint position rows of the theta primitive e = i NJ + k (DESIGN.md section 3d)
+template <int NJ, bool LIM = false>
 __device__ __forceinline__ double w_row_rhs(int cid, const WView &s, const WDims &P) {
   if (cid < P.OH) return s.orhs[cid];
   const int e = cid - P.OH, pr = e >> 1, neg = e & 1;
@@ -129,6 +159,7 @@ __device__ __forceinline__ double w_row_rhs(int cid, const WView &s, const WDims
     const double lim = __ldg(P.lim + k), w0 = s.x0s[NJ + k];
     return neg ? lim + w0 : lim - w0;
   }
+  if (LIM && pr >= 2 * P.n) return w_pos_rhs(pr - 2 * P.n, neg, NJ, s.x0s, P.qlim, P.dt);
   return __ldg(P.umax + (pr - P.n));
 }
 
@@ -136,9 +167,10 @@ __device__ __forceinline__ double w_row_rhs(int cid, const WView &s, const WDims
 //   obstacle row (j,i):        sum_{jj<=i} sum_k cv[k] (0.5+(i-jj)) dt^2 vec[jj,k]      (CFS_FANUC.m:121, B_theta blocks)
 //   velocity row (i,k), +-:    +- dt sum_{jj<=i} vec[jj,k]                               (CFS_FANUC.m:126-129)
 //   control row c, +-:         +- vec[c]                                                  (lb/ub of CFS_FANUC.m:85)
+//   LIM, position row (i,k), +-: +- sum_{jj<=i} (0.5+(i-jj)) dt^2 vec[jj,k]
 // Every lane returns the same value.  Not inlined (four call sites); every argument is a scalar, so nothing goes through
 // local memory.
-template <int NJ>
+template <int NJ, bool LIM = false>
 static __device__ __noinline__ double w_row_dot(int cid, const double *vec, const double *ocoef, int OH, int H, int n, double dt) {
   const int lane = threadIdx.x & 31;
   if (cid < OH) {
@@ -161,9 +193,15 @@ static __device__ __noinline__ double w_row_dot(int cid, const double *vec, cons
     for (int jj = lane; jj <= i; jj += 32) acc += vec[jj * NJ + k];
     return sgn * dt * warp_sum(acc);
   }
+  if (LIM && pr >= 2 * n) {
+    const int i = (pr - 2 * n) / NJ, k = (pr - 2 * n) - i * NJ;
+    double acc = 0.0;
+    for (int jj = lane; jj <= i; jj += 32) acc += (0.5 * dt * dt + ((i - jj) * dt) * dt) * vec[jj * NJ + k];
+    return sgn * warp_sum(acc);
+  }
   return sgn * vec[pr - n];
 }
-#define W_ROW_DOT(cid, vec) w_row_dot<NJ>(cid, vec, s.ocoef, P.OH, P.H, P.n, P.dt)
+#define W_ROW_DOT(cid, vec) w_row_dot<NJ, LIM>(cid, vec, s.ocoef, P.OH, P.H, P.n, P.dt)
 
 // primal recovery u = u0 - sum_w lambda_w z_w (n <= 32 * W_NC)
 #define W_NC 10
@@ -215,8 +253,9 @@ __device__ __forceinline__ void w_prefix2(double a0, double a1, double &s0, doub
 // (-1: none) and its slack.  B_theta u / B_omega u come from prefix sums held in registers (H <= 64: one pair of waypoints
 // per lane, the NJ joints' scans interleaved); obstacles are taken two at a time.  While phase-A masking is on, the
 // candidates of the masked levels are tracked in the same pass: when no unmasked row is violated, the next level is
-// unmasked and its most violated row taken, exactly as a rescan with the same u would do.
-template <int NJ>
+// unmasked and its most violated row taken, exactly as a rescan with the same u would do.  LIM: the joint position rows
+// are tested from the same registers (never masked).
+template <int NJ, bool LIM = false>
 __device__ __forceinline__ int w_scan(const WView &s, const WDims &P, int &masked, double &slack_out) {
   const int lane = threadIdx.x & 31, n = P.n, H = P.H, OH = P.OH, O = P.O;
   const double dt = P.dt, dt2 = dt * dt;
@@ -256,6 +295,25 @@ __device__ __forceinline__ int w_scan(const WView &s, const WDims &P, int &maske
             const int e = (h ? i1 : i0) * NJ + k, cu = OH + 2 * e + (vw < 0.0 ? 1 : 0);
             const double gd = __ldg(P.gdiag + n + e), sg = gd * gd;
             if (sg > 0.0 && !s.inact[cu]) {
+              const double key = -(sl * sl) / sg;
+              if (key < best || bidx < 0) { best = key; bidx = cu; bsl = sl; }
+            }
+          }
+        }
+      }
+      if (LIM && j0 == 0) {  // position rows theta <= qmax, -theta <= -qmin: at most one side violated (qmin <= qmax)
+        const double qhi = __ldg(P.qlim + k), qlo = __ldg(P.qlim + NJ + k), th00 = s.x0s[k], w0 = s.x0s[NJ + k];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int i = h ? i1 : i0;
+          const double fm = th00 + ((i + 1) * dt) * w0, th = h ? th1 : th0;
+          const double hi = qhi - fm, lo = fm - qlo, up = hi - th, dn = lo + th;
+          const bool neg = dn < up;
+          const double sl = neg ? dn : up;
+          if ((h ? v1 : v0) && sl < -1e-11 * (1.0 + fabs(neg ? lo : hi))) {
+            const int e = i * NJ + k, cu = OH + 4 * n + 2 * e + (neg ? 1 : 0);
+            const double gd = __ldg(P.gdiag + e), sg = gd * gd;
+            if (sg > 0.0 && !w_inact<LIM>(s, OH + 4 * n, cu)) {
               const double key = -(sl * sl) / sg;
               if (key < best || bidx < 0) { best = key; bidx = cu; bsl = sl; }
             }
@@ -376,7 +434,7 @@ __device__ __forceinline__ int w_mask_antiparallel(const WView &s, const WDims &
 // Solves  min 1/2 u'QQ u + ff'u  s.t. the rows in (s.ocoef, s.orhs, lim, umax), starting from u0s.  On return (status 0)
 // s.uq holds the optimum, s.lam / s.act / q the multipliers and the working set.
 // status: 0 optimal, 2 infeasible, 3 numerical, 4 escalate (step_cap exceeded / working set outgrew the direction slots).
-template <int NJ>
+template <int NJ, bool LIM = false>
 __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double cost0, double fupper, int step_cap, int masked,
                                          int &q_out, int &steps_out, int &qmax_seen) {
   const int lane = threadIdx.x & 31, n = P.n, OH = P.OH;
@@ -392,7 +450,7 @@ __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double 
   while (status < 0) {
     w_refresh(s, P, q);
     double sp;
-    const int p = w_scan<NJ>(s, P, masked, sp);
+    const int p = w_scan<NJ, LIM>(s, P, masked, sp);
     if (p < 0) {
       if (q == 0 || polished || (steps <= 6 && q <= 6)) {
         status = 0;
@@ -402,7 +460,7 @@ __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double 
 #pragma unroll 1
       for (int w = 0; w < q; ++w) {
         const int cw = s.act[w];
-        const double val = W_ROW_DOT(cw, s.uq) - w_row_rhs<NJ>(cw, s, P);
+        const double val = W_ROW_DOT(cw, s.uq) - w_row_rhs<NJ, LIM>(cw, s, P);
         if (lane == 0) s.g[w] = val;
       }
       __syncwarp();
@@ -442,7 +500,8 @@ __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double 
       } else {
         const int e = p - OH;
         const double coef = (e & 1) ? -1.0 : 1.0;
-        const double *__restrict__ G0 = Gu + (size_t)(n + (e >> 1)) * P.np;
+        // primitive row of G: omega / control rows n + pr, LIM position rows pr - 2n (the theta block)
+        const double *__restrict__ G0 = Gu + (size_t)((LIM && (e >> 1) >= 2 * n) ? (e >> 1) - 2 * n : n + (e >> 1)) * P.np;
 #pragma unroll 4
         for (int c = lane; c < n; c += 32) zp[c] = coef * G0[c];
       }
@@ -554,7 +613,7 @@ __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double 
         if (lane == 0) {
           s.act[q] = p;
           s.lam[q] = lam_p;
-          s.inact[p] = 1;
+          w_set_inact<LIM>(s, OH + 4 * n, p, 1);
         }
         ++q;
         if (q > qmax_seen) qmax_seen = q;
@@ -583,7 +642,7 @@ __device__ __forceinline__ int wqp_solve(const WView &s, const WDims &P, double 
           for (int w = lane; w < q; w += 32) Mp[l + (size_t)ldm * w] = Mp[last + (size_t)ldm * w];
         }
         if (lane == 0) {
-          s.inact[s.act[l]] = 0;
+          w_set_inact<LIM>(s, OH + 4 * n, s.act[l], 0);
           s.act[l] = s.act[last];
           s.lam[l] = s.lam[last];
           s.g[l] = s.g[last];
