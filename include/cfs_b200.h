@@ -328,7 +328,7 @@ typedef struct {
   double ms_total;        /* last cfs_solve_batch*: device time of the whole solve (CUDA events)          */
   double ms_grad;         /* ... of the distance/gradient kernel launches                                 */
   double ms_qp;           /* ... of the QP/rollout kernel launches                                        */
-  double ms_h2d, ms_d2h;  /* host-pointer entry only                                                      */
+  double ms_h2d, ms_d2h;  /* ... of its H2D / D2H copies when a host-pointer form ran it, 0 for a _device form */
   long long grad_waypoints; /* (problem, waypoint, obstacle) gradient evaluations done                    */
   long long problem_iters;  /* sum over problems of outer iterations                                      */
   long long qp_steps;       /* sum of dual active-set iterations                                          */

@@ -82,7 +82,6 @@ struct cfs_ctx {
   size_t stage_in_cap = 0, stage_out_cap = 0;
   struct CopyBack { void *dst; const void *src; size_t bytes; };
   std::vector<CopyBack> copy_back;  // staged results to hand to the caller in cfs_wait
-  bool staged_last = false;
   // timing
   std::vector<cudaEvent_t> ev;
   cudaEvent_t ev_a = nullptr, ev_b = nullptr;
@@ -904,6 +903,7 @@ static int collect_stats(cfs_ctx *ctx, int B, int max_outer, const int *d_iters,
   ctx->stats.problem_iters = pit;
   ctx->stats.grad_waypoints = gev * ctx->H * ctx->nobs;
   ctx->stats.ms_grad = ctx->stats.ms_qp = 0;
+  ctx->stats.ms_h2d = ctx->stats.ms_d2h = 0;  // a host form's copy times follow in flush_staged
   ctx->stats.ms_bulk = ctx->stats.ms_heavy = 0;
   if (ctx->timing_level >= 2 && ctx->fused_last && ctx->ev.size() >= 3) {
     float a = 0, b = 0;
@@ -954,58 +954,88 @@ static void host_copy(void *dst, const void *src, size_t bytes) {
   for (size_t k = 0; k < started; ++k) th[k].join();
 }
 
-static int finish_pending(cfs_ctx *ctx);
+// ---- the solve family: cfs_solve_batch*, cfs_solve_start_goal*, cfs_solve_routes*, cfs_solve_batch_margins*, cfs_solve_checked*
+// Every entry describes its call (SolveCall) and hands it to one validator (check_solve), one enqueue on device pointers
+// (enqueue_solve) and, for a host form, one transfer path (upload / download through the pinned staging area).
+enum SolveForm { FORM_ARRAYS, FORM_START_GOAL, FORM_ROUTES };
 
-static int check_solve_args(cfs_ctx *ctx, int B, int solver, int grad, const void *x0, const void *ff, const void *caug,
-                            const void *xref, int max_outer, const void *u, const void *x, const void *cost_hist,
-                            const void *iters, const void *status) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, true);
-  if (rc) return rc;
-  if (B < 0 || max_outer < 0) return fail(ctx, CFS_E_ARG, "cfs_solve_batch: B=%d max_outer=%d", B, max_outer);
-  if (solver != CFS_SOLVER_CFS && solver != CFS_SOLVER_PSGCFS) return fail(ctx, CFS_E_ARG, "cfs_solve_batch: solver=%d", solver);
-  if (grad != CFS_GRAD_NUMJAC && grad != CFS_GRAD_DERIVEST) return fail(ctx, CFS_E_ARG, "cfs_solve_batch: grad=%d", grad);
-  if (B > 0 && (!x0 || !ff || !caug || !xref || !u || !cost_hist || !iters || !status))
-    return fail(ctx, CFS_E_ARG, "cfs_solve_batch: NULL buffer");
-  return 0;
+// The problems of a call: the reference's per-problem arrays, or start/goal pairs or routes from which the device builds them
+// (main_FANUC.m:38-49,98-103; RRTstar_CFS.m:96-163).  Routes are nj x W x B with route_len[b] valid columns (NULL: all W);
+// need_len: the entry requires route_len.  noise and margin_off may be NULL.
+struct SolveIn {
+  SolveForm form;
+  const double *x0, *ff, *caug, *xref, *theta0, *thetag, *routes;
+  int W;
+  const int *route_len;
+  bool need_len;
+  const double *noise, *margin_off;
+};
+static SolveIn arrays_in(const double *x0, const double *ff, const double *caug, const double *xref, const double *noise,
+                         const double *margin_off = nullptr) {
+  return {FORM_ARRAYS, x0, ff, caug, xref, nullptr, nullptr, nullptr, 0, nullptr, false, noise, margin_off};
+}
+static SolveIn start_goal_in(const double *theta0, const double *thetag, const double *noise) {
+  return {FORM_START_GOAL, nullptr, nullptr, nullptr, nullptr, theta0, thetag, nullptr, 0, nullptr, false, noise, nullptr};
+}
+static SolveIn routes_in(const double *routes, int W, const int *route_len, bool need_len, const double *noise) {
+  return {FORM_ROUTES, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, routes, W, route_len, need_len, noise, nullptr};
+}
+struct SolveOut {  // x and e_u_hist may be NULL in a host form (not copied back)
+  double *u, *x, *cost_hist, *e_u_hist;
+  int *iters, *status;
+};
+struct CheckedIo {  // the checked solve's arguments and its outputs beyond SolveOut (margin_off may be NULL)
+  double eta;
+  int max_evals, rounds;
+  double gain;
+  int *verdict;
+  double *t_hit, *cmin;
+  int *rounds_used;
+  double *margin_off;
+};
+struct SolveCall {
+  const char *who;  // the public entry, named in the error messages
+  bool device;      // every pointer a device pointer
+  int B, solver, grad;
+  double eps_outer;
+  int max_outer;
+  double alpha;
+  SolveIn in;
+  SolveOut out;
+  const CheckedIo *chk = nullptr;  // the checked solve only
+};
+
+// The batch whose statistics cfs_wait collects (d: the call on device pointers; host: a host form, whose copy times are
+// collected too), or none (d = NULL).  The only writer of ctx->pending.
+static void set_pending(cfs_ctx *ctx, const SolveCall *d = nullptr, bool host = false) {
+  ctx->pending = {};
+  if (!d) return;
+  ctx->pending.active = true;
+  ctx->pending.host = host;
+  ctx->pending.B = d->B;
+  ctx->pending.max_outer = d->max_outer;
+  ctx->pending.d_iters = d->out.iters;
+  ctx->pending.d_status = d->out.status;
 }
 
-extern "C" int cfs_solve_batch_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
-                                      const double *caug, const double *xref, const double *noise, double eps_outer,
-                                      int max_outer, double alpha, double *u, double *x, double *cost_hist,
-                                      double *e_u_hist, int *iters, int *status, int sync) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  if (!x) return fail(ctx, CFS_E_ARG, "cfs_solve_batch_device: NULL x");
-  CU(cudaSetDevice(ctx->device));
-  ctx->pending.active = false;  // device-pointer entry: statistics of an un-waited earlier batch are dropped
-  rc = solve_device(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x, cost_hist,
-                    e_u_hist, iters, status);
-  if (rc) return rc;
-  ctx->pending.active = true;
-  ctx->pending.host = false;
-  ctx->pending.B = B;
-  ctx->pending.max_outer = max_outer;
-  ctx->pending.d_iters = iters;
-  ctx->pending.d_status = status;
-  if (sync) return finish_pending(ctx);
-  return 0;
+// After the stream has synchronised: the staged results to the caller's buffers and, for a host form, the times of its copies
+static void flush_staged(cfs_ctx *ctx, bool host) {
+  for (const cfs_ctx::CopyBack &cb : ctx->copy_back) host_copy(cb.dst, cb.src, cb.bytes);
+  ctx->copy_back.clear();
+  if (!host) return;
+  float a = 0, b = 0;
+  cudaEventElapsedTime(&a, ctx->ev_h[0], ctx->ev_h[1]);
+  cudaEventElapsedTime(&b, ctx->ev_h[2], ctx->ev_h[3]);
+  ctx->stats.ms_h2d = a;
+  ctx->stats.ms_d2h = b;
 }
 
 static int finish_pending(cfs_ctx *ctx) {
   if (!ctx->pending.active) return 0;
-  ctx->pending.active = false;
-  int rc = collect_stats(ctx, ctx->pending.B, ctx->pending.max_outer, ctx->pending.d_iters, ctx->pending.d_status);
-  for (const cfs_ctx::CopyBack &cb : ctx->copy_back) host_copy(cb.dst, cb.src, cb.bytes);  // staged results -> caller's buffers
-  ctx->copy_back.clear();
-  if (ctx->pending.host) {
-    float a = 0, b = 0;
-    cudaEventElapsedTime(&a, ctx->ev_h[0], ctx->ev_h[1]);
-    cudaEventElapsedTime(&b, ctx->ev_h[2], ctx->ev_h[3]);
-    ctx->stats.ms_h2d = a;
-    ctx->stats.ms_d2h = b;
-  }
+  const auto p = ctx->pending;
+  set_pending(ctx);
+  int rc = collect_stats(ctx, p.B, p.max_outer, p.d_iters, p.d_status);
+  flush_staged(ctx, p.host);
   return rc;
 }
 
@@ -1073,232 +1103,288 @@ struct StageOut {
   }
 };
 
-// host-pointer solve, asynchronous.  Either the reference's per-problem arrays (x0, ff, caug, xref) or, with theta0/thetag,
-// start/goal pairs from which the device builds them (main_FANUC.m:38-49,98-103).  x and e_u_hist may be NULL (not copied back).
-static int solve_host_async(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
-                            const double *xref, const double *theta0, const double *thetag, const double *noise,
-                            double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
-                            double *e_u_hist, int *iters, int *status, const double *routes = nullptr, int W = 0,
-                            const int *route_len = nullptr) {
+static int check_traj_args(cfs_ctx *ctx, const char *who, int B, int H, double eta, int margin_is_D, int max_evals);
+
+// The argument checks of every solve entry, in this order: the context; robot, obstacles, cost and, for the start/goal and
+// routes forms, the cost blocks (CFS_E_STATE); the scalars and the checked solve's rules (CFS_E_ARG); B == 0 (0: nothing to
+// enqueue); NULL required buffers and the margin offsets (CFS_E_ARG).  A device form checks the offsets on the device and
+// synchronises once for that.
+static int check_solve(cfs_ctx *ctx, const SolveCall &s) {
+  if (!ctx) return CFS_E_ARG;
+  const SolveIn &in = s.in;
+  const SolveOut &o = s.out;
+  const CheckedIo *c = s.chk;
+  int rc = check_ready(ctx, true);
+  if (rc) return fail(ctx, rc, "%s: %s", s.who, ctx->err.c_str());
+  if (in.form != FORM_ARRAYS && !ctx->have_blocks)
+    return fail(ctx, CFS_E_STATE, "%s: the cost must be set with cfs_set_cost_blocks", s.who);
+  if (s.B < 0 || s.max_outer < 0) return fail(ctx, CFS_E_ARG, "%s: B=%d max_outer=%d", s.who, s.B, s.max_outer);
+  if (s.solver != CFS_SOLVER_CFS && s.solver != CFS_SOLVER_PSGCFS) return fail(ctx, CFS_E_ARG, "%s: solver=%d", s.who, s.solver);
+  if (s.grad != CFS_GRAD_NUMJAC && s.grad != CFS_GRAD_DERIVEST) return fail(ctx, CFS_E_ARG, "%s: grad=%d", s.who, s.grad);
+  if (in.form == FORM_ROUTES && in.W < 2) return fail(ctx, CFS_E_ARG, "%s: W=%d", s.who, in.W);
+  if (c) {  // the margin of the check is the solver's
+    if ((rc = check_traj_args(ctx, s.who, s.B, ctx->H, c->eta, s.solver == CFS_SOLVER_PSGCFS, c->max_evals))) return rc;
+    if (c->rounds < 0) return fail(ctx, CFS_E_ARG, "%s: rounds=%d", s.who, c->rounds);
+    if (!(c->gain > 0.0) || !std::isfinite(c->gain))
+      return fail(ctx, CFS_E_ARG, "%s: gain must be positive and finite (%g)", s.who, c->gain);
+  }
+  if (s.B == 0) return 0;
+  const bool no_in = in.form == FORM_ARRAYS       ? !in.x0 || !in.ff || !in.caug || !in.xref
+                     : in.form == FORM_START_GOAL ? !in.theta0 || !in.thetag
+                                                  : !in.routes || (in.need_len && !in.route_len);
+  if (no_in || !o.u || !o.cost_hist || !o.iters || !o.status || ((s.device || c) && !o.x) ||
+      (c && (!c->verdict || !c->t_hit || !c->cmin || !c->rounds_used)))
+    return fail(ctx, CFS_E_ARG, "%s: NULL buffer", s.who);
+  if (!in.margin_off) return 0;
+  if (s.device) {
+    CU(cudaSetDevice(ctx->device));
+    if ((rc = ensure(ctx, ctx->chk_ctr, 64))) return rc;
+    int *bad = ptr<int>(ctx->chk_ctr) + 8, hbad = 0;
+    CU(launch_offsets_bad((long long)ctx->nobs * ctx->H * s.B, in.margin_off, bad, ctx->stream));
+    CU(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    if (hbad) return fail(ctx, CFS_E_ARG, "%s: margin_off has a negative or non-finite entry", s.who);
+    return 0;
+  }
+  for (size_t e = 0, N = (size_t)ctx->nobs * ctx->H * s.B; e < N; ++e)
+    if (!(in.margin_off[e] >= 0.0 && in.margin_off[e] < INFINITY))
+      return fail(ctx, CFS_E_ARG, "%s: margin_off[%zu] = %g is negative or non-finite", s.who, e, in.margin_off[e]);
+  return 0;
+}
+
+// The context's batch buffers of a call: the problem arrays (uploaded by a host form, built on the device by the start/goal and
+// routes forms) with theta0 / thetag, and a host form's other inputs and its outputs.  Size 0: not needed.
+static int ensure_batch(cfs_ctx *ctx, const SolveCall &s) {
+  const SolveIn &in = s.in;
+  const size_t B = s.B, nj = ctx->nj, n = ctx->n, K = s.max_outer > 0 ? s.max_outer : 1, OH = (size_t)ctx->nobs * ctx->H;
+  const size_t D = sizeof(double), I = sizeof(int);
+  const bool host = !s.device, built = in.form != FORM_ARRAYS, arrays = host || built;
+  const CheckedIo *c = s.chk;
+  const struct { DevBuf &b; size_t bytes; } bufs[] = {
+      {ctx->x0, arrays ? D * 2 * nj * B : 0}, {ctx->ff, arrays ? D * n * B : 0}, {ctx->caug, arrays ? D * B : 0},
+      {ctx->xref, arrays ? D * 2 * n * B : 0}, {ctx->th0, built ? D * nj * B : 0}, {ctx->thg, built ? D * nj * B : 0},
+      {ctx->routes, host && in.routes ? D * nj * in.W * B : 0}, {ctx->rlen, host && in.route_len ? I * B : 0},
+      {ctx->noise, host && in.noise ? D * n * K * B : 0}, {ctx->rep_off, host && in.margin_off ? D * OH * B : 0},
+      {ctx->u, host ? D * n * B : 0}, {ctx->x, host ? D * 2 * n * B : 0}, {ctx->cost, host ? D * K * B : 0},
+      {ctx->eu, host ? D * K * B : 0}, {ctx->iters, host ? I * B : 0}, {ctx->status, host ? I * B : 0},
+      {ctx->chk_out, host && c ? (2 * D + 2 * I) * B + 64 : 0}, {ctx->rep_offo, host && c && c->margin_off ? D * OH * B : 0}};
+  int rc;
+  for (const auto &e : bufs)
+    if ((rc = ensure(ctx, e.b, e.bytes))) return rc;
+  return 0;
+}
+
+// One solve on device pointers: the start/goal and routes forms first build their problems into the context's batch buffers
+// (routes: N1 cubicpolytraj resampling, then the mains' set-up), then the solver, then CFS_STATUS_NO_ROUTE for the routes
+// shorter than 2 waypoints (a no-op without route_len).
+static int enqueue_solve(cfs_ctx *ctx, const SolveCall &s) {
+  const SolveIn &in = s.in;
+  const SolveOut &o = s.out;
+  const int nj = ctx->nj, H = ctx->H;
+  cudaStream_t st = ctx->stream;
+  const double *x0 = in.x0, *ff = in.ff, *caug = in.caug, *xref = in.xref;
+  if (in.form != FORM_ARRAYS) {
+    double *th0 = ptr<double>(ctx->th0), *thg = ptr<double>(ctx->thg), *bx0 = ptr<double>(ctx->x0), *bff = ptr<double>(ctx->ff),
+           *bcaug = ptr<double>(ctx->caug), *bxref = ptr<double>(ctx->xref);
+    if (in.form == FORM_ROUTES)
+      CU(launch_resample_routes(s.B, in.W, H, nj, ctx->htab.dt, in.routes, in.route_len, th0, thg, bxref, st));
+    CU(launch_build_problems(s.B, H, nj, ctx->htab.dt, ctx->dQblk, ctx->stage_w, ctx->term_w, th0, thg, bx0,
+                             in.form == FORM_ROUTES ? nullptr : bxref, bff, bcaug, st));
+    x0 = bx0, ff = bff, caug = bcaug, xref = bxref;
+  }
+  int rc = solve_device(ctx, s.B, s.solver, s.grad, x0, ff, caug, xref, in.noise, s.eps_outer, s.max_outer, s.alpha, o.u, o.x,
+                        o.cost_hist, o.e_u_hist, o.iters, o.status, in.margin_off);
+  if (rc) return rc;
+  CU(launch_mark_no_route(s.B, in.route_len, o.status, o.iters, st));
+  return 0;
+}
+
+// A host form on the context's batch buffers: the call on device pointers (d, dc) and the copies between those buffers and the
+// caller's (a NULL caller buffer is not copied)
+struct HostIo {
+  struct In { const void *host; void *dev; size_t bytes; };
+  struct Out { void *host; const void *dev; size_t bytes; };
+  SolveCall d;
+  CheckedIo dc;
+  std::vector<In> in;
+  std::vector<Out> out;
+  StageOut sout{nullptr, false};
+};
+
+// Host forms, before the enqueue: the batch buffers, the call on them and the H2D copies.  Pageable caller buffers go through
+// the context's pinned staging area (one memcpy each way) so that every copy is truly asynchronous; pinned / registered buffers
+// are used in place.
+static int upload(cfs_ctx *ctx, const SolveCall &s, HostIo &io) {
   int rc;
   CU(cudaSetDevice(ctx->device));
-  if (ctx->pending.active && (rc = finish_pending(ctx))) return rc;  // one batch in flight per context
-  const int nj = ctx->nj, n = ctx->n, K = max_outer > 0 ? max_outer : 1;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->x0, sizeof(double) * 2 * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->ff, sizeof(double) * (size_t)n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->caug, sizeof(double) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->xref, sizeof(double) * (size_t)2 * n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->u, sizeof(double) * (size_t)n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->x, sizeof(double) * (size_t)2 * n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->cost, sizeof(double) * (size_t)K * B))) return rc;
-  if ((rc = ensure(ctx, ctx->eu, sizeof(double) * (size_t)K * B))) return rc;
-  if ((rc = ensure(ctx, ctx->iters, sizeof(int) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->status, sizeof(int) * B))) return rc;
-  if (noise && (rc = ensure(ctx, ctx->noise, sizeof(double) * (size_t)n * K * B))) return rc;
+  if ((rc = finish_pending(ctx))) return rc;  // one batch in flight per context
+  if ((rc = ensure_batch(ctx, s))) return rc;
+  const size_t B = s.B, nj = ctx->nj, n = ctx->n, K = s.max_outer, K1 = K > 0 ? K : 1, OH = (size_t)ctx->nobs * ctx->H;
+  const size_t D = sizeof(double), I = sizeof(int);
+  auto up = [&](auto h, DevBuf &b, size_t bytes) {  // -> the device copy of input h (NULL: none)
+    io.in.push_back({h, b.p, bytes});
+    return h ? static_cast<decltype(h)>(b.p) : nullptr;
+  };
+  auto down = [&](auto h, void *dev, size_t bytes) {  // -> where output h is computed
+    io.out.push_back({h, dev, bytes});
+    return static_cast<decltype(h)>(dev);
+  };
+  const SolveIn &h = s.in;
+  io.d = s;
+  io.d.device = true;
+  io.d.in = {h.form, up(h.x0, ctx->x0, D * 2 * nj * B), up(h.ff, ctx->ff, D * n * B), up(h.caug, ctx->caug, D * B),
+             up(h.xref, ctx->xref, D * 2 * n * B), up(h.theta0, ctx->th0, D * nj * B), up(h.thetag, ctx->thg, D * nj * B),
+             up(h.routes, ctx->routes, D * nj * h.W * B), h.W, up(h.route_len, ctx->rlen, I * B), h.need_len,
+             up(h.noise, ctx->noise, D * n * K1 * B), up(h.margin_off, ctx->rep_off, D * OH * B)};
+  io.d.out = {down(s.out.u, ctx->u.p, D * n * B), down(s.out.x, ctx->x.p, D * 2 * n * B),
+              down(s.out.cost_hist, ctx->cost.p, D * K * B), down(s.out.e_u_hist, ctx->eu.p, D * K * B),
+              down(s.out.iters, ctx->iters.p, I * B), down(s.out.status, ctx->status.p, I * B)};
+  if (s.chk) {  // chk_out = t_hit | cmin (doubles) | verdict | rounds_used (ints)
+    const CheckedIo &c = *s.chk;
+    double *t = ptr<double>(ctx->chk_out);
+    int *v = reinterpret_cast<int *>(t + 2 * B);
+    io.dc = {c.eta, c.max_evals, c.rounds, c.gain, down(c.verdict, v, I * B), down(c.t_hit, t, D * B), down(c.cmin, t + B, D * B),
+             down(c.rounds_used, v + B, I * B), c.margin_off && OH ? down(c.margin_off, ctx->rep_offo.p, D * OH * B) : nullptr};
+    io.d.chk = &io.dc;
+  }
+  auto staged = [](const auto &copies, size_t &bytes) {  // -> some caller buffer is pageable; bytes: the staging area they take
+    bool pageable = false;
+    for (const auto &e : copies)
+      if (e.host && e.bytes) { bytes += (e.bytes + 255) / 256 * 256; pageable = pageable || !is_pinned_host(e.host); }
+    return pageable;
+  };
+  size_t in_bytes = 0, out_bytes = 0;
+  StageIn sin{ctx, staged(io.in, in_bytes)};
+  io.sout = {ctx, staged(io.out, out_bytes)};
+  if (sin.use && (rc = ensure_stage(ctx, ctx->stage_in, ctx->stage_in_cap, in_bytes))) return rc;
+  if (io.sout.use && (rc = ensure_stage(ctx, ctx->stage_out, ctx->stage_out_cap, out_bytes))) return rc;
+  ctx->copy_back.clear();
   for (cudaEvent_t &e : ctx->ev_h)
     if (!e) CU(cudaEventCreate(&e));
-  // pageable caller buffers go through the context's pinned staging area (one memcpy each way) so that every copy below is
-  // truly asynchronous; pinned / registered buffers are used in place
-  const size_t al = 256;
-  auto pad = [al](size_t b) { return (b + al - 1) / al * al; };
-  size_t in_bytes = 0, out_bytes = 0;
-  bool pinned_in = true, pinned_out = true;
-  auto in = [&](const void *hp, size_t b) { if (hp && b) { in_bytes += pad(b); pinned_in = pinned_in && is_pinned_host(hp); } };
-  auto outb = [&](const void *hp, size_t b) { if (hp && b) { out_bytes += pad(b); pinned_out = pinned_out && is_pinned_host(hp); } };
-  in(routes, sizeof(double) * (size_t)nj * W * B); in(route_len, sizeof(int) * B);
-  in(theta0, sizeof(double) * nj * B); in(thetag, sizeof(double) * nj * B);
-  in(x0, sizeof(double) * 2 * nj * B); in(ff, sizeof(double) * (size_t)n * B); in(caug, sizeof(double) * B);
-  in(xref, sizeof(double) * (size_t)2 * n * B); in(noise, sizeof(double) * (size_t)n * K * B);
-  outb(u, sizeof(double) * (size_t)n * B); outb(x, sizeof(double) * (size_t)2 * n * B);
-  outb(cost_hist, sizeof(double) * (size_t)max_outer * B); outb(e_u_hist, sizeof(double) * (size_t)max_outer * B);
-  outb(iters, sizeof(int) * B); outb(status, sizeof(int) * B);
-  StageIn sin{ctx, !pinned_in};
-  StageOut sout{ctx, !pinned_out};
-  if (sin.use && (rc = ensure_stage(ctx, ctx->stage_in, ctx->stage_in_cap, in_bytes))) return rc;
-  if (sout.use && (rc = ensure_stage(ctx, ctx->stage_out, ctx->stage_out_cap, out_bytes))) return rc;
-  ctx->copy_back.clear();
-  ctx->staged_last = sin.use || sout.use;
-  CU(cudaEventRecord(ctx->ev_h[0], st));
+  CU(cudaEventRecord(ctx->ev_h[0], ctx->stream));
   {
     NvtxRange r("cfs:h2d");
-    if (routes) {
-      if ((rc = ensure(ctx, ctx->th0, sizeof(double) * nj * B))) return rc;
-      if ((rc = ensure(ctx, ctx->thg, sizeof(double) * nj * B))) return rc;
-      if ((rc = ensure(ctx, ctx->routes, sizeof(double) * (size_t)nj * W * B))) return rc;
-      CU(sin.put(ctx->routes.p, routes, sizeof(double) * (size_t)nj * W * B, st));
-      if (route_len) {
-        if ((rc = ensure(ctx, ctx->rlen, sizeof(int) * B))) return rc;
-        CU(sin.put(ctx->rlen.p, route_len, sizeof(int) * B, st));
-      }
-    } else if (theta0) {
-      if ((rc = ensure(ctx, ctx->th0, sizeof(double) * nj * B))) return rc;
-      if ((rc = ensure(ctx, ctx->thg, sizeof(double) * nj * B))) return rc;
-      CU(sin.put(ctx->th0.p, theta0, sizeof(double) * nj * B, st));
-      CU(sin.put(ctx->thg.p, thetag, sizeof(double) * nj * B, st));
-    } else {
-      CU(sin.put(ctx->x0.p, x0, sizeof(double) * 2 * nj * B, st));
-      CU(sin.put(ctx->ff.p, ff, sizeof(double) * (size_t)n * B, st));
-      CU(sin.put(ctx->caug.p, caug, sizeof(double) * B, st));
-      CU(sin.put(ctx->xref.p, xref, sizeof(double) * (size_t)2 * n * B, st));
-    }
-    if (noise) CU(sin.put(ctx->noise.p, noise, sizeof(double) * (size_t)n * K * B, st));
+    for (const HostIo::In &e : io.in) CU(sin.put(e.dev, e.host, e.bytes, ctx->stream));
   }
-  CU(cudaEventRecord(ctx->ev_h[1], st));
-  if (routes) {  // N1: cubicpolytraj resampling, then the same problem set-up around that reference
-    CU(launch_resample_routes(B, W, ctx->H, nj, ctx->htab.dt, ptr<double>(ctx->routes), route_len ? ptr<int>(ctx->rlen) : nullptr,
-                              ptr<double>(ctx->th0), ptr<double>(ctx->thg), ptr<double>(ctx->xref), st));
-    CU(launch_build_problems(B, ctx->H, nj, ctx->htab.dt, ctx->dQblk, ctx->stage_w, ctx->term_w, ptr<double>(ctx->th0),
-                             ptr<double>(ctx->thg), ptr<double>(ctx->x0), nullptr, ptr<double>(ctx->ff),
-                             ptr<double>(ctx->caug), st));
-  } else if (theta0) {
-    CU(launch_build_problems(B, ctx->H, nj, ctx->htab.dt, ctx->dQblk, ctx->stage_w, ctx->term_w, ptr<double>(ctx->th0),
-                             ptr<double>(ctx->thg), ptr<double>(ctx->x0), ptr<double>(ctx->xref), ptr<double>(ctx->ff),
-                             ptr<double>(ctx->caug), st));
-  }
-  rc = solve_device(ctx, B, solver, grad, ptr<double>(ctx->x0), ptr<double>(ctx->ff), ptr<double>(ctx->caug),
-                    ptr<double>(ctx->xref), noise ? ptr<double>(ctx->noise) : nullptr, eps_outer, max_outer, alpha,
-                    ptr<double>(ctx->u), ptr<double>(ctx->x), ptr<double>(ctx->cost), ptr<double>(ctx->eu),
-                    ptr<int>(ctx->iters), ptr<int>(ctx->status));
-  if (rc) return rc;
-  if (routes && route_len) CU(launch_mark_no_route(B, ptr<int>(ctx->rlen), ptr<int>(ctx->status), ptr<int>(ctx->iters), st));
-  CU(cudaEventRecord(ctx->ev_h[2], st));
+  CU(cudaEventRecord(ctx->ev_h[1], ctx->stream));
+  return 0;
+}
+
+// Host forms, after the enqueue: the D2H copies (staged ones reach the caller's buffers in flush_staged)
+static int download(cfs_ctx *ctx, HostIo &io) {
+  CU(cudaEventRecord(ctx->ev_h[2], ctx->stream));
   {
     NvtxRange r("cfs:d2h");
-    CU(sout.get(u, ctx->u.p, sizeof(double) * (size_t)n * B, st));
-    CU(sout.get(x, ctx->x.p, sizeof(double) * (size_t)2 * n * B, st));  // x, e_u_hist may be NULL: not copied back
-    CU(sout.get(cost_hist, ctx->cost.p, sizeof(double) * (size_t)max_outer * B, st));
-    CU(sout.get(e_u_hist, ctx->eu.p, sizeof(double) * (size_t)max_outer * B, st));
-    CU(sout.get(iters, ctx->iters.p, sizeof(int) * B, st));
-    CU(sout.get(status, ctx->status.p, sizeof(int) * B, st));
+    for (const HostIo::Out &e : io.out) CU(io.sout.get(e.host, e.dev, e.bytes, ctx->stream));
   }
-  CU(cudaEventRecord(ctx->ev_h[3], st));
-  ctx->pending.active = true;
-  ctx->pending.host = true;
-  ctx->pending.B = B;
-  ctx->pending.max_outer = max_outer;
-  ctx->pending.d_iters = ptr<int>(ctx->iters);
-  ctx->pending.d_status = ptr<int>(ctx->status);
+  CU(cudaEventRecord(ctx->ev_h[3], ctx->stream));
   return 0;
+}
+
+// Every entry but the checked solve's: a host form through the staging area, a device form on the caller's pointers;
+// asynchronous, or followed by cfs_wait
+static int solve(cfs_ctx *ctx, const SolveCall &s, bool wait) {
+  int rc = check_solve(ctx, s);
+  if (rc || s.B == 0) return rc;
+  HostIo io;
+  if (s.device) {
+    CU(cudaSetDevice(ctx->device));
+    set_pending(ctx);  // statistics of an un-waited earlier batch are dropped
+    if ((rc = ensure_batch(ctx, s)) || (rc = enqueue_solve(ctx, s))) return rc;
+  } else if ((rc = upload(ctx, s, io)) || (rc = enqueue_solve(ctx, io.d)) || (rc = download(ctx, io))) {
+    return rc;
+  }
+  set_pending(ctx, s.device ? &s : &io.d, !s.device);
+  return wait ? cfs_wait(ctx) : 0;
+}
+
+extern "C" int cfs_solve_batch(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                               const double *caug, const double *xref, const double *noise, double eps_outer,
+                               int max_outer, double alpha, double *u, double *x, double *cost_hist, double *e_u_hist,
+                               int *iters, int *status) {
+  return solve(ctx, {"cfs_solve_batch", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise), {u, x, cost_hist, e_u_hist, iters, status}}, true);
 }
 
 extern "C" int cfs_solve_batch_async(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
                                      const double *caug, const double *xref, const double *noise, double eps_outer,
                                      int max_outer, double alpha, double *u, double *x, double *cost_hist,
                                      double *e_u_hist, int *iters, int *status) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  return solve_host_async(ctx, B, solver, grad, x0, ff, caug, xref, nullptr, nullptr, noise, eps_outer, max_outer, alpha, u, x,
-                          cost_hist, e_u_hist, iters, status);
+  return solve(ctx, {"cfs_solve_batch_async", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise), {u, x, cost_hist, e_u_hist, iters, status}}, false);
+}
+
+extern "C" int cfs_solve_start_goal(cfs_ctx *ctx, int B, int solver, int grad, const double *theta0, const double *thetag,
+                                    const double *noise, double eps_outer, int max_outer, double alpha, double *u, double *x,
+                                    double *cost_hist, double *e_u_hist, int *iters, int *status) {
+  return solve(ctx, {"cfs_solve_start_goal", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    start_goal_in(theta0, thetag, noise), {u, x, cost_hist, e_u_hist, iters, status}}, true);
 }
 
 extern "C" int cfs_solve_start_goal_async(cfs_ctx *ctx, int B, int solver, int grad, const double *theta0, const double *thetag,
                                           const double *noise, double eps_outer, int max_outer, double alpha, double *u,
                                           double *x, double *cost_hist, double *e_u_hist, int *iters, int *status) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, true);
-  if (rc) return rc;
-  if (!ctx->have_blocks) return fail(ctx, CFS_E_STATE, "cfs_solve_start_goal: the cost must be set with cfs_set_cost_blocks");
-  if (B < 0 || max_outer < 0 || (solver != CFS_SOLVER_CFS && solver != CFS_SOLVER_PSGCFS) ||
-      (grad != CFS_GRAD_NUMJAC && grad != CFS_GRAD_DERIVEST))
-    return fail(ctx, CFS_E_ARG, "cfs_solve_start_goal: bad argument");
-  if (B > 0 && (!theta0 || !thetag || !u || !cost_hist || !iters || !status))
-    return fail(ctx, CFS_E_ARG, "cfs_solve_start_goal: NULL buffer");
-  if (B == 0) return 0;
-  return solve_host_async(ctx, B, solver, grad, nullptr, nullptr, nullptr, nullptr, theta0, thetag, noise, eps_outer, max_outer,
-                          alpha, u, x, cost_hist, e_u_hist, iters, status);
-}
-
-extern "C" int cfs_solve_routes_async(cfs_ctx *ctx, int B, int W, int solver, int grad, const double *routes, const double *noise,
-                                      double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
-                                      double *e_u_hist, int *iters, int *status) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, true);
-  if (rc) return rc;
-  if (!ctx->have_blocks) return fail(ctx, CFS_E_STATE, "cfs_solve_routes: the cost must be set with cfs_set_cost_blocks");
-  if (B < 0 || W < 2 || max_outer < 0 || (solver != CFS_SOLVER_CFS && solver != CFS_SOLVER_PSGCFS) ||
-      (grad != CFS_GRAD_NUMJAC && grad != CFS_GRAD_DERIVEST))
-    return fail(ctx, CFS_E_ARG, "cfs_solve_routes: bad argument");
-  if (B > 0 && (!routes || !u || !cost_hist || !iters || !status)) return fail(ctx, CFS_E_ARG, "cfs_solve_routes: NULL buffer");
-  if (B == 0) return 0;
-  return solve_host_async(ctx, B, solver, grad, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, noise, eps_outer, max_outer,
-                          alpha, u, x, cost_hist, e_u_hist, iters, status, routes, W);
+  return solve(ctx, {"cfs_solve_start_goal_async", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    start_goal_in(theta0, thetag, noise), {u, x, cost_hist, e_u_hist, iters, status}}, false);
 }
 
 extern "C" int cfs_solve_routes(cfs_ctx *ctx, int B, int W, int solver, int grad, const double *routes, const double *noise,
                                 double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
                                 double *e_u_hist, int *iters, int *status) {
-  int rc = cfs_solve_routes_async(ctx, B, W, solver, grad, routes, noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist,
-                                  iters, status);
-  if (rc || B == 0) return rc;
-  return cfs_wait(ctx);
+  return solve(ctx, {"cfs_solve_routes", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    routes_in(routes, W, nullptr, false, noise), {u, x, cost_hist, e_u_hist, iters, status}}, true);
 }
 
-static int check_routes_args(cfs_ctx *ctx, const char *who, int B, int W, int solver, int grad, int max_outer, const void *routes,
-                             const void *u, const void *cost_hist, const void *iters, const void *status) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, true);
-  if (rc) return rc;
-  if (!ctx->have_blocks) return fail(ctx, CFS_E_STATE, "%s: the cost must be set with cfs_set_cost_blocks", who);
-  if (B < 0 || W < 2 || max_outer < 0 || (solver != CFS_SOLVER_CFS && solver != CFS_SOLVER_PSGCFS) ||
-      (grad != CFS_GRAD_NUMJAC && grad != CFS_GRAD_DERIVEST))
-    return fail(ctx, CFS_E_ARG, "%s: bad argument", who);
-  if (B > 0 && (!routes || !u || !cost_hist || !iters || !status)) return fail(ctx, CFS_E_ARG, "%s: NULL buffer", who);
-  return 0;
-}
-
-extern "C" int cfs_solve_routes_var_async(cfs_ctx *ctx, int B, int W, const int *route_len, int solver, int grad,
-                                          const double *routes, const double *noise, double eps_outer, int max_outer, double alpha,
-                                          double *u, double *x, double *cost_hist, double *e_u_hist, int *iters, int *status) {
-  int rc = check_routes_args(ctx, "cfs_solve_routes_var", B, W, solver, grad, max_outer, routes, u, cost_hist, iters, status);
-  if (rc || B == 0) return rc;
-  if (!route_len) return fail(ctx, CFS_E_ARG, "cfs_solve_routes_var: NULL route_len");
-  return solve_host_async(ctx, B, solver, grad, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, noise, eps_outer, max_outer,
-                          alpha, u, x, cost_hist, e_u_hist, iters, status, routes, W, route_len);
+extern "C" int cfs_solve_routes_async(cfs_ctx *ctx, int B, int W, int solver, int grad, const double *routes, const double *noise,
+                                      double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                                      double *e_u_hist, int *iters, int *status) {
+  return solve(ctx, {"cfs_solve_routes_async", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    routes_in(routes, W, nullptr, false, noise), {u, x, cost_hist, e_u_hist, iters, status}}, false);
 }
 
 extern "C" int cfs_solve_routes_var(cfs_ctx *ctx, int B, int W, const int *route_len, int solver, int grad, const double *routes,
                                     const double *noise, double eps_outer, int max_outer, double alpha, double *u, double *x,
                                     double *cost_hist, double *e_u_hist, int *iters, int *status) {
-  int rc = cfs_solve_routes_var_async(ctx, B, W, route_len, solver, grad, routes, noise, eps_outer, max_outer, alpha, u, x, cost_hist,
-                                      e_u_hist, iters, status);
-  if (rc || B == 0) return rc;
-  return cfs_wait(ctx);
+  return solve(ctx, {"cfs_solve_routes_var", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    routes_in(routes, W, route_len, true, noise), {u, x, cost_hist, e_u_hist, iters, status}}, true);
+}
+
+extern "C" int cfs_solve_routes_var_async(cfs_ctx *ctx, int B, int W, const int *route_len, int solver, int grad,
+                                          const double *routes, const double *noise, double eps_outer, int max_outer, double alpha,
+                                          double *u, double *x, double *cost_hist, double *e_u_hist, int *iters, int *status) {
+  return solve(ctx, {"cfs_solve_routes_var_async", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    routes_in(routes, W, route_len, true, noise), {u, x, cost_hist, e_u_hist, iters, status}}, false);
 }
 
 extern "C" int cfs_solve_routes_device(cfs_ctx *ctx, int B, int W, const int *route_len, int solver, int grad, const double *routes,
                                        const double *noise, double eps_outer, int max_outer, double alpha, double *u, double *x,
                                        double *cost_hist, double *e_u_hist, int *iters, int *status, int sync) {
-  int rc = check_routes_args(ctx, "cfs_solve_routes_device", B, W, solver, grad, max_outer, routes, u, cost_hist, iters, status);
-  if (rc || B == 0) return rc;
-  if (!x) return fail(ctx, CFS_E_ARG, "cfs_solve_routes_device: NULL x");
-  CU(cudaSetDevice(ctx->device));
-  ctx->pending.active = false;
-  const int nj = ctx->nj, n = ctx->n;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->x0, sizeof(double) * 2 * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->ff, sizeof(double) * (size_t)n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->caug, sizeof(double) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->xref, sizeof(double) * (size_t)2 * n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->th0, sizeof(double) * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->thg, sizeof(double) * nj * B))) return rc;
-  CU(launch_resample_routes(B, W, ctx->H, nj, ctx->htab.dt, routes, route_len, ptr<double>(ctx->th0), ptr<double>(ctx->thg),
-                            ptr<double>(ctx->xref), st));
-  CU(launch_build_problems(B, ctx->H, nj, ctx->htab.dt, ctx->dQblk, ctx->stage_w, ctx->term_w, ptr<double>(ctx->th0),
-                           ptr<double>(ctx->thg), ptr<double>(ctx->x0), nullptr, ptr<double>(ctx->ff), ptr<double>(ctx->caug), st));
-  rc = solve_device(ctx, B, solver, grad, ptr<double>(ctx->x0), ptr<double>(ctx->ff), ptr<double>(ctx->caug), ptr<double>(ctx->xref),
-                    noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist, iters, status);
-  if (rc) return rc;
-  CU(launch_mark_no_route(B, route_len, status, iters, st));
-  ctx->pending.active = true;
-  ctx->pending.host = false;
-  ctx->pending.B = B;
-  ctx->pending.max_outer = max_outer;
-  ctx->pending.d_iters = iters;
-  ctx->pending.d_status = status;
-  if (sync) return finish_pending(ctx);
-  return 0;
+  return solve(ctx, {"cfs_solve_routes_device", true, B, solver, grad, eps_outer, max_outer, alpha,
+                    routes_in(routes, W, route_len, false, noise), {u, x, cost_hist, e_u_hist, iters, status}}, sync);
+}
+
+extern "C" int cfs_solve_batch_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                      const double *caug, const double *xref, const double *noise, double eps_outer,
+                                      int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                                      double *e_u_hist, int *iters, int *status, int sync) {
+  return solve(ctx, {"cfs_solve_batch_device", true, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise), {u, x, cost_hist, e_u_hist, iters, status}}, sync);
+}
+
+extern "C" int cfs_solve_batch_margins(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                       const double *caug, const double *xref, const double *noise, const double *margin_off,
+                                       double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
+                                       double *e_u_hist, int *iters, int *status) {
+  return solve(ctx, {"cfs_solve_batch_margins", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise, margin_off), {u, x, cost_hist, e_u_hist, iters, status}}, true);
+}
+
+extern "C" int cfs_solve_batch_margins_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
+                                              const double *caug, const double *xref, const double *noise, const double *margin_off,
+                                              double eps_outer, int max_outer, double alpha, double *u, double *x,
+                                              double *cost_hist, double *e_u_hist, int *iters, int *status, int sync) {
+  return solve(ctx, {"cfs_solve_batch_margins_device", true, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise, margin_off), {u, x, cost_hist, e_u_hist, iters, status}}, sync);
 }
 
 extern "C" int cfs_resample_routes(cfs_ctx *ctx, int B, int W, int H, const double *routes, double *sampled) {
@@ -1326,25 +1412,6 @@ extern "C" int cfs_resample_routes(cfs_ctx *ctx, int B, int W, int H, const doub
                          cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return 0;
-}
-
-extern "C" int cfs_solve_start_goal(cfs_ctx *ctx, int B, int solver, int grad, const double *theta0, const double *thetag,
-                                    const double *noise, double eps_outer, int max_outer, double alpha, double *u, double *x,
-                                    double *cost_hist, double *e_u_hist, int *iters, int *status) {
-  int rc = cfs_solve_start_goal_async(ctx, B, solver, grad, theta0, thetag, noise, eps_outer, max_outer, alpha, u, x, cost_hist,
-                                      e_u_hist, iters, status);
-  if (rc || B == 0) return rc;
-  return cfs_wait(ctx);
-}
-
-extern "C" int cfs_solve_batch(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
-                               const double *caug, const double *xref, const double *noise, double eps_outer,
-                               int max_outer, double alpha, double *u, double *x, double *cost_hist, double *e_u_hist,
-                               int *iters, int *status) {
-  int rc = cfs_solve_batch_async(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x,
-                                 cost_hist, e_u_hist, iters, status);
-  if (rc || B == 0) return rc;
-  return cfs_wait(ctx);
 }
 
 // ---- CHOMP_FANUC (Lib/CHOMP_FANUC.m), k_chomp.cu ----------------------------------------------------------------------
@@ -1737,146 +1804,27 @@ extern "C" int cfs_check_trajectories(cfs_ctx *ctx, int B, int H, const double *
   return 0;
 }
 
-// ---- per-waypoint margin offsets and the checked solve (include/cfs_b200.h) ----------------------------------------------------
-static int check_offsets_device(cfs_ctx *ctx, const char *who, int B, const double *margin_off) {
-  const long long N = (long long)ctx->nobs * ctx->H * B;
-  int rc;
-  if (!margin_off) return 0;
-  if ((rc = ensure(ctx, ctx->chk_ctr, 64))) return rc;
-  int *bad = ptr<int>(ctx->chk_ctr) + 8, hbad = 0;
-  CU(launch_offsets_bad(N, margin_off, bad, ctx->stream));
-  CU(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  if (hbad) return fail(ctx, CFS_E_ARG, "%s: margin_off has a negative or non-finite entry", who);
-  return 0;
-}
-
-extern "C" int cfs_solve_batch_margins_device(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
-                                              const double *caug, const double *xref, const double *noise, const double *margin_off,
-                                              double eps_outer, int max_outer, double alpha, double *u, double *x,
-                                              double *cost_hist, double *e_u_hist, int *iters, int *status, int sync) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  if (!x) return fail(ctx, CFS_E_ARG, "cfs_solve_batch_margins_device: NULL x");
-  CU(cudaSetDevice(ctx->device));
-  if ((rc = check_offsets_device(ctx, "cfs_solve_batch_margins_device", B, margin_off))) return rc;
-  ctx->pending.active = false;
-  rc = solve_device(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist, iters,
-                    status, margin_off);
-  if (rc) return rc;
-  ctx->pending.active = true;
-  ctx->pending.host = false;
-  ctx->pending.B = B;
-  ctx->pending.max_outer = max_outer;
-  ctx->pending.d_iters = iters;
-  ctx->pending.d_status = status;
-  if (sync) return finish_pending(ctx);
-  return 0;
-}
-
-// host form of the margin / checked solves: inputs to the context's batch buffers, the device form, results back (synchronous)
-struct HostBatch {
-  double *x0, *ff, *caug, *xref, *noise, *off, *u, *x, *ch, *eu;
-  int *iters, *status;
-};
-static int host_batch_in(cfs_ctx *ctx, int B, int max_outer, const double *x0, const double *ff, const double *caug,
-                         const double *xref, const double *noise, const double *off, HostBatch &d) {
-  const int nj = ctx->nj, n = ctx->n, K = max_outer > 0 ? max_outer : 1;
-  const size_t OH = (size_t)ctx->nobs * ctx->H;
-  cudaStream_t st = ctx->stream;
-  int rc;
-  if (ctx->pending.active && (rc = finish_pending(ctx))) return rc;
-  if ((rc = ensure(ctx, ctx->x0, sizeof(double) * 2 * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->ff, sizeof(double) * (size_t)n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->caug, sizeof(double) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->xref, sizeof(double) * (size_t)2 * n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->u, sizeof(double) * (size_t)n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->x, sizeof(double) * (size_t)2 * n * B))) return rc;
-  if ((rc = ensure(ctx, ctx->cost, sizeof(double) * (size_t)K * B))) return rc;
-  if ((rc = ensure(ctx, ctx->eu, sizeof(double) * (size_t)K * B))) return rc;
-  if ((rc = ensure(ctx, ctx->iters, sizeof(int) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->status, sizeof(int) * B))) return rc;
-  if (noise && (rc = ensure(ctx, ctx->noise, sizeof(double) * (size_t)n * K * B))) return rc;
-  if ((rc = ensure(ctx, ctx->rep_off, sizeof(double) * (OH ? OH : 1) * B))) return rc;
-  d.x0 = ptr<double>(ctx->x0); d.ff = ptr<double>(ctx->ff); d.caug = ptr<double>(ctx->caug); d.xref = ptr<double>(ctx->xref);
-  d.noise = noise ? ptr<double>(ctx->noise) : nullptr;
-  d.off = off ? ptr<double>(ctx->rep_off) : nullptr;
-  d.u = ptr<double>(ctx->u); d.x = ptr<double>(ctx->x); d.ch = ptr<double>(ctx->cost); d.eu = ptr<double>(ctx->eu);
-  d.iters = ptr<int>(ctx->iters); d.status = ptr<int>(ctx->status);
-  CU(cudaMemcpyAsync(d.x0, x0, sizeof(double) * 2 * nj * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d.ff, ff, sizeof(double) * (size_t)n * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d.caug, caug, sizeof(double) * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d.xref, xref, sizeof(double) * (size_t)2 * n * B, cudaMemcpyHostToDevice, st));
-  if (noise) CU(cudaMemcpyAsync(d.noise, noise, sizeof(double) * (size_t)n * K * B, cudaMemcpyHostToDevice, st));
-  if (off && OH) CU(cudaMemcpyAsync(d.off, off, sizeof(double) * OH * B, cudaMemcpyHostToDevice, st));
-  return 0;
-}
-static int host_batch_out(cfs_ctx *ctx, int B, int max_outer, const HostBatch &d, double *u, double *x, double *cost_hist,
-                          double *e_u_hist, int *iters, int *status) {
-  const int n = ctx->n;
-  cudaStream_t st = ctx->stream;
-  CU(cudaMemcpyAsync(u, d.u, sizeof(double) * (size_t)n * B, cudaMemcpyDeviceToHost, st));
-  if (x) CU(cudaMemcpyAsync(x, d.x, sizeof(double) * (size_t)2 * n * B, cudaMemcpyDeviceToHost, st));
-  if (max_outer > 0) {
-    CU(cudaMemcpyAsync(cost_hist, d.ch, sizeof(double) * (size_t)max_outer * B, cudaMemcpyDeviceToHost, st));
-    if (e_u_hist) CU(cudaMemcpyAsync(e_u_hist, d.eu, sizeof(double) * (size_t)max_outer * B, cudaMemcpyDeviceToHost, st));
-  }
-  CU(cudaMemcpyAsync(iters, d.iters, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(status, d.status, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
-}
-
-extern "C" int cfs_solve_batch_margins(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff,
-                                       const double *caug, const double *xref, const double *noise, const double *margin_off,
-                                       double eps_outer, int max_outer, double alpha, double *u, double *x, double *cost_hist,
-                                       double *e_u_hist, int *iters, int *status) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  if (margin_off)
-    for (size_t e = 0, N = (size_t)ctx->nobs * ctx->H * B; e < N; ++e)
-      if (!(margin_off[e] >= 0.0 && margin_off[e] < INFINITY))
-        return fail(ctx, CFS_E_ARG, "cfs_solve_batch_margins: margin_off[%zu] = %g is negative or not finite", e, margin_off[e]);
-  CU(cudaSetDevice(ctx->device));
-  HostBatch d;
-  if ((rc = host_batch_in(ctx, B, max_outer, x0, ff, caug, xref, noise, margin_off, d))) return rc;
-  ctx->pending.active = false;
-  rc = solve_device(ctx, B, solver, grad, d.x0, d.ff, d.caug, d.xref, d.noise, eps_outer, max_outer, alpha, d.u, d.x, d.ch,
-                    e_u_hist ? d.eu : nullptr, d.iters, d.status, d.off);
-  if (rc) return rc;
-  if ((rc = collect_stats(ctx, B, max_outer, d.iters, d.status))) return rc;
-  return host_batch_out(ctx, B, max_outer, d, u, x, cost_hist, e_u_hist, iters, status);
-}
-
-static int check_checked_args(cfs_ctx *ctx, const char *who, int B, int solver, double eta, int max_evals, int rounds, double gain) {
-  int rc = check_traj_args(ctx, who, B, ctx->H > 0 ? ctx->H : 1, eta, solver == CFS_SOLVER_PSGCFS, max_evals);
-  if (rc) return rc;
-  if (rounds < 0) return fail(ctx, CFS_E_ARG, "%s: rounds=%d", who, rounds);
-  if (!(gain > 0.0) || !std::isfinite(gain)) return fail(ctx, CFS_E_ARG, "%s: gain must be positive and finite (%g)", who, gain);
-  return 0;
-}
-
+// ---- the checked solve (include/cfs_b200.h) ------------------------------------------------------------------------
 // The round loop.  Problem-indexed state lives in the caller's (device) buffers; the sub-batch of a round (at most B problems) in
 // context buffers: rep_in = x0 | ff | caug | xref | noise | offsets, rep_out = u | x | cost | e_u | verdict | t_hit | cmin (doubles)
 // then iters | status | verdict (ints), rep_list = sel | list A | list B | count.  rep_off holds the accumulated offsets of every
 // problem; margin_off_out (NULL: not returned) receives the offsets of the round each returned solution comes from.
-static int solve_checked_dev(cfs_ctx *ctx, int B, int solver, int grad, const double *x0, const double *ff, const double *caug,
-                             const double *xref, const double *noise, double eps_outer, int max_outer, double alpha, double eta,
-                             int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
-                             int *iters, int *status, int *verdict, double *t_hit, double *cmin, int *rounds_used,
-                             double *margin_off_out) {
+static int solve_checked_dev(cfs_ctx *ctx, const SolveCall &s) {
+  const CheckedIo &c = *s.chk;
+  const int B = s.B, solver = s.solver, grad = s.grad, max_outer = s.max_outer, max_evals = c.max_evals, rounds = c.rounds;
+  const double eps_outer = s.eps_outer, alpha = s.alpha, eta = c.eta, gain = c.gain;
+  const double *x0 = s.in.x0, *ff = s.in.ff, *caug = s.in.caug, *xref = s.in.xref, *noise = s.in.noise;
+  double *u = s.out.u, *x = s.out.x, *cost_hist = s.out.cost_hist, *e_u_hist = s.out.e_u_hist, *t_hit = c.t_hit, *cmin = c.cmin,
+         *margin_off_out = c.margin_off;
+  int *iters = s.out.iters, *status = s.out.status, *verdict = c.verdict, *rounds_used = c.rounds_used;
   const int nj = ctx->nj, n = ctx->n, H = ctx->H, O = ctx->nobs, K = max_outer;
   const size_t OH = (size_t)O * H, nx0 = 2 * nj, N = 2 * (size_t)n, nnz = noise ? (size_t)n * K : 0;
   const int margin_is_D = solver == CFS_SOLVER_PSGCFS;
   cudaStream_t st = ctx->stream;
   int rc;
-  ctx->pending.active = false;
+  set_pending(ctx);
   // round 0: the plain solve and its check
-  if ((rc = solve_device(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, u, x, cost_hist, e_u_hist,
-                         iters, status)))
-    return rc;
+  if ((rc = enqueue_solve(ctx, s))) return rc;
   if ((rc = collect_stats(ctx, B, max_outer, iters, status))) return rc;  // cfs_get_stats: round 0's solve
   if ((rc = check_traj_dev(ctx, B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin, nullptr))) return rc;
   CU(cudaMemsetAsync(rounds_used, 0, sizeof(int) * B, st));
@@ -1958,15 +1906,13 @@ extern "C" int cfs_solve_checked_device(cfs_ctx *ctx, int B, int solver, int gra
                                         int max_outer, double alpha, double eta, int max_evals, int rounds, double gain, double *u,
                                         double *x, double *cost_hist, double *e_u_hist, int *iters, int *status, int *verdict,
                                         double *t_hit, double *cmin, int *rounds_used, double *margin_off, int sync) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if ((rc = check_checked_args(ctx, "cfs_solve_checked_device", B, solver, eta, max_evals, rounds, gain))) return rc;
-  if (B == 0) return 0;
-  if (!x || !verdict || !t_hit || !cmin || !rounds_used) return fail(ctx, CFS_E_ARG, "cfs_solve_checked_device: NULL buffer");
+  const CheckedIo c{eta, max_evals, rounds, gain, verdict, t_hit, cmin, rounds_used, margin_off};
+  const SolveCall s{"cfs_solve_checked_device", true, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise), {u, x, cost_hist, e_u_hist, iters, status}, &c};
+  int rc = check_solve(ctx, s);
+  if (rc || B == 0) return rc;
   CU(cudaSetDevice(ctx->device));
-  if ((rc = solve_checked_dev(ctx, B, solver, grad, x0, ff, caug, xref, noise, eps_outer, max_outer, alpha, eta, max_evals, rounds,
-                              gain, u, x, cost_hist, e_u_hist, iters, status, verdict, t_hit, cmin, rounds_used, margin_off)))
-    return rc;
+  if ((rc = solve_checked_dev(ctx, s))) return rc;
   if (sync) CU(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
@@ -1976,34 +1922,16 @@ extern "C" int cfs_solve_checked(cfs_ctx *ctx, int B, int solver, int grad, cons
                                  int max_evals, int rounds, double gain, double *u, double *x, double *cost_hist, double *e_u_hist,
                                  int *iters, int *status, int *verdict, double *t_hit, double *cmin, int *rounds_used,
                                  double *margin_off) {
-  int rc = check_solve_args(ctx, B, solver, grad, x0, ff, caug, xref, max_outer, u, x, cost_hist, iters, status);
-  if (rc) return rc;
-  if ((rc = check_checked_args(ctx, "cfs_solve_checked", B, solver, eta, max_evals, rounds, gain))) return rc;
-  if (B == 0) return 0;
-  if (!x || !verdict || !t_hit || !cmin || !rounds_used) return fail(ctx, CFS_E_ARG, "cfs_solve_checked: NULL buffer");
-  CU(cudaSetDevice(ctx->device));
-  HostBatch d;
-  if ((rc = host_batch_in(ctx, B, max_outer, x0, ff, caug, xref, noise, nullptr, d))) return rc;
-  const size_t OH = (size_t)ctx->nobs * ctx->H;
-  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)B + 64))) return rc;
-  double *d_t = ptr<double>(ctx->chk_out), *d_c = d_t + B;
-  int *d_v = reinterpret_cast<int *>(d_c + B), *d_r = d_v + B;
-  double *d_off = nullptr;
-  if (margin_off && OH) {
-    if ((rc = ensure(ctx, ctx->rep_offo, sizeof(double) * OH * B))) return rc;
-    d_off = ptr<double>(ctx->rep_offo);
-  }
-  if ((rc = solve_checked_dev(ctx, B, solver, grad, d.x0, d.ff, d.caug, d.xref, d.noise, eps_outer, max_outer, alpha, eta, max_evals,
-                              rounds, gain, d.u, d.x, d.ch, e_u_hist ? d.eu : nullptr, d.iters, d.status, d_v, d_t, d_c, d_r,
-                              d_off)))
-    return rc;
-  cudaStream_t st = ctx->stream;
-  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(t_hit, d_t, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(rounds_used, d_r, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-  if (d_off) CU(cudaMemcpyAsync(margin_off, d_off, sizeof(double) * OH * B, cudaMemcpyDeviceToHost, st));
-  return host_batch_out(ctx, B, max_outer, d, u, x, cost_hist, e_u_hist, iters, status);
+  const CheckedIo c{eta, max_evals, rounds, gain, verdict, t_hit, cmin, rounds_used, margin_off};
+  const SolveCall s{"cfs_solve_checked", false, B, solver, grad, eps_outer, max_outer, alpha,
+                    arrays_in(x0, ff, caug, xref, noise), {u, x, cost_hist, e_u_hist, iters, status}, &c};
+  int rc = check_solve(ctx, s);
+  if (rc || B == 0) return rc;
+  HostIo io;
+  if ((rc = upload(ctx, s, io)) || (rc = solve_checked_dev(ctx, io.d)) || (rc = download(ctx, io))) return rc;
+  CU(cudaStreamSynchronize(ctx->stream));
+  flush_staged(ctx, true);
+  return 0;
 }
 
 extern "C" int cfs_nearest_steer(cfs_ctx *ctx, int n_nodes, const double *nodes, int S, const double *samples,
