@@ -188,7 +188,12 @@ int cfs_chomp_batch(cfs_ctx *ctx, int B, const double *x0 /*2nj x B*/, const dou
                     double *u /*n x B*/, double *x /*2njH x B or NULL*/, double *cost_hist /*max_outer x B*/,
                     double *e_u_hist /*max_outer x B or NULL*/, int *iters /*B*/, int *status /*B*/);
 
-/* Blocks until the context's stream is idle and collects the statistics of the batch in flight (if any). */
+/* Blocks until the context's stream is idle and collects the statistics of the batch in flight (if any).  Every synchronous
+ * host-pointer entry (the host solve forms, cfs_resample_routes, cfs_chomp_batch, cfs_dist_grad, cfs_time_dist_grad,
+ * cfs_get_con, cfs_nodes_feasible, cfs_check_edges, cfs_check_trajectories, cfs_nearest_steer, cfs_rrt_find_routes) does the
+ * same before it enqueues work of its own: the batch's outputs are in the caller's buffers when that entry returns, and
+ * cfs_get_stats describes the batch (cfs_chomp_batch then reports its own ms_total and launches).  The _device forms do not
+ * wait for it. */
 int cfs_wait(cfs_ctx *ctx);
 /* Same, every pointer is a DEVICE pointer on ctx's device (inputs already resident in HBM); asynchronous on the
  * context stream unless sync != 0. */

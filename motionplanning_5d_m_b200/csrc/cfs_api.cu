@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -73,8 +74,9 @@ struct cfs_ctx {
   DevBuf th0, thg;
   // batch buffers
   DevBuf x0, ff, caug, xref, noise, u, x, cost, eu, u0, v0, cost0, dist, grad, lid, iters, status, flags, listA, listB,
-      counters, slab, scratch_theta, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen, rrt_in,
-      chk_in, chk_out, chk_seg, chk_ctr, rep_off, rep_offo, rep_in, rep_out, rep_list, zero_off;
+      counters, slab, scratch_out, qpsteps, fupper, probsteps, psg_w, psg_cost, psg_skip, routes, zslab, cont, rlen,
+      chk_out, chk_seg, chk_ctr, rep_off, rep_offo, rep_in, rep_out, rep_list, zero_off;
+  DevBuf area;  // the regions of the synchronous host-pointer entries (Area)
   int slab_grid = 0, slab_ld = 0;
   // pinned staging of the host-pointer entries: pageable caller buffers (MATLAB's mxGetPr memory, numpy arrays) are copied
   // through these so that cudaMemcpyAsync stays asynchronous; pinned / registered caller buffers are used in place
@@ -274,11 +276,11 @@ extern "C" void cfs_destroy(cfs_ctx *ctx) {
   cudaStreamSynchronize(ctx->stream);
   DevBuf *bufs[] = {&ctx->x0, &ctx->ff, &ctx->caug, &ctx->xref, &ctx->noise, &ctx->u, &ctx->x, &ctx->cost, &ctx->eu,
                     &ctx->u0, &ctx->v0, &ctx->cost0, &ctx->dist, &ctx->grad, &ctx->lid, &ctx->iters, &ctx->status,
-                    &ctx->flags, &ctx->listA, &ctx->listB, &ctx->counters, &ctx->slab, &ctx->scratch_theta,
+                    &ctx->flags, &ctx->listA, &ctx->listB, &ctx->counters, &ctx->slab,
                     &ctx->scratch_out, &ctx->qpsteps, &ctx->fupper, &ctx->probsteps, &ctx->routes, &ctx->psg_w, &ctx->psg_cost,
-                    &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen, &ctx->rrt_in,
-                    &ctx->chk_in, &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr, &ctx->rep_off, &ctx->rep_offo, &ctx->rep_in,
-                    &ctx->rep_out, &ctx->rep_list, &ctx->zero_off};
+                    &ctx->psg_skip, &ctx->th0, &ctx->thg, &ctx->zslab, &ctx->cont, &ctx->rlen,
+                    &ctx->chk_out, &ctx->chk_seg, &ctx->chk_ctr, &ctx->rep_off, &ctx->rep_offo, &ctx->rep_in,
+                    &ctx->rep_out, &ctx->rep_list, &ctx->zero_off, &ctx->area};
   for (DevBuf *b : bufs) free_buf(*b);
   if (ctx->dQblk) cudaFree(ctx->dQblk);
   if (ctx->dqlim) cudaFree(ctx->dqlim);
@@ -545,6 +547,18 @@ static int check_ready(cfs_ctx *ctx, bool need_cost) {
   if (!ctx->have_obs) return fail(ctx, CFS_E_STATE, "obstacles not set (cfs_set_obstacles)");
   if (need_cost && !ctx->have_cost) return fail(ctx, CFS_E_STATE, "cost not set (cfs_set_cost)");
   return 0;
+}
+
+// The distance/gradient kernel over B trajectories (x: 2n x B, H waypoints each): dist and flags per problem, [b][obstacle][i]
+static GradArgs traj_grad_args(const cfs_ctx *ctx, int B, const double *x, double *dist, double *grad, int *flags) {
+  GradArgs g;
+  memset(&g, 0, sizeof(g));
+  g.tab = ctx->dtab; g.dv = ctx->ddv;
+  g.x = x; g.ld_prob = 2 * ctx->n; g.ld_i = 2 * ctx->nj;
+  g.nslots = B; g.H = ctx->H; g.nj = ctx->nj; g.nobs = ctx->nobs;
+  g.o_prob = ctx->nobs * ctx->H; g.o_obs = ctx->H; g.o_i = 1;
+  g.dist = dist; g.grad = grad; g.flags = flags;
+  return g;
 }
 
 // ---- the solve, device pointers --------------------------------------------------------------------------------------
@@ -829,14 +843,7 @@ static int solve_device(cfs_ctx *ctx, int B, int solver, int grad, const double 
     CU(launch_v0(a, st)); ++launches;
   }
 
-  GradArgs g;
-  memset(&g, 0, sizeof(g));
-  g.tab = ctx->dtab; g.dv = ctx->ddv;
-  g.x = x; g.ld_prob = 2 * n; g.ld_i = 2 * nj;
-  g.nslots = B; g.H = H; g.nj = nj; g.nobs = O;
-  g.o_prob = OH; g.o_obs = H; g.o_i = 1;
-  g.dist = a.dist; g.linkid = nullptr; g.grad = a.grad; g.flags = a.flags;
-
+  GradArgs g = traj_grad_args(ctx, B, x, a.dist, a.grad, a.flags);
   for (int it = 1; it <= max_outer; ++it) {
     NvtxRange nvtx_it("cfs:outer iteration (gradient | QP)");
     a.outer_iter = it;
@@ -956,7 +963,7 @@ static void host_copy(void *dst, const void *src, size_t bytes) {
 
 // ---- the solve family: cfs_solve_batch*, cfs_solve_start_goal*, cfs_solve_routes*, cfs_solve_batch_margins*, cfs_solve_checked*
 // Every entry describes its call (SolveCall) and hands it to one validator (check_solve), one enqueue on device pointers
-// (enqueue_solve) and, for a host form, one transfer path (upload / download through the pinned staging area).
+// (enqueue_solve) and, for a host form, the transfer path (upload, then Transfer::d2h).
 enum SolveForm { FORM_ARRAYS, FORM_START_GOAL, FORM_ROUTES };
 
 // The problems of a call: the reference's per-problem arrays, or start/goal pairs or routes from which the device builds them
@@ -1103,6 +1110,118 @@ struct StageOut {
   }
 };
 
+namespace {  // internal linkage: none of this is part of the library's exported symbols
+
+// The one transfer path of every host-pointer entry: copies between caller buffers and device buffers.  With stage set (the
+// solve family), pageable caller buffers go through the context's pinned staging area (one memcpy each way) so that every copy
+// is truly asynchronous; pinned / registered buffers are used in place.  A NULL caller buffer is not copied.  Staged results
+// reach the caller's buffers in flush_staged, after the stream has synchronised.
+struct Transfer {
+  struct In { const void *host; void *dev; size_t bytes; };
+  struct Out { void *host; const void *dev; size_t bytes; };
+  std::vector<In> in;
+  std::vector<Out> out;
+  StageOut sout{nullptr, false};
+  // Off for the synchronous entries (Area): their call waits for its copies anyway, and the driver's own copy from pageable
+  // memory overlaps its staging memcpy with the DMA, where the staging area copies first and transfers after (measured on a
+  // B200: cfs_nodes_feasible, N = 100000, 0.49 ms staged against 0.43 ms direct)
+  bool stage = true;
+
+  // the staging decision of both directions, the staging area they take, and the H2D copies
+  int h2d(cfs_ctx *ctx) {
+    auto staged = [](const auto &copies, size_t &bytes) {  // -> some caller buffer is pageable; bytes: the staging area they take
+      bool pageable = false;
+      for (const auto &e : copies)
+        if (e.host && e.bytes) { bytes += (e.bytes + 255) / 256 * 256; pageable = pageable || !is_pinned_host(e.host); }
+      return pageable;
+    };
+    size_t in_bytes = 0, out_bytes = 0;
+    StageIn sin{ctx, stage && staged(in, in_bytes)};
+    sout = {ctx, stage && staged(out, out_bytes)};
+    int rc;
+    if (sin.use && (rc = ensure_stage(ctx, ctx->stage_in, ctx->stage_in_cap, in_bytes))) return rc;
+    if (sout.use && (rc = ensure_stage(ctx, ctx->stage_out, ctx->stage_out_cap, out_bytes))) return rc;
+    ctx->copy_back.clear();
+    for (cudaEvent_t &e : ctx->ev_h)
+      if (!e) CU(cudaEventCreate(&e));
+    CU(cudaEventRecord(ctx->ev_h[0], ctx->stream));
+    {
+      NvtxRange r("cfs:h2d");
+      for (const In &e : in) CU(sin.put(e.dev, e.host, e.bytes, ctx->stream));
+    }
+    CU(cudaEventRecord(ctx->ev_h[1], ctx->stream));
+    return 0;
+  }
+
+  int d2h(cfs_ctx *ctx) {
+    CU(cudaEventRecord(ctx->ev_h[2], ctx->stream));
+    {
+      NvtxRange r("cfs:d2h");
+      for (const Out &e : out) CU(sout.get(e.host, e.dev, e.bytes, ctx->stream));
+    }
+    CU(cudaEventRecord(ctx->ev_h[3], ctx->stream));
+    return 0;
+  }
+};
+
+// The device side of a synchronous host-pointer entry: regions of one context-owned buffer (ctx->area), each 256-byte aligned.
+// A region is uploaded from a caller's buffer (in), downloaded to one (out), both (inout), or neither (tmp: a device-only
+// temporary).  upload() completes the batch in flight first: its staged results wait in stage_out until then, and its
+// statistics in ev_a / ev_b.
+class Area {
+ public:
+  explicit Area(cfs_ctx *ctx) : ctx_(ctx) { io_.stage = false; }
+  template <class T> Area &in(T *&dev, const T *host, size_t count) { return add<T>(dev, count, host, nullptr); }
+  template <class T> Area &out(T *&dev, T *host, size_t count) { return add<T>(dev, count, nullptr, host); }
+  template <class T> Area &inout(T *&dev, const T *host_in, T *host_out, size_t count) { return add<T>(dev, count, host_in, host_out); }
+  template <class T> Area &tmp(T *&dev, size_t count) { return add<T>(dev, count, nullptr, nullptr); }
+
+  // the pending batch, the buffer, the region pointers and the H2D copies
+  int upload() {
+    cfs_ctx *ctx = ctx_;
+    int rc;
+    CU(cudaSetDevice(ctx->device));
+    if ((rc = finish_pending(ctx)) || (rc = ensure(ctx, ctx->area, bytes_))) return rc;
+    char *base = static_cast<char *>(ctx->area.p);
+    for (const Region &r : regions_) {
+      r.place(base + r.off);
+      if (r.in) io_.in.push_back({r.in, base + r.off, r.bytes});
+      if (r.out) io_.out.push_back({r.out, base + r.off, r.bytes});
+    }
+    return io_.h2d(ctx);
+  }
+
+  // the D2H copies, the synchronise and the staged results to the caller's buffers
+  int download() {
+    cfs_ctx *ctx = ctx_;
+    int rc;
+    if ((rc = io_.d2h(ctx))) return rc;
+    CU(cudaStreamSynchronize(ctx->stream));
+    flush_staged(ctx, false);
+    return 0;
+  }
+
+ private:
+  struct Region {
+    size_t off, bytes;
+    const void *in;
+    void *out;
+    std::function<void(char *)> place;
+  };
+  template <class T> Area &add(T *&dev, size_t count, const T *in, T *out) {
+    const size_t bytes = sizeof(T) * count;
+    regions_.push_back({bytes_, bytes, in, out, [&dev](char *p) { dev = reinterpret_cast<T *>(p); }});
+    bytes_ += (bytes + 255) / 256 * 256;
+    return *this;
+  }
+  cfs_ctx *ctx_;
+  std::vector<Region> regions_;
+  size_t bytes_ = 0;
+  Transfer io_;
+};
+
+}  // namespace
+
 static int check_traj_args(cfs_ctx *ctx, const char *who, int B, int H, double eta, int margin_is_D, int max_evals);
 
 // The argument checks of every solve entry, in this order: the context; robot, obstacles, cost and, for the start/goal and
@@ -1200,20 +1319,14 @@ static int enqueue_solve(cfs_ctx *ctx, const SolveCall &s) {
 }
 
 // A host form on the context's batch buffers: the call on device pointers (d, dc) and the copies between those buffers and the
-// caller's (a NULL caller buffer is not copied)
+// caller's
 struct HostIo {
-  struct In { const void *host; void *dev; size_t bytes; };
-  struct Out { void *host; const void *dev; size_t bytes; };
   SolveCall d;
   CheckedIo dc;
-  std::vector<In> in;
-  std::vector<Out> out;
-  StageOut sout{nullptr, false};
+  Transfer t;
 };
 
-// Host forms, before the enqueue: the batch buffers, the call on them and the H2D copies.  Pageable caller buffers go through
-// the context's pinned staging area (one memcpy each way) so that every copy is truly asynchronous; pinned / registered buffers
-// are used in place.
+// Host forms, before the enqueue: the batch buffers, the call on them and the H2D copies
 static int upload(cfs_ctx *ctx, const SolveCall &s, HostIo &io) {
   int rc;
   CU(cudaSetDevice(ctx->device));
@@ -1222,11 +1335,11 @@ static int upload(cfs_ctx *ctx, const SolveCall &s, HostIo &io) {
   const size_t B = s.B, nj = ctx->nj, n = ctx->n, K = s.max_outer, K1 = K > 0 ? K : 1, OH = (size_t)ctx->nobs * ctx->H;
   const size_t D = sizeof(double), I = sizeof(int);
   auto up = [&](auto h, DevBuf &b, size_t bytes) {  // -> the device copy of input h (NULL: none)
-    io.in.push_back({h, b.p, bytes});
+    io.t.in.push_back({h, b.p, bytes});
     return h ? static_cast<decltype(h)>(b.p) : nullptr;
   };
   auto down = [&](auto h, void *dev, size_t bytes) {  // -> where output h is computed
-    io.out.push_back({h, dev, bytes});
+    io.t.out.push_back({h, dev, bytes});
     return static_cast<decltype(h)>(dev);
   };
   const SolveIn &h = s.in;
@@ -1247,38 +1360,7 @@ static int upload(cfs_ctx *ctx, const SolveCall &s, HostIo &io) {
              down(c.rounds_used, v + B, I * B), c.margin_off && OH ? down(c.margin_off, ctx->rep_offo.p, D * OH * B) : nullptr};
     io.d.chk = &io.dc;
   }
-  auto staged = [](const auto &copies, size_t &bytes) {  // -> some caller buffer is pageable; bytes: the staging area they take
-    bool pageable = false;
-    for (const auto &e : copies)
-      if (e.host && e.bytes) { bytes += (e.bytes + 255) / 256 * 256; pageable = pageable || !is_pinned_host(e.host); }
-    return pageable;
-  };
-  size_t in_bytes = 0, out_bytes = 0;
-  StageIn sin{ctx, staged(io.in, in_bytes)};
-  io.sout = {ctx, staged(io.out, out_bytes)};
-  if (sin.use && (rc = ensure_stage(ctx, ctx->stage_in, ctx->stage_in_cap, in_bytes))) return rc;
-  if (io.sout.use && (rc = ensure_stage(ctx, ctx->stage_out, ctx->stage_out_cap, out_bytes))) return rc;
-  ctx->copy_back.clear();
-  for (cudaEvent_t &e : ctx->ev_h)
-    if (!e) CU(cudaEventCreate(&e));
-  CU(cudaEventRecord(ctx->ev_h[0], ctx->stream));
-  {
-    NvtxRange r("cfs:h2d");
-    for (const HostIo::In &e : io.in) CU(sin.put(e.dev, e.host, e.bytes, ctx->stream));
-  }
-  CU(cudaEventRecord(ctx->ev_h[1], ctx->stream));
-  return 0;
-}
-
-// Host forms, after the enqueue: the D2H copies (staged ones reach the caller's buffers in flush_staged)
-static int download(cfs_ctx *ctx, HostIo &io) {
-  CU(cudaEventRecord(ctx->ev_h[2], ctx->stream));
-  {
-    NvtxRange r("cfs:d2h");
-    for (const HostIo::Out &e : io.out) CU(io.sout.get(e.host, e.dev, e.bytes, ctx->stream));
-  }
-  CU(cudaEventRecord(ctx->ev_h[3], ctx->stream));
-  return 0;
+  return io.t.h2d(ctx);
 }
 
 // Every entry but the checked solve's: a host form through the staging area, a device form on the caller's pointers;
@@ -1291,7 +1373,7 @@ static int solve(cfs_ctx *ctx, const SolveCall &s, bool wait) {
     CU(cudaSetDevice(ctx->device));
     set_pending(ctx);  // statistics of an un-waited earlier batch are dropped
     if ((rc = ensure_batch(ctx, s)) || (rc = enqueue_solve(ctx, s))) return rc;
-  } else if ((rc = upload(ctx, s, io)) || (rc = enqueue_solve(ctx, io.d)) || (rc = download(ctx, io))) {
+  } else if ((rc = upload(ctx, s, io)) || (rc = enqueue_solve(ctx, io.d)) || (rc = io.t.d2h(ctx))) {
     return rc;
   }
   set_pending(ctx, s.device ? &s : &io.d, !s.device);
@@ -1393,25 +1475,21 @@ extern "C" int cfs_resample_routes(cfs_ctx *ctx, int B, int W, int H, const doub
   if (rc) return rc;
   if (B < 0 || W < 2 || H < 1 || (B > 0 && (!routes || !sampled))) return fail(ctx, CFS_E_ARG, "cfs_resample_routes: bad argument");
   if (B == 0) return 0;
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj;
+  const size_t nj = ctx->nj;
   cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->routes, sizeof(double) * (size_t)nj * W * B))) return rc;
-  if ((rc = ensure(ctx, ctx->th0, sizeof(double) * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->thg, sizeof(double) * nj * B))) return rc;
-  if ((rc = ensure(ctx, ctx->scratch_out, sizeof(double) * (size_t)2 * nj * H * B))) return rc;
-  CU(cudaMemcpyAsync(ctx->routes.p, routes, sizeof(double) * (size_t)nj * W * B, cudaMemcpyHostToDevice, st));
-  CU(launch_resample_routes(B, W, H, nj, ctx->htab.dt, ptr<double>(ctx->routes), nullptr, ptr<double>(ctx->th0),
-                            ptr<double>(ctx->thg), ptr<double>(ctx->scratch_out), st));
-  // sampled (nj x (H+1) x B): column 0 = theta0, columns 1..H = the theta rows of x_
-  CU(cudaMemcpy2DAsync(sampled, sizeof(double) * nj * (H + 1), ctx->th0.p, sizeof(double) * nj, sizeof(double) * nj, B,
+  double *d_routes, *th0, *thg, *xs;
+  Area ar(ctx);
+  ar.in(d_routes, routes, nj * W * B).tmp(th0, nj * B).tmp(thg, nj * B).tmp(xs, 2 * nj * H * B);
+  if ((rc = ar.upload())) return rc;
+  CU(launch_resample_routes(B, W, H, nj, ctx->htab.dt, d_routes, nullptr, th0, thg, xs, st));
+  // the one strided output, gathered straight into the caller's buffer: sampled (nj x (H+1) x B), column 0 = theta0,
+  // columns 1..H = the theta rows of x_
+  CU(cudaMemcpy2DAsync(sampled, sizeof(double) * nj * (H + 1), th0, sizeof(double) * nj, sizeof(double) * nj, B,
                        cudaMemcpyDeviceToHost, st));
   for (int i = 0; i < H; ++i)
-    CU(cudaMemcpy2DAsync(sampled + (size_t)nj * (i + 1), sizeof(double) * nj * (H + 1),
-                         ptr<double>(ctx->scratch_out) + (size_t)2 * nj * i, sizeof(double) * 2 * nj * H, sizeof(double) * nj, B,
-                         cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
+    CU(cudaMemcpy2DAsync(sampled + nj * (i + 1), sizeof(double) * nj * (H + 1), xs + 2 * nj * i, sizeof(double) * 2 * nj * H,
+                         sizeof(double) * nj, B, cudaMemcpyDeviceToHost, st));
+  return ar.download();
 }
 
 // ---- CHOMP_FANUC (Lib/CHOMP_FANUC.m), k_chomp.cu ----------------------------------------------------------------------
@@ -1425,62 +1503,42 @@ extern "C" int cfs_chomp_batch(cfs_ctx *ctx, int B, const double *x0, const doub
   if (B == 0) return 0;
   if (!x0 || !ff || !caug || !xref || !u_init || !u || !cost_hist || !iters || !status)
     return fail(ctx, CFS_E_ARG, "cfs_chomp_batch: NULL buffer");
-  if ((rc = finish_pending(ctx))) return rc;
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj, H = ctx->H, n = ctx->n, N = 2 * n, O = ctx->nobs, OH = O * H, K = max_outer;
+  const size_t nj = ctx->nj, n = ctx->n, K = max_outer, OH = (size_t)ctx->nobs * ctx->H;
   cudaStream_t st = ctx->stream;
   NvtxRange nvtx("cfs:chomp");
-  // one device buffer: x0 | ff | caug | u | x | w | cost | e_u | dist | grad | linkdist | flags
-  size_t o_x0 = 0, o_ff = o_x0 + (size_t)2 * nj * B, o_caug = o_ff + (size_t)n * B, o_u = o_caug + B, o_x = o_u + (size_t)n * B,
-         o_w = o_x + (size_t)N * B, o_cost = o_w + (size_t)n * B, o_eu = o_cost + (size_t)K * B + 1,
-         o_dist = o_eu + (size_t)K * B + 1, o_grad = o_dist + (size_t)OH * B + 1, o_ld = o_grad + (size_t)OH * B * nj + 1,
-         o_fl = o_ld + (size_t)OH * B * nj + 1, total = o_fl + (size_t)(B + 1) / 2 + 1;
-  if ((rc = ensure(ctx, ctx->scratch_out, sizeof(double) * total))) return rc;
-  double *d = ptr<double>(ctx->scratch_out);
-  int *d_flags = reinterpret_cast<int *>(d + o_fl);
-  CU(cudaMemcpyAsync(d + o_x0, x0, sizeof(double) * (size_t)2 * nj * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_ff, ff, sizeof(double) * (size_t)n * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_caug, caug, sizeof(double) * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_u, u_init, sizeof(double) * (size_t)n * B, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_x, xref, sizeof(double) * (size_t)N * B, cudaMemcpyHostToDevice, st));
+  double *d_x0, *d_ff, *d_caug, *d_u, *d_x, *d_w, *d_cost, *d_eu, *d_dist, *d_grad, *d_ld;
+  int *d_flags;
+  std::vector<int> fl(B);
+  Area ar(ctx);
+  ar.in(d_x0, x0, 2 * nj * B).in(d_ff, ff, n * B).in(d_caug, caug, B).inout(d_u, u_init, u, n * B).inout(d_x, xref, x, 2 * n * B)
+      .tmp(d_w, n * B).out(d_cost, cost_hist, K * B).out(d_eu, e_u_hist, K * B).tmp(d_dist, OH * B).tmp(d_grad, OH * nj * B)
+      .tmp(d_ld, OH * nj * B).out(d_flags, fl.data(), B);
+  if ((rc = ar.upload())) return rc;
   CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * B, st));
-  GradArgs g;
-  memset(&g, 0, sizeof(g));
-  g.tab = ctx->dtab; g.dv = ctx->ddv;
-  g.x = d + o_x; g.ld_prob = N; g.ld_i = 2 * nj;
-  g.nslots = B; g.H = H; g.nj = nj; g.nobs = O;
-  g.o_prob = OH; g.o_obs = H; g.o_i = 1;
-  g.dist = d + o_dist; g.grad = d + o_grad; g.linkdist = d + o_ld; g.flags = d_flags;
+  GradArgs g = traj_grad_args(ctx, B, d_x, d_dist, d_grad, d_flags);
+  g.linkdist = d_ld;
   g.no_off = 1;
   ChompArgs a;
   memset(&a, 0, sizeof(a));
-  a.B = B; a.n = n; a.nj = nj; a.H = H; a.nobs = O; a.max_outer = K; a.alpha = alpha; a.tab = ctx->dtab;
-  a.x0 = d + o_x0; a.ff = d + o_ff; a.caug = d + o_caug; a.u = d + o_u; a.x = d + o_x; a.w = d + o_w;
-  a.dist = g.dist; a.grad = g.grad; a.linkdist = g.linkdist;
-  a.cost_hist = d + o_cost; a.e_u_hist = d + o_eu;
+  a.B = B; a.n = n; a.nj = nj; a.H = ctx->H; a.nobs = ctx->nobs; a.max_outer = K; a.alpha = alpha; a.tab = ctx->dtab;
+  a.x0 = d_x0; a.ff = d_ff; a.caug = d_caug; a.u = d_u; a.x = d_x; a.w = d_w;
+  a.dist = d_dist; a.grad = d_grad; a.linkdist = d_ld;
+  a.cost_hist = d_cost; a.e_u_hist = d_eu;
   int launches = 0;
   CU(cudaEventRecord(ctx->ev_a, st));
-  if (O > 0) { CU(launch_grad_derivest(g, st)); ++launches; }
-  CU(launch_dgemm(n, B, n, 1.0, ctx->dQQraw, n, false, a.u, n, d + o_w, n, st)); ++launches;
-  for (int it = 1; it <= K; ++it) {
+  if (ctx->nobs > 0) { CU(launch_grad_derivest(g, st)); ++launches; }
+  CU(launch_dgemm(n, B, n, 1.0, ctx->dQQraw, n, false, d_u, n, d_w, n, st)); ++launches;
+  for (int it = 1; it <= max_outer; ++it) {
     a.it = it;
     CU(launch_chomp_step(a, st)); ++launches;
-    if (O > 0) { CU(launch_grad_derivest(g, st)); ++launches; }
-    CU(launch_dgemm(n, B, n, 1.0, ctx->dQQraw, n, false, a.u, n, d + o_w, n, st)); ++launches;
+    if (ctx->nobs > 0) { CU(launch_grad_derivest(g, st)); ++launches; }
+    CU(launch_dgemm(n, B, n, 1.0, ctx->dQQraw, n, false, d_u, n, d_w, n, st)); ++launches;
     CU(launch_chomp_cost(a, st)); ++launches;
   }
   CU(cudaEventRecord(ctx->ev_b, st));
-  CU(cudaMemcpyAsync(u, d + o_u, sizeof(double) * (size_t)n * B, cudaMemcpyDeviceToHost, st));
-  if (x) CU(cudaMemcpyAsync(x, d + o_x, sizeof(double) * (size_t)N * B, cudaMemcpyDeviceToHost, st));
-  if (K > 0) {
-    CU(cudaMemcpyAsync(cost_hist, d + o_cost, sizeof(double) * (size_t)K * B, cudaMemcpyDeviceToHost, st));
-    if (e_u_hist) CU(cudaMemcpyAsync(e_u_hist, d + o_eu, sizeof(double) * (size_t)K * B, cudaMemcpyDeviceToHost, st));
-  }
-  std::vector<int> fl(B);
-  CU(cudaMemcpyAsync(fl.data(), d_flags, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
+  if ((rc = ar.download())) return rc;
   for (int b = 0; b < B; ++b) {
-    iters[b] = K;
+    iters[b] = max_outer;
     status[b] = CFS_STATUS_MAX_ITER | (fl[b] & 0x100);  // stop_outer only ends at iter_O > MAX_O_ITER (CHOMP_FANUC.m:56)
   }
   float ms = 0;
@@ -1505,6 +1563,26 @@ extern "C" int cfs_dev_timeline(cfs_ctx *ctx, cfs_ctx *ref, double *out4) {
 }
 
 // ---- direct kernels -------------------------------------------------------------------------------------------------
+// cfs_dist_grad and cfs_time_dist_grad: theta uploaded, and the distance/gradient kernel with one "problem" per configuration so
+// that flags are per configuration: dist (n_obs x N) is dist[j + O * prob].  NULL outputs are computed and not copied back.
+static int config_grad(cfs_ctx *ctx, Area &ar, int N, const double *theta, double *dist, int *linkid, double *grad, int *flags,
+                       GradArgs &g) {
+  const size_t nj = ctx->nj, O = ctx->nobs;
+  double *d_theta, *d_dist, *d_grad;
+  int *d_lid, *d_flags;
+  ar.in(d_theta, theta, nj * N).out(d_dist, dist, O * N).out(d_grad, grad, O * N * nj).out(d_lid, linkid, O * N).out(d_flags, flags, N);
+  int rc = ar.upload();
+  if (rc) return rc;
+  CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * N, ctx->stream));
+  memset(&g, 0, sizeof(g));
+  g.tab = ctx->dtab; g.dv = ctx->ddv;
+  g.x = d_theta;
+  g.ld_prob = nj; g.ld_i = 0; g.nslots = N; g.H = 1; g.nj = nj; g.nobs = O;
+  g.o_prob = O; g.o_obs = 1; g.o_i = 0;
+  g.dist = d_dist; g.linkid = d_lid; g.grad = d_grad; g.flags = d_flags;
+  return 0;
+}
+
 extern "C" int cfs_dist_grad(cfs_ctx *ctx, int N, int grad_mode, const double *theta, double *dist, int *linkid,
                              double *grad, int *flags) {
   if (!ctx) return CFS_E_ARG;
@@ -1512,33 +1590,11 @@ extern "C" int cfs_dist_grad(cfs_ctx *ctx, int N, int grad_mode, const double *t
   if (rc) return rc;
   if (N < 0 || (N > 0 && (!theta || !dist || !grad))) return fail(ctx, CFS_E_ARG, "cfs_dist_grad: bad argument");
   if (N == 0 || ctx->nobs == 0) return 0;
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj, O = ctx->nobs;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->scratch_theta, sizeof(double) * (size_t)nj * N))) return rc;
-  const size_t bytes_out = (sizeof(double) * (1 + nj) + sizeof(int)) * (size_t)O * N + sizeof(int) * (size_t)N + 64;
-  if ((rc = ensure(ctx, ctx->scratch_out, bytes_out))) return rc;
-  double *d_dist = ptr<double>(ctx->scratch_out);
-  double *d_grad = d_dist + (size_t)O * N;
-  int *d_lid = reinterpret_cast<int *>(d_grad + (size_t)O * N * nj);
-  int *d_flags = d_lid + (size_t)O * N;
-  CU(cudaMemcpyAsync(ctx->scratch_theta.p, theta, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
-  CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * N, st));
+  Area ar(ctx);
   GradArgs g;
-  memset(&g, 0, sizeof(g));
-  g.tab = ctx->dtab; g.dv = ctx->ddv;
-  g.x = ptr<double>(ctx->scratch_theta);
-  // one "problem" per configuration so that flags are per configuration: prob = i
-  g.ld_prob = nj; g.ld_i = 0; g.nslots = N; g.H = 1; g.nj = nj; g.nobs = O;
-  g.o_prob = O; g.o_obs = 1; g.o_i = 0;  // dist (n_obs x N): dist[j + O*prob]
-  g.dist = d_dist; g.linkid = d_lid; g.grad = d_grad; g.flags = d_flags;
-  CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, st) : launch_grad_numjac(g, st));
-  CU(cudaMemcpyAsync(dist, d_dist, sizeof(double) * (size_t)O * N, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(grad, d_grad, sizeof(double) * (size_t)O * N * nj, cudaMemcpyDeviceToHost, st));
-  if (linkid) CU(cudaMemcpyAsync(linkid, d_lid, sizeof(int) * (size_t)O * N, cudaMemcpyDeviceToHost, st));
-  if (flags) CU(cudaMemcpyAsync(flags, d_flags, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
+  if ((rc = config_grad(ctx, ar, N, theta, dist, linkid, grad, flags, g))) return rc;
+  CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, ctx->stream) : launch_grad_numjac(g, ctx->stream));
+  return ar.download();
 }
 
 extern "C" int cfs_time_dist_grad(cfs_ctx *ctx, int N, int grad_mode, const double *theta, int reps, double *ms_per_launch) {
@@ -1546,34 +1602,39 @@ extern "C" int cfs_time_dist_grad(cfs_ctx *ctx, int N, int grad_mode, const doub
   int rc = check_ready(ctx, false);
   if (rc) return rc;
   if (ctx->nobs == 0) return fail(ctx, CFS_E_STATE, "cfs_time_dist_grad: no obstacles");
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj, O = ctx->nobs;
   cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->scratch_theta, sizeof(double) * (size_t)nj * N))) return rc;
-  const size_t bytes_out = (sizeof(double) * (1 + nj) + sizeof(int)) * (size_t)O * N + sizeof(int) * (size_t)N + 64;
-  if ((rc = ensure(ctx, ctx->scratch_out, bytes_out))) return rc;
-  double *d_dist = ptr<double>(ctx->scratch_out);
-  double *d_grad = d_dist + (size_t)O * N;
-  int *d_lid = reinterpret_cast<int *>(d_grad + (size_t)O * N * nj);
-  int *d_flags = d_lid + (size_t)O * N;
-  CU(cudaMemcpyAsync(ctx->scratch_theta.p, theta, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
-  CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * N, st));
+  Area ar(ctx);
   GradArgs g;
-  memset(&g, 0, sizeof(g));
-  g.tab = ctx->dtab; g.dv = ctx->ddv;
-  g.x = ptr<double>(ctx->scratch_theta);
-  g.ld_prob = nj; g.ld_i = 0; g.nslots = N; g.H = 1; g.nj = nj; g.nobs = O;
-  g.o_prob = O; g.o_obs = 1; g.o_i = 0;
-  g.dist = d_dist; g.linkid = d_lid; g.grad = d_grad; g.flags = d_flags;
+  if ((rc = config_grad(ctx, ar, N, theta, nullptr, nullptr, nullptr, nullptr, g))) return rc;
   for (int w = 0; w < 2; ++w) CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, st) : launch_grad_numjac(g, st));
   CU(cudaEventRecord(ctx->ev_a, st));
   for (int r = 0; r < reps; ++r) CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, st) : launch_grad_numjac(g, st));
   CU(cudaEventRecord(ctx->ev_b, st));
-  CU(cudaStreamSynchronize(st));
+  if ((rc = ar.download())) return rc;
   float ms = 0;
   cudaEventElapsedTime(&ms, ctx->ev_a, ctx->ev_b);
   *ms_per_launch = ms / reps;
   return 0;
+}
+
+// The reference's rows of CFS_FANUC.get_con for one problem, computed on the device: A (m x n, column-major) and b (m)
+static int con_rows(cfs_ctx *ctx, int grad_mode, int margin_is_D, const double *x0, const double *xcur, const double *u, int m,
+                    double *A, double *b) {
+  const size_t nj = ctx->nj, n = ctx->n, OH = (size_t)ctx->nobs * ctx->H;
+  cudaStream_t st = ctx->stream;
+  double *d_x0, *d_x, *d_u, *d_dist, *d_grad, *d_A, *d_b;
+  int *d_flags;
+  Area ar(ctx);
+  ar.in(d_x0, x0, 2 * nj).in(d_x, xcur, 2 * n).in(d_u, u, n).tmp(d_dist, OH).tmp(d_grad, OH * nj).out(d_A, A, m * n)
+      .out(d_b, b, m).tmp(d_flags, 1);
+  int rc = ar.upload();
+  if (rc) return rc;
+  CU(cudaMemsetAsync(d_flags, 0, sizeof(int), st));
+  const GradArgs g = traj_grad_args(ctx, 1, d_x, d_dist, d_grad, d_flags);
+  CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, st) : launch_grad_numjac(g, st));
+  CU(launch_get_con_rows(ctx->dtab, ctx->H, nj, ctx->nobs, ctx->has_lim, margin_is_D, d_x0, d_u, ctx->dlim, d_dist, d_grad, d_A,
+                         d_b, m, st));
+  return ar.download();
 }
 
 extern "C" int cfs_get_con(cfs_ctx *ctx, int grad_mode, int margin_is_D, const double *x0, const double *xcur,
@@ -1582,64 +1643,31 @@ extern "C" int cfs_get_con(cfs_ctx *ctx, int grad_mode, int margin_is_D, const d
   int rc = check_ready(ctx, true);
   if (rc) return rc;
   if (!x0 || !xcur || !u || !Ainq || !binq) return fail(ctx, CFS_E_ARG, "cfs_get_con: NULL argument");
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj, H = ctx->H, n = ctx->n, O = ctx->nobs, OH = O * H;
-  const int m = OH * (ctx->has_lim ? 1 + 2 * nj : 1);
-  if (ctx->has_qlim) {  // joint position rows after the reference's rows: theta_(i+1),k <= qmax_k, then -theta_(i+1),k <= -qmin_k
-    const int mt = m + 2 * n;
-    std::vector<double> A0((size_t)m * n), b0(m);
-    if (m > 0) {
-      ctx->has_qlim = false;
-      rc = cfs_get_con(ctx, grad_mode, margin_is_D, x0, xcur, u, A0.data(), b0.data());
-      ctx->has_qlim = true;
-      if (rc) return rc;
-    }
-    const double dt = ctx->htab.dt;
-    for (int c = 0; c < n; ++c) {
-      for (int r = 0; r < m; ++r) Ainq[r + (size_t)mt * c] = A0[r + (size_t)m * c];
-      const int jj = c / nj, kc = c - jj * nj;
-      for (int e = 0; e < n; ++e) {
-        const int i = e / nj, k = e - i * nj;
-        const double v = (k == kc && jj <= i) ? (0.5 * dt * dt + ((i - jj) * dt) * dt) : 0.0;
-        Ainq[m + e + (size_t)mt * c] = v;
-        Ainq[m + n + e + (size_t)mt * c] = -v;
-      }
-    }
-    for (int r = 0; r < m; ++r) binq[r] = b0[r];
+  const int nj = ctx->nj, n = ctx->n;
+  const int m = ctx->nobs * ctx->H * (ctx->has_lim ? 1 + 2 * nj : 1);
+  if (!ctx->has_qlim) return m > 0 ? con_rows(ctx, grad_mode, margin_is_D, x0, xcur, u, m, Ainq, binq) : 0;
+  // joint position rows after the reference's rows: theta_(i+1),k <= qmax_k, then -theta_(i+1),k <= -qmin_k
+  const int mt = m + 2 * n;
+  std::vector<double> A0((size_t)m * n), b0(m);
+  if (m > 0 && (rc = con_rows(ctx, grad_mode, margin_is_D, x0, xcur, u, m, A0.data(), b0.data()))) return rc;
+  const double dt = ctx->htab.dt;
+  for (int c = 0; c < n; ++c) {
+    for (int r = 0; r < m; ++r) Ainq[r + (size_t)mt * c] = A0[r + (size_t)m * c];
+    const int jj = c / nj, kc = c - jj * nj;
     for (int e = 0; e < n; ++e) {
       const int i = e / nj, k = e - i * nj;
-      const double fm = x0[k] + ((i + 1) * dt) * x0[nj + k];
-      binq[m + e] = ctx->hqlim[k] - fm;
-      binq[m + n + e] = fm - ctx->hqlim[nj + k];
+      const double v = (k == kc && jj <= i) ? (0.5 * dt * dt + ((i - jj) * dt) * dt) : 0.0;
+      Ainq[m + e + (size_t)mt * c] = v;
+      Ainq[m + n + e + (size_t)mt * c] = -v;
     }
-    return 0;
   }
-  if (m == 0) return 0;
-  cudaStream_t st = ctx->stream;
-  const size_t in_d = (size_t)2 * nj + 2 * n + n;
-  if ((rc = ensure(ctx, ctx->scratch_theta, sizeof(double) * in_d))) return rc;
-  const size_t out_d = (size_t)OH + (size_t)OH * nj + (size_t)m * n + m;
-  if ((rc = ensure(ctx, ctx->scratch_out, sizeof(double) * out_d + sizeof(int) * 4))) return rc;
-  double *d_x0 = ptr<double>(ctx->scratch_theta), *d_x = d_x0 + 2 * nj, *d_u = d_x + 2 * n;
-  double *d_dist = ptr<double>(ctx->scratch_out), *d_grad = d_dist + OH, *d_A = d_grad + (size_t)OH * nj,
-         *d_b = d_A + (size_t)m * n;
-  int *d_flags = reinterpret_cast<int *>(d_b + m);
-  CU(cudaMemcpyAsync(d_x0, x0, sizeof(double) * 2 * nj, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_x, xcur, sizeof(double) * 2 * n, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_u, u, sizeof(double) * n, cudaMemcpyHostToDevice, st));
-  CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * 4, st));
-  GradArgs g;
-  memset(&g, 0, sizeof(g));
-  g.tab = ctx->dtab; g.dv = ctx->ddv;
-  g.x = d_x; g.ld_prob = 2 * n; g.ld_i = 2 * nj; g.nslots = 1; g.H = H; g.nj = nj; g.nobs = O;
-  g.o_prob = OH; g.o_obs = H; g.o_i = 1;
-  g.dist = d_dist; g.linkid = nullptr; g.grad = d_grad; g.flags = d_flags;
-  CU(grad_mode == CFS_GRAD_DERIVEST ? launch_grad_derivest(g, st) : launch_grad_numjac(g, st));
-  CU(launch_get_con_rows(ctx->dtab, H, nj, O, ctx->has_lim, margin_is_D, d_x0, d_u, ctx->dlim, d_dist, d_grad, d_A, d_b,
-                         m, st));
-  CU(cudaMemcpyAsync(Ainq, d_A, sizeof(double) * (size_t)m * n, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(binq, d_b, sizeof(double) * m, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
+  for (int r = 0; r < m; ++r) binq[r] = b0[r];
+  for (int e = 0; e < n; ++e) {
+    const int i = e / nj, k = e - i * nj;
+    const double fm = x0[k] + ((i + 1) * dt) * x0[nj + k];
+    binq[m + e] = ctx->hqlim[k] - fm;
+    binq[m + n + e] = fm - ctx->hqlim[nj + k];
+  }
   return 0;
 }
 
@@ -1649,19 +1677,14 @@ extern "C" int cfs_nodes_feasible(cfs_ctx *ctx, int N, const double *theta, unsi
   if (rc) return rc;
   if (N < 0 || (N > 0 && (!theta || !feasible))) return fail(ctx, CFS_E_ARG, "cfs_nodes_feasible: bad argument");
   if (N == 0) return 0;
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->scratch_theta, sizeof(double) * (size_t)nj * N))) return rc;
-  if ((rc = ensure(ctx, ctx->scratch_out, (sizeof(double) + 1) * (size_t)N + 64))) return rc;
-  double *d_dmin = ptr<double>(ctx->scratch_out);
-  unsigned char *d_feas = reinterpret_cast<unsigned char *>(d_dmin + N);
-  CU(cudaMemcpyAsync(ctx->scratch_theta.p, theta, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
-  CU(launch_nodes_feasible(ctx->dtab, nj, ctx->nobs, N, ptr<double>(ctx->scratch_theta), d_feas, d_dmin, st));
-  CU(cudaMemcpyAsync(feasible, d_feas, (size_t)N, cudaMemcpyDeviceToHost, st));
-  if (dmin) CU(cudaMemcpyAsync(dmin, d_dmin, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
+  const size_t nj = ctx->nj;
+  double *d_theta, *d_dmin;
+  unsigned char *d_feas;
+  Area ar(ctx);
+  ar.in(d_theta, theta, nj * N).out(d_feas, feasible, N).out(d_dmin, dmin, N);
+  if ((rc = ar.upload())) return rc;
+  CU(launch_nodes_feasible(ctx->dtab, nj, ctx->nobs, N, d_theta, d_feas, d_dmin, ctx->stream));
+  return ar.download();
 }
 
 // ---- continuous collision checks (k_check.cu) ------------------------------------------------------------------------
@@ -1719,13 +1742,20 @@ static int check_traj_dev(cfs_ctx *ctx, int B, int H, const double *x0, const do
   return 0;
 }
 
+// The argument checks of cfs_check_edges and its device form: check_check_args, then (N > 0) the required buffers
+static int check_edges_call(cfs_ctx *ctx, const char *who, int N, const void *theta_a, const void *theta_b, double eta,
+                            int margin_is_D, int max_evals, const void *verdict, const void *s_hit, const void *cmin) {
+  int rc = check_check_args(ctx, who, N, eta, margin_is_D, max_evals);
+  if (rc || N == 0) return rc;
+  if (!theta_a || !theta_b || !verdict || !s_hit || !cmin) return fail(ctx, CFS_E_ARG, "%s: NULL buffer", who);
+  return 0;
+}
+
 extern "C" int cfs_check_edges_device(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta,
                                       int margin_is_D, int max_evals, int *verdict, double *s_hit, double *cmin, int *evals,
                                       int sync) {
-  int rc = check_check_args(ctx, "cfs_check_edges", N, eta, margin_is_D, max_evals);
-  if (rc) return rc;
-  if (N == 0) return 0;
-  if (!theta_a || !theta_b || !verdict || !s_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_edges_device: NULL buffer");
+  int rc = check_edges_call(ctx, "cfs_check_edges_device", N, theta_a, theta_b, eta, margin_is_D, max_evals, verdict, s_hit, cmin);
+  if (rc || N == 0) return rc;
   CU(cudaSetDevice(ctx->device));
   if ((rc = check_edges_dev(ctx, N, theta_a, theta_b, eta, margin_is_D, max_evals, verdict, s_hit, cmin, evals))) return rc;
   if (sync) CU(cudaStreamSynchronize(ctx->stream));
@@ -1734,27 +1764,15 @@ extern "C" int cfs_check_edges_device(cfs_ctx *ctx, int N, const double *theta_a
 
 extern "C" int cfs_check_edges(cfs_ctx *ctx, int N, const double *theta_a, const double *theta_b, double eta, int margin_is_D,
                                int max_evals, int *verdict, double *s_hit, double *cmin, int *evals) {
-  int rc = check_check_args(ctx, "cfs_check_edges", N, eta, margin_is_D, max_evals);
-  if (rc) return rc;
-  if (N == 0) return 0;
-  if (!theta_a || !theta_b || !verdict || !s_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_edges: NULL buffer");
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->chk_in, sizeof(double) * 2 * (size_t)nj * N))) return rc;
-  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)N + 64))) return rc;
-  double *d_a = ptr<double>(ctx->chk_in), *d_b = d_a + (size_t)nj * N;
-  double *d_s = ptr<double>(ctx->chk_out), *d_c = d_s + N;
-  int *d_v = reinterpret_cast<int *>(d_c + N), *d_e = d_v + N;
-  CU(cudaMemcpyAsync(d_a, theta_a, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_b, theta_b, sizeof(double) * (size_t)nj * N, cudaMemcpyHostToDevice, st));
-  if ((rc = check_edges_dev(ctx, N, d_a, d_b, eta, margin_is_D, max_evals, d_v, d_s, d_c, d_e))) return rc;
-  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(s_hit, d_s, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  if (evals) CU(cudaMemcpyAsync(evals, d_e, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
+  int rc = check_edges_call(ctx, "cfs_check_edges", N, theta_a, theta_b, eta, margin_is_D, max_evals, verdict, s_hit, cmin);
+  if (rc || N == 0) return rc;
+  const size_t nj = ctx->nj;
+  double *d_a, *d_b, *d_s, *d_c;
+  int *d_v, *d_e;
+  Area ar(ctx);
+  ar.in(d_a, theta_a, nj * N).in(d_b, theta_b, nj * N).out(d_v, verdict, N).out(d_s, s_hit, N).out(d_c, cmin, N).out(d_e, evals, N);
+  if ((rc = ar.upload()) || (rc = check_edges_dev(ctx, N, d_a, d_b, eta, margin_is_D, max_evals, d_v, d_s, d_c, d_e))) return rc;
+  return ar.download();
 }
 
 static int check_traj_args(cfs_ctx *ctx, const char *who, int B, int H, double eta, int margin_is_D, int max_evals) {
@@ -1765,13 +1783,20 @@ static int check_traj_args(cfs_ctx *ctx, const char *who, int B, int H, double e
   return 0;
 }
 
+// The argument checks of cfs_check_trajectories and its device form: check_traj_args, then (B > 0) the required buffers
+static int check_traj_call(cfs_ctx *ctx, const char *who, int B, int H, const void *x0, const void *x, const void *u, double eta,
+                           int margin_is_D, int max_evals, const void *verdict, const void *t_hit, const void *cmin) {
+  int rc = check_traj_args(ctx, who, B, H, eta, margin_is_D, max_evals);
+  if (rc || B == 0) return rc;
+  if (!x0 || !x || !u || !verdict || !t_hit || !cmin) return fail(ctx, CFS_E_ARG, "%s: NULL buffer", who);
+  return 0;
+}
+
 extern "C" int cfs_check_trajectories_device(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u,
                                              double eta, int margin_is_D, int max_evals, int *verdict, double *t_hit,
                                              double *cmin, int *evals, int sync) {
-  int rc = check_traj_args(ctx, "cfs_check_trajectories", B, H, eta, margin_is_D, max_evals);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  if (!x0 || !x || !u || !verdict || !t_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_trajectories_device: NULL buffer");
+  int rc = check_traj_call(ctx, "cfs_check_trajectories_device", B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin);
+  if (rc || B == 0) return rc;
   CU(cudaSetDevice(ctx->device));
   if ((rc = check_traj_dev(ctx, B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin, evals))) return rc;
   if (sync) CU(cudaStreamSynchronize(ctx->stream));
@@ -1780,28 +1805,17 @@ extern "C" int cfs_check_trajectories_device(cfs_ctx *ctx, int B, int H, const d
 
 extern "C" int cfs_check_trajectories(cfs_ctx *ctx, int B, int H, const double *x0, const double *x, const double *u, double eta,
                                       int margin_is_D, int max_evals, int *verdict, double *t_hit, double *cmin, int *evals) {
-  int rc = check_traj_args(ctx, "cfs_check_trajectories", B, H, eta, margin_is_D, max_evals);
-  if (rc) return rc;
-  if (B == 0) return 0;
-  if (!x0 || !x || !u || !verdict || !t_hit || !cmin) return fail(ctx, CFS_E_ARG, "cfs_check_trajectories: NULL buffer");
-  CU(cudaSetDevice(ctx->device));
-  const size_t nj = ctx->nj, nx0 = 2 * nj * B, nx = 2 * nj * H * B, nu = nj * H * B;
-  cudaStream_t st = ctx->stream;
-  if ((rc = ensure(ctx, ctx->chk_in, sizeof(double) * (nx0 + nx + nu)))) return rc;
-  if ((rc = ensure(ctx, ctx->chk_out, (2 * sizeof(double) + 2 * sizeof(int)) * (size_t)B + 64))) return rc;
-  double *d_x0 = ptr<double>(ctx->chk_in), *d_x = d_x0 + nx0, *d_u = d_x + nx;
-  double *d_t = ptr<double>(ctx->chk_out), *d_c = d_t + B;
-  int *d_v = reinterpret_cast<int *>(d_c + B), *d_e = d_v + B;
-  CU(cudaMemcpyAsync(d_x0, x0, sizeof(double) * nx0, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_x, x, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_u, u, sizeof(double) * nu, cudaMemcpyHostToDevice, st));
-  if ((rc = check_traj_dev(ctx, B, H, d_x0, d_x, d_u, eta, margin_is_D, max_evals, d_v, d_t, d_c, d_e))) return rc;
-  CU(cudaMemcpyAsync(verdict, d_v, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(t_hit, d_t, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(cmin, d_c, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, st));
-  if (evals) CU(cudaMemcpyAsync(evals, d_e, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return 0;
+  int rc = check_traj_call(ctx, "cfs_check_trajectories", B, H, x0, x, u, eta, margin_is_D, max_evals, verdict, t_hit, cmin);
+  if (rc || B == 0) return rc;
+  const size_t nj = ctx->nj, S = (size_t)B * H;
+  double *d_x0, *d_x, *d_u, *d_t, *d_c;
+  int *d_v, *d_e;
+  Area ar(ctx);
+  ar.in(d_x0, x0, 2 * nj * B).in(d_x, x, 2 * nj * S).in(d_u, u, nj * S).out(d_v, verdict, B).out(d_t, t_hit, B).out(d_c, cmin, B)
+      .out(d_e, evals, B);
+  if ((rc = ar.upload()) || (rc = check_traj_dev(ctx, B, H, d_x0, d_x, d_u, eta, margin_is_D, max_evals, d_v, d_t, d_c, d_e)))
+    return rc;
+  return ar.download();
 }
 
 // ---- the checked solve (include/cfs_b200.h) ------------------------------------------------------------------------
@@ -1928,7 +1942,7 @@ extern "C" int cfs_solve_checked(cfs_ctx *ctx, int B, int solver, int grad, cons
   int rc = check_solve(ctx, s);
   if (rc || B == 0) return rc;
   HostIo io;
-  if ((rc = upload(ctx, s, io)) || (rc = solve_checked_dev(ctx, io.d)) || (rc = download(ctx, io))) return rc;
+  if ((rc = upload(ctx, s, io)) || (rc = solve_checked_dev(ctx, io.d)) || (rc = io.t.d2h(ctx))) return rc;
   CU(cudaStreamSynchronize(ctx->stream));
   flush_staged(ctx, true);
   return 0;
@@ -1941,23 +1955,44 @@ extern "C" int cfs_nearest_steer(cfs_ctx *ctx, int n_nodes, const double *nodes,
   if (n_nodes < 1 || S < 0 || !nodes || (S > 0 && (!samples || !ratial || !parent || !newnode)))
     return fail(ctx, CFS_E_ARG, "cfs_nearest_steer: bad argument");
   if (S == 0) return 0;
-  CU(cudaSetDevice(ctx->device));
+  const size_t nj = ctx->nj;
+  double *d_nodes, *d_s, *d_r, *d_new;
+  int *d_par;
+  Area ar(ctx);
+  ar.in(d_nodes, nodes, nj * n_nodes).in(d_s, samples, nj * S).in(d_r, ratial, nj).out(d_par, parent, S).out(d_new, newnode, nj * S);
+  int rc = ar.upload();
+  if (rc) return rc;
+  CU(launch_nearest_steer(nj, n_nodes, d_nodes, S, d_s, d_r, step, d_par, d_new, ctx->stream));
+  return ar.download();
+}
+
+// The argument checks of cfs_rrt_find_routes and its device form (have_params: the four parameter vectors, or params, given)
+static int check_rrt_call(cfs_ctx *ctx, const char *who, int S, int max_iter, int nrnd, const void *x0, const void *goal,
+                          const void *goal_th, bool have_params, const void *rnd, const void *routes, const void *route_len,
+                          const void *n_nodes, const void *fail_out, const void *rnd_used) {
+  if (!ctx) return CFS_E_ARG;
+  int rc = check_ready(ctx, false);
+  if (rc) return rc;
+  if (S < 0 || max_iter < 1 || nrnd < 1 ||
+      (S > 0 && (!x0 || !goal || !goal_th || !have_params || !rnd || !routes || !route_len || !n_nodes || !fail_out || !rnd_used)))
+    return fail(ctx, CFS_E_ARG, "%s: bad argument", who);
+  return 0;
+}
+
+// Both forms of cfs_rrt_find_routes on device pointers: params = region_g | region_s | sample_off | ratial (nj each); the tree
+// outputs may be NULL
+static int rrt_dev(cfs_ctx *ctx, int S, int star, const double *x0, const double *goal, const double *goal_th, const double *params,
+                   double bi, int max_iter, const double *rnd, int nrnd, double *routes, int *route_len, int *n_nodes, int *fail_out,
+                   int *rnd_used, double *tree_nodes, int *tree_parent, double *tree_total) {
   const int nj = ctx->nj;
-  cudaStream_t st = ctx->stream;
-  int rc;
-  const size_t in_d = (size_t)nj * n_nodes + (size_t)nj * S + CFS_MAXL;
-  if ((rc = ensure(ctx, ctx->scratch_theta, sizeof(double) * in_d))) return rc;
-  if ((rc = ensure(ctx, ctx->scratch_out, sizeof(double) * (size_t)nj * S + sizeof(int) * (size_t)S + 64))) return rc;
-  double *d_nodes = ptr<double>(ctx->scratch_theta), *d_s = d_nodes + (size_t)nj * n_nodes, *d_r = d_s + (size_t)nj * S;
-  double *d_new = ptr<double>(ctx->scratch_out);
-  int *d_par = reinterpret_cast<int *>(d_new + (size_t)nj * S);
-  CU(cudaMemcpyAsync(d_nodes, nodes, sizeof(double) * (size_t)nj * n_nodes, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_s, samples, sizeof(double) * (size_t)nj * S, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_r, ratial, sizeof(double) * nj, cudaMemcpyHostToDevice, st));
-  CU(launch_nearest_steer(nj, n_nodes, d_nodes, S, d_s, d_r, step, d_par, d_new, st));
-  CU(cudaMemcpyAsync(parent, d_par, sizeof(int) * (size_t)S, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(newnode, d_new, sizeof(double) * (size_t)nj * S, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
+  RrtArgs a;
+  memset(&a, 0, sizeof(a));
+  a.tab = ctx->dtab; a.nj = nj; a.nobs = ctx->nobs; a.star = star; a.max_iter = max_iter; a.nrnd = nrnd; a.bi = bi;
+  a.x0 = x0; a.goal = goal; a.goal_th = goal_th;
+  a.region_g = params; a.region_s = params + nj; a.sample_off = params + 2 * nj; a.ratial = params + 3 * nj;
+  a.rnd = rnd; a.routes = routes; a.route_len = route_len; a.n_nodes = n_nodes; a.fail = fail_out; a.rnd_used = rnd_used;
+  a.tree_nodes = tree_nodes; a.tree_total = tree_total; a.tree_parent = tree_parent;
+  CU(launch_rrt_find_routes(a, S, ctx->stream));
   return 0;
 }
 
@@ -1966,58 +2001,28 @@ extern "C" int cfs_rrt_find_routes(cfs_ctx *ctx, int S, int star, const double *
                                    const double *ratial, double bi, int max_iter, const double *rnd, int nrnd, double *routes,
                                    int *route_len, int *n_nodes, int *fail_out, int *rnd_used, double *tree_nodes,
                                    int *tree_parent, double *tree_total, double *ms_kernel) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, false);
-  if (rc) return rc;
-  if (S < 0 || max_iter < 1 || nrnd < 1 ||
-      (S > 0 && (!x0 || !goal || !goal_th || !region_g || !region_s || !sample_off || !ratial || !rnd || !routes || !route_len ||
-                 !n_nodes || !fail_out || !rnd_used)))
-    return fail(ctx, CFS_E_ARG, "cfs_rrt_find_routes: bad argument");
-  if (S == 0) return 0;
-  CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj, cap = max_iter + 2;
-  cudaStream_t st = ctx->stream;
-  const size_t n_in = (size_t)3 * nj * S + 4 * (size_t)nj + (size_t)nrnd * S;
-  if ((rc = ensure(ctx, ctx->routes, sizeof(double) * n_in))) return rc;
+  int rc = check_rrt_call(ctx, "cfs_rrt_find_routes", S, max_iter, nrnd, x0, goal, goal_th,
+                          region_g && region_s && sample_off && ratial, rnd, routes, route_len, n_nodes, fail_out, rnd_used);
+  if (rc || S == 0) return rc;
+  const size_t nj = ctx->nj, cap = (size_t)max_iter + 2;
+  std::vector<double> params(4 * nj);  // the device form's params block
+  const double *parts[4] = {region_g, region_s, sample_off, ratial};
+  for (int p = 0; p < 4; ++p) memcpy(params.data() + p * nj, parts[p], sizeof(double) * nj);
   const bool tree = tree_nodes && tree_parent && tree_total;
-  const size_t out_d = (size_t)nj * cap * S + (tree ? (size_t)nj * cap * S + (size_t)cap * S : 0);
-  const size_t out_i = (size_t)4 * S + (tree ? (size_t)cap * S : 0);
-  if ((rc = ensure(ctx, ctx->scratch_out, sizeof(double) * out_d + sizeof(int) * out_i + 64))) return rc;
-  double *d_in = ptr<double>(ctx->routes);
-  double *d_x0 = d_in, *d_goal = d_x0 + (size_t)nj * S, *d_gth = d_goal + (size_t)nj * S, *d_rg = d_gth + (size_t)nj * S;
-  double *d_rs = d_rg + nj, *d_off = d_rs + nj, *d_rat = d_off + nj, *d_rnd = d_rat + nj;
-  double *d_routes = ptr<double>(ctx->scratch_out);
-  double *d_tn = tree ? d_routes + (size_t)nj * cap * S : nullptr, *d_tt = tree ? d_tn + (size_t)nj * cap * S : nullptr;
-  int *d_int = reinterpret_cast<int *>(d_routes + out_d);
-  int *d_len = d_int, *d_nn = d_len + S, *d_fail = d_nn + S, *d_used = d_fail + S, *d_tp = tree ? d_used + S : nullptr;
-  CU(cudaMemcpyAsync(d_x0, x0, sizeof(double) * nj * S, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_goal, goal, sizeof(double) * nj * S, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_gth, goal_th, sizeof(double) * nj * S, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_rg, region_g, sizeof(double) * nj, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_rs, region_s, sizeof(double) * nj, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_off, sample_off, sizeof(double) * nj, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_rat, ratial, sizeof(double) * nj, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_rnd, rnd, sizeof(double) * (size_t)nrnd * S, cudaMemcpyHostToDevice, st));
-  RrtArgs a;
-  memset(&a, 0, sizeof(a));
-  a.tab = ctx->dtab; a.nj = nj; a.nobs = ctx->nobs; a.star = star; a.max_iter = max_iter; a.nrnd = nrnd; a.bi = bi;
-  a.x0 = d_x0; a.goal = d_goal; a.goal_th = d_gth; a.region_g = d_rg; a.region_s = d_rs; a.sample_off = d_off; a.ratial = d_rat;
-  a.rnd = d_rnd; a.routes = d_routes; a.route_len = d_len; a.n_nodes = d_nn; a.fail = d_fail; a.rnd_used = d_used;
-  a.tree_nodes = d_tn; a.tree_total = d_tt; a.tree_parent = d_tp;
-  CU(cudaEventRecord(ctx->ev_a, st));
-  CU(launch_rrt_find_routes(a, S, st));
-  CU(cudaEventRecord(ctx->ev_b, st));
-  CU(cudaMemcpyAsync(routes, d_routes, sizeof(double) * (size_t)nj * cap * S, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(route_len, d_len, sizeof(int) * S, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(n_nodes, d_nn, sizeof(int) * S, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(fail_out, d_fail, sizeof(int) * S, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(rnd_used, d_used, sizeof(int) * S, cudaMemcpyDeviceToHost, st));
-  if (tree) {
-    CU(cudaMemcpyAsync(tree_nodes, d_tn, sizeof(double) * (size_t)nj * cap * S, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(tree_total, d_tt, sizeof(double) * (size_t)cap * S, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(tree_parent, d_tp, sizeof(int) * (size_t)cap * S, cudaMemcpyDeviceToHost, st));
-  }
-  CU(cudaStreamSynchronize(st));
+  double *d_x0, *d_goal, *d_gth, *d_params, *d_rnd, *d_routes, *d_tn = nullptr, *d_tt = nullptr;
+  int *d_len, *d_nn, *d_fail, *d_used, *d_tp = nullptr;
+  Area ar(ctx);
+  ar.in(d_x0, x0, nj * S).in(d_goal, goal, nj * S).in(d_gth, goal_th, nj * S).in(d_params, params.data(), 4 * nj)
+      .in(d_rnd, rnd, (size_t)nrnd * S).out(d_routes, routes, nj * cap * S).out(d_len, route_len, S).out(d_nn, n_nodes, S)
+      .out(d_fail, fail_out, S).out(d_used, rnd_used, S);
+  if (tree) ar.out(d_tn, tree_nodes, nj * cap * S).out(d_tt, tree_total, cap * S).out(d_tp, tree_parent, cap * S);
+  if ((rc = ar.upload())) return rc;
+  CU(cudaEventRecord(ctx->ev_a, ctx->stream));
+  if ((rc = rrt_dev(ctx, S, star, d_x0, d_goal, d_gth, d_params, bi, max_iter, d_rnd, nrnd, d_routes, d_len, d_nn, d_fail, d_used,
+                    d_tn, d_tp, d_tt)))
+    return rc;
+  CU(cudaEventRecord(ctx->ev_b, ctx->stream));
+  if ((rc = ar.download())) return rc;
   if (ms_kernel) {
     float ms = 0;
     cudaEventElapsedTime(&ms, ctx->ev_a, ctx->ev_b);
@@ -2030,25 +2035,15 @@ extern "C" int cfs_rrt_find_routes_device(cfs_ctx *ctx, int S, int star, const d
                                           const double *params, double bi, int max_iter, const double *rnd, int nrnd,
                                           double *routes, int *route_len, int *n_nodes, int *fail_out, int *rnd_used,
                                           int *route_len_or_fail, int sync) {
-  if (!ctx) return CFS_E_ARG;
-  int rc = check_ready(ctx, false);
-  if (rc) return rc;
-  if (S < 0 || max_iter < 1 || nrnd < 1 ||
-      (S > 0 && (!x0 || !goal || !goal_th || !params || !rnd || !routes || !route_len || !n_nodes || !fail_out || !rnd_used)))
-    return fail(ctx, CFS_E_ARG, "cfs_rrt_find_routes_device: bad argument");
-  if (S == 0) return 0;
+  int rc = check_rrt_call(ctx, "cfs_rrt_find_routes_device", S, max_iter, nrnd, x0, goal, goal_th, params != nullptr, rnd, routes,
+                          route_len, n_nodes, fail_out, rnd_used);
+  if (rc || S == 0) return rc;
   CU(cudaSetDevice(ctx->device));
-  const int nj = ctx->nj;
-  cudaStream_t st = ctx->stream;
-  RrtArgs a;
-  memset(&a, 0, sizeof(a));
-  a.tab = ctx->dtab; a.nj = nj; a.nobs = ctx->nobs; a.star = star; a.max_iter = max_iter; a.nrnd = nrnd; a.bi = bi;
-  a.x0 = x0; a.goal = goal; a.goal_th = goal_th;
-  a.region_g = params; a.region_s = params + nj; a.sample_off = params + 2 * nj; a.ratial = params + 3 * nj;
-  a.rnd = rnd; a.routes = routes; a.route_len = route_len; a.n_nodes = n_nodes; a.fail = fail_out; a.rnd_used = rnd_used;
-  CU(launch_rrt_find_routes(a, S, st));
-  if (route_len_or_fail) CU(launch_route_len_or_fail(S, route_len, fail_out, route_len_or_fail, st));
-  if (sync) CU(cudaStreamSynchronize(st));
+  if ((rc = rrt_dev(ctx, S, star, x0, goal, goal_th, params, bi, max_iter, rnd, nrnd, routes, route_len, n_nodes, fail_out, rnd_used,
+                    nullptr, nullptr, nullptr)))
+    return rc;
+  if (route_len_or_fail) CU(launch_route_len_or_fail(S, route_len, fail_out, route_len_or_fail, ctx->stream));
+  if (sync) CU(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 
